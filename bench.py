@@ -2,7 +2,7 @@
 """bench.py -- PD-UNet reconstruction throughput (slices/s) on BASELINE.json configs[1]:
 parallel-beam CT, 256x256, 64 -> 512 views sinogram upsampling, batch 16 per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step is one inference pass of the unrolled PD-UNet over one batch of synthetic sparse-view
@@ -13,7 +13,7 @@ between steps outside the events), max over ranks.  `e2e`: the same pass from pi
 to a host result.  `roofline`: the Radon forward-projection call timed live with CUDA events inside
 those same K steps.  `cpu_baseline` / `--impl reference`: the CPU oracle port of the same model and the
 same batch of 16 slices per step on all host cores -- `cpu_baseline` repeats the step until about 10 s are
-on the clock, `--impl reference` runs W warm-up and K timed steps, bounded at 150 s (the reference's own
+on the clock, `--impl reference` runs at most one warm-up and K timed steps (the reference's own
 operators, torch_radon, are CUDA-only and not mounted: SURVEY.md section 8c/8d).
 `operators`: every hot-path operator alone (L2 flushed): Radon forward / adjoint / filter at configs[1], NUFFT
 forward / adjoint at configs[0] and at the configs[3] per-GPU share, GSamples/s and fraction of the HBM roof.
@@ -21,6 +21,8 @@ forward / adjoint at configs[0] and at the configs[3] per-GPU share, GSamples/s 
 (256^2, 32 -> 256 spokes, one slice, CUDA graph), configs[2] fan-beam CT (512^2, 128 -> 1024 views, 8 slices per GPU),
 configs[3] radial-MRI training step (320^2, 8 coils, 48 spokes; forward + loss + backward + Adam captured in one CUDA
 graph, DDP's NCCL all-reduce inside it when --gpus N > 1).
+`--dump-outputs DIR`: what the last timed step of each leg returned, as .npy files.  Inputs and weights are seeded, so
+two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -129,6 +131,20 @@ def synthetic_sparse_sinograms(radon, device, batch, seed):
     return radon.forward(x)[:, None, ::UP].contiguous()
 
 
+def keep_output(dumps, name, t):
+    """For --dump-outputs: a host float32 copy of what the last timed step returned (complex as trailing re/im pairs).
+    Call it after the timed window has been synchronised: a captured graph's output is overwritten by its next replay."""
+    if dumps is not None:
+        t = t.detach()
+        dumps[name] = (torch.view_as_real(t) if t.is_complex() else t).float().cpu()
+
+
+def write_outputs(out_dir, dumps):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in dumps.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+
+
 # ============================================================================= our arm
 def run_ours(args):
     import pd_unet_b200 as pdu
@@ -208,9 +224,11 @@ def run_ours(args):
         for s, e in ev:
             flush.zero_()
             s.record()
-            run_step()
+            rec = run_step()
             e.record()
         torch.cuda.synchronize()
+    dumps = {} if args.dump_outputs and rank == 0 else None
+    keep_output(dumps, "reconstruction", rec)
     parallel.barrier()
     total_ms = parallel.max_over_ranks(sum(s.elapsed_time(e) for s, e in ev), dev)
 
@@ -234,10 +252,12 @@ def run_ours(args):
     # ---- the other BASELINE configs as model-level legs (every rank takes part: the training leg is DDP)
     del graphed
     torch.cuda.empty_cache()
-    extras = {} if args.no_extras else extra_legs(dev, flush, rank, world, local, args)
+    extras = {} if args.no_extras else extra_legs(dev, flush, rank, world, local, args, dumps)
 
     if rank != 0:
         return
+    if dumps is not None:
+        write_outputs(args.dump_outputs, dumps)
     peak, peak_src = peaks()
     slices = BATCH * world * args.steps
     alg_bytes = 4.0 * BATCH * (N * N + A_FULL * N)               # DESIGN.md: 4 B (N^2 + A D) per call
@@ -357,14 +377,15 @@ def _timed_steps(run, flush, steps, dev):
     return parallel.max_over_ranks(sum(a.elapsed_time(b) for a, b in ev), dev) / steps
 
 
-def extra_legs(dev, flush, rank, world, local, args):
+def extra_legs(dev, flush, rank, world, local, args, dumps=None):
     """configs[0], configs[2] and configs[3] at model level (see the module docstring).  Every leg is weak scaling
-    (fixed work per GPU); values are whole-job aggregates over the `world` GPUs, CUDA-event time, max over ranks."""
+    (fixed work per GPU); values are whole-job aggregates over the `world` GPUs, CUDA-event time, max over ranks.
+    Each leg times --steps steps; with `dumps` (a dict) it also keeps what the last of them returned."""
     import pd_unet_b200 as pdu
     from pd_unet_b200 import data, parallel
     from pd_unet_b200.graph import GraphedInference, GraphedTrainingStep
     from pd_unet_b200.model import PrimalDualUNetCT, PrimalDualUNetMRI
-    steps = max(3, min(args.steps, 10))
+    steps = args.steps
     out = {}
     # ---- configs[0]: radial-MRI inference, 256^2, 32 measured spokes regridded to 256, one slice per GPU
     n, sp_s, sp_f = 256, 32, 256
@@ -377,6 +398,7 @@ def extra_legs(dev, flush, rank, world, local, args):
     with torch.no_grad():
         g = GraphedInference(fn, d["kdata"], warmup=2)
     ms = _timed_steps(g.replay, flush, steps, dev)
+    keep_output(dumps, "cfg1_mri_inference", g.static_out)
     out["cfg1_mri_inference"] = {"workload": "configs[0]: radial-MRI PD-UNet 256x256, 32 spokes regridded to 256 on the GPU (own NUFFT), "
                                              "1 slice per GPU, CUDA graph", "ms_per_step": ms, "slices_per_s": world / (ms * 1e-3)}
     del g, mri, d
@@ -390,6 +412,7 @@ def extra_legs(dev, flush, rank, world, local, args):
     with torch.no_grad():
         g = GraphedInference(ct, sparse, warmup=2)
     ms = _timed_steps(g.replay, flush, steps, dev)
+    keep_output(dumps, "cfg3_fan_ct_inference", g.static_out)
     out["cfg3_fan_ct_inference"] = {"workload": "configs[2]: fan-beam CT PD-UNet 512x512, 128->1024 views, 8 slices per GPU, CUDA graph",
                                     "ms_per_step": ms, "slices_per_s": b * world / (ms * 1e-3),
                                     "peak_mem_GiB": torch.cuda.max_memory_allocated(dev) / 2 ** 30}
@@ -406,6 +429,7 @@ def extra_legs(dev, flush, rank, world, local, args):
     loss_fn = lambda o, t: (o - t).abs().pow(2).mean()
     step = GraphedTrainingStep(ddp, opt, loss_fn, (d["kdata"], d["omega"], d["smaps"], d["dcf"]), d["image"], warmup=3)
     ms = _timed_steps(step.graph.replay, flush, steps, dev)
+    keep_output(dumps, "cfg4_mri_training_loss", step.static_loss)
     out["cfg4_mri_training"] = {"workload": "configs[3]: radial-MRI PD-UNet 320x320, 8 coils, 48 spokes, training step (forward + MSE + "
                                             "backward + Adam), 2 slices per GPU, one CUDA graph" + (", DDP NCCL all-reduce inside" if world > 1 else ""),
                                 "ms_per_step": ms, "slices_per_s": b * world / (ms * 1e-3), "loss": float(step.static_loss.detach()),
@@ -496,18 +520,16 @@ def run_reference(args):
     warm = min(args.warmup, 1)                   # each step is seconds of CPU work
     for _ in range(warm):
         cpu_model_step(model, sparse, trig, g)
-    steps = args.steps
+    done = args.steps
     t0 = time.perf_counter()
-    done = 0
-    for _ in range(steps):
-        cpu_model_step(model, sparse, trig, g)
-        done += 1
-        if time.perf_counter() - t0 > 150.0:     # bounded: a few minutes for the whole run
-            break
+    for _ in range(done):
+        rec = cpu_model_step(model, sparse, trig, g)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"reconstruction": rec.float()})
     v = sample * done / dt
     base = {"value": v, "unit": "slices/s", "cores": cpu_cores(), "kind": "port", "host_cpus": os.cpu_count(),
-            "sample": f"{sample} slices per step, {done} step(s) timed (bounded at 150 s); " + CPU_NOTE}
+            "sample": f"{sample} slices per step, {done} step(s) timed; " + CPU_NOTE}
     _STDOUT.restore()
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": v, "unit": "slices/s", "n_gpus": args.gpus, "steps": done,
@@ -538,12 +560,18 @@ class StdoutToStderr:
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of every leg")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[0] / [2] / [3] model-level legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of each leg returned, on rank 0, as DIR/<name>.npy in float32 "
+                         "(about 13 MB): reconstruction and, unless --no-extras, cfg1_mri_inference (re/im in the last "
+                         "axis), cfg3_fan_ct_inference, cfg4_mri_training_loss; --impl reference writes its reconstruction")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     global _STDOUT
     _STDOUT = StdoutToStderr()
     if args.impl == "reference":

@@ -55,6 +55,13 @@ def kaiser_bessel_scaling(n: int, k: int, numpoints: int, kbwidth: float) -> np.
     return np.i0(alpha) / (J * ratio)
 
 
+# Device handles of plans collected while the current stream was capturing a CUDA graph.  Destroying a plan calls
+# cufftDestroy and cudaFree, which invalidate a capture, and a collection can happen inside one: an MRI model refers to
+# itself through its operator closures, so the cyclic garbage collector frees it (and its plans) at whatever allocation
+# triggers a collection.  The handles are destroyed with the next plan collected outside a capture.
+_DEFERRED_DESTROY: list = []
+
+
 class _Plan:
     """Owns one pdu_nufft_plan_t per device."""
 
@@ -224,8 +231,13 @@ class _Plan:
 
     def __del__(self):
         try:
-            for h in self._handles.values():
-                lib().pdu_nufft_plan_destroy(h)
+            if not self._handles:
+                return
+            _DEFERRED_DESTROY.extend(self._handles.values())
+            if torch.cuda.is_current_stream_capturing():
+                return
+            while _DEFERRED_DESTROY:
+                lib().pdu_nufft_plan_destroy(_DEFERRED_DESTROY.pop())
         except Exception:
             pass
 

@@ -355,3 +355,35 @@ def test_split_layout_and_density_weights():
         (AH(ksr, om, smaps=sm, norm="ortho", split=True, kweight=w) * xs[:, :2 * co]).sum().backward()
         want = A(xs, om, smaps=sm, norm="ortho", split=True) * w
         assert rel_l2(ksr.grad, want) <= 1e-5
+
+
+def test_a_plan_collected_during_graph_capture_leaves_the_capture_intact():
+    """An MRI model refers to itself through its operator closures, so the cyclic garbage collector may free it, and its
+    NUFFT plans, inside another CUDA-graph capture.  Releasing a plan's device memory there would invalidate that
+    capture; it is released with the next plan collected outside a capture instead."""
+    import gc
+    from pd_unet_b200 import nufft as nufft_mod
+    im = (128, 128)
+    omd = torch.from_numpy(_traj(12, 256)).to(DEV)
+    x = seeded((1, 1) + im, 91, complex_=True).to(DEV)
+    cycle = [pdu.KbNufft(im)]
+    cycle.append(cycle)
+    cycle[0]._plan.use_fused = True                  # builds the trajectory's row bins (device buffer + CUDA event)
+    cycle[0](x, omd)
+    a = torch.arange(1024.0, device=DEV)
+    gc.collect()                                     # only this test's plan is left to collect inside the capture
+    torch.cuda.synchronize()
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g):
+        del cycle
+        gc.collect()
+        b = a * 2
+    assert nufft_mod._DEFERRED_DESTROY
+    g.replay()
+    torch.cuda.synchronize()
+    assert torch.equal(b, a * 2)
+    op = pdu.KbNufft(im)
+    op(x, omd)
+    del op
+    gc.collect()
+    assert not nufft_mod._DEFERRED_DESTROY

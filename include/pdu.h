@@ -70,8 +70,8 @@ PDU_API long pdu_launch_count(int reset);
  * their loads so that the path can be tested. */
 PDU_API int pdu_device_error(int reset);
 /* Name and shape of the kernel the dispatcher of an operator chose in this thread's most recent
- * call: op in {"radon_fwd", "radon_adj", "filter", "nufft_fwd", "nufft_adj"}; "" before the first
- * call.  The string stays valid until the thread's next call of that operator. */
+ * call: op in {"radon_fwd", "radon_adj", "filter", "nufft_fwd", "nufft_adj", "toep"}; "" before the
+ * first call.  The string stays valid until the thread's next call of that operator. */
 PDU_API const char* pdu_last_kernel(const char* op);
 
 /* ------------------------------------------------------------------ CT ---- */
@@ -215,6 +215,36 @@ PDU_API int pdu_nufft_adj_binned_c64(pdu_nufft_plan_t* plan, const float* kdata,
                                      const float* smaps, const float* kweight, int batch, int coils,
                                      int smaps_batch, long m, float scale, const void* bins, int flags,
                                      void* workspace, size_t workspace_bytes, pdu_stream_t stream);
+
+/* Toeplitz-embedded normal operator A^H W A of the NUFFT: no interpolation, one zero-padded 2n0 x 2n1
+ * FFT, a pointwise multiply by a kernel and one cropped inverse FFT, whatever the trajectory length.
+ *   pdu_toep_plan_create      a plan with grid 2 n per axis, unit apodisation, marked as a Toeplitz plan
+ *                             (destroy it with pdu_nufft_plan_destroy).  PDU_EUNSUPPORTED for sizes whose
+ *                             2 n has a prime factor above 5 (or whose rows do not fit the shared-memory FFT).
+ *                             A Toeplitz plan passed to a pdu_nufft_* entry point, or a Kaiser-Bessel plan to
+ *                             a pdu_toep_* one, is PDU_EINVAL.
+ *   pdu_toep_workspace_bytes  scratch of pdu_toep_apply_c64 for `planes` = batch*coils planes; a call is cut
+ *                             into batch chunks of at most 512 MB of scratch, and wants the size of one chunk.
+ *   pdu_toep_kernel_c64       kernel [kernels, 2 n0, 2 n1] = fft2(p_circ) (unnormalised), p_circ the circulant
+ *                             layout of the point-spread function assembled from q1 = A^H w (omega) and
+ *                             q2 = A^H w (omega0 negated), both [kernels, n0, n1] c64 with n_shift 0, times
+ *                             `scale` (1, or 1/(k0 k1) of the NUFFT grid for norm="ortho").  ws: kernels * 4 n0 n1
+ *                             complex64 values.  Real weights only (p[-r] = conj p[r]).
+ *   pdu_toep_apply_c64        out = crop(ifft2(kernel . fft2(zero_pad(x)))) with ifft2 carrying 1/(4 n0 n1).
+ *                             image [batch, ci, n0, n1] c64 (ci == coils, or 1 with smaps [smaps_batch (1 or
+ *                             batch), coils, n0, n1]: out [batch, 1, n0, n1] = sum_c conj(S_c) T(S_c x));
+ *                             kernel [kernel_batch (1 or batch), 2 n0, 2 n1]; conj_kernel != 0 multiplies by
+ *                             conj(kernel) (the adjoint).  Square images with 2 n in {256, 512, 640, 1024, 2048}
+ *                             take three register-FFT launches, other sizes the generic pruned FFT passes;
+ *                             pdu_last_kernel("toep") says which.  Atomics-free and bit-reproducible.
+ * Replace [RECALL] torchkbnufft `ToepNufft.forward` and the FFT / assembly steps of `calc_toeplitz_kernel`. */
+PDU_API int pdu_toep_plan_create(pdu_nufft_plan_t** plan, int n0, int n1);
+PDU_API size_t pdu_toep_workspace_bytes(const pdu_nufft_plan_t* plan, int planes);
+PDU_API int pdu_toep_kernel_c64(pdu_nufft_plan_t* plan, const float* q1, const float* q2, float* kernel,
+                                int kernels, float scale, void* ws, size_t ws_bytes, pdu_stream_t stream);
+PDU_API int pdu_toep_apply_c64(pdu_nufft_plan_t* plan, const float* image, float* out, const float* kernel,
+                               int kernel_batch, const float* smaps, int batch, int coils, int smaps_batch,
+                               int conj_kernel, void* ws, size_t ws_bytes, pdu_stream_t stream);
 
 /* The layout change on its own, for the generic (complex64) entry points: split [planes, 2, n] float32 <-> complex64
  * [planes, n]; `weight` (nullable, float32 [n]) multiplies element e of every plane (the density compensation). */

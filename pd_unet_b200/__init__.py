@@ -4,8 +4,8 @@ See DESIGN.md.  Importing the package does not load the CUDA library; the first 
 and raises if it is missing (there is no CPU fallback)."""
 from ._lib import PduError, launch_count, set_option  # noqa: F401
 from .radon import Radon, RadonFanbeam  # noqa: F401
-from .nufft import (KbInterp, KbInterpAdjoint, KbNufft, KbNufftAdjoint,  # noqa: F401
-                    calc_density_compensation_function)
+from .nufft import (KbInterp, KbInterpAdjoint, KbNufft, KbNufftAdjoint, ToepNufft,  # noqa: F401
+                    calc_density_compensation_function, calc_toeplitz_kernel)
 from . import updates, parallel  # noqa: F401
 
 __version__ = "0.1.0"

@@ -15,6 +15,7 @@ PDU_GEOM_PARALLEL, PDU_GEOM_FAN = 0, 1
 WRAP_MODES = {"flip": 0, "periodic": 1, "clamp": 2}
 LAYOUT_NCHW, LAYOUT_NHWC = 0, 1
 NUFFT_IMAGE_SPLIT, NUFFT_KDATA_SPLIT = 1, 2
+PDU_EINVAL, PDU_EUNSUPPORTED = -1, -4
 
 
 class PduError(RuntimeError):
@@ -68,6 +69,10 @@ SIGNATURES = {
                                            C.c_size_t, _p]),
     "pdu_nufft_adj_binned_c64": (C.c_int, [_p, _p, _p, _p, _p, C.c_int, C.c_int, C.c_int, C.c_long, C.c_float, _p, C.c_int, _p,
                                            C.c_size_t, _p]),
+    "pdu_toep_plan_create": (C.c_int, [C.POINTER(_p), C.c_int, C.c_int]),
+    "pdu_toep_workspace_bytes": (C.c_size_t, [_p, C.c_int]),
+    "pdu_toep_kernel_c64": (C.c_int, [_p, _p, _p, _p, C.c_int, C.c_float, _p, C.c_size_t, _p]),
+    "pdu_toep_apply_c64": (C.c_int, [_p, _p, _p, _p, C.c_int, _p, C.c_int, C.c_int, C.c_int, C.c_int, _p, C.c_size_t, _p]),
     "pdu_complex_from_split_f32": (C.c_int, [_p, _p, _p, C.c_long, C.c_long, _p]),
     "pdu_split_from_complex_f32": (C.c_int, [_p, _p, C.c_long, C.c_long, _p]),
     "pdu_nufft_csr_build": (C.c_int, [_p, _p, C.c_long, _p, C.c_size_t, _p]),

@@ -6,6 +6,11 @@
 //                N non-zero rows) ; ff_cols_fwd_kernel (pruned column FFT)        -- pfft_fast.cuh, 2 passes
 //              other grids: apod_pad_kernel + cuFFT, or the generic pruned FFT of pfft.cuh (variant 1)
 //              interp_fwd_kernel J x J table-weighted gather per k-space sample, * phase
+//   normal operator (Toeplitz embedding, pdu_toep_*; no interpolation):
+//              square 2 N a FastFft size: ff_rows_fwd_kernel (unit apodisation) ; tz_cols_kernel (pruned column FFT,
+//                x kernel column, pruned inverse column FFT, in place) ; tz_rows_out_kernel (pruned inverse row FFT,
+//                x conj(smaps) summed over coils)                                  -- 3 launches, no K x K grid
+//              other 2, 3, 5 sizes: pfft rows / cols forward, tz_mul_kernel, pfft rows / cols adjoint, crop_apod_kernel
 //   adjoint :  trajectory used more than once: sorted (CSR) gather interp_adj_csrT_kernel on plane-interleaved
 //                kdata -- no atomics, no memset, reproducible; else memset + interp_adj_kernel (float2 atomics)
 //              inverse FFT: ff_rows_adj_kernel / ff_cols_adj_kernel (only the N kept outputs per axis), or cuFFT
@@ -1060,6 +1065,7 @@ int launch_crop_apod(pdu_nufft_plan* p, const float2* U, const float2* smaps, fl
 static int check_call(const pdu_nufft_plan* p, const void* a, const void* b, const void* omega, int batch, int coils,
                       int smaps_batch, const void* smaps, long m, const char* who) {
     PDU_REQUIRE(p != nullptr, "%s: plan is null", who);
+    PDU_REQUIRE(!p->toep, "%s: a Toeplitz plan (pdu_toep_plan_create) has no interpolation tables", who);
     PDU_REQUIRE(a && b && omega, "%s: null pointer", who);
     PDU_REQUIRE(batch > 0 && coils > 0 && m > 0, "%s: batch, coils and m must be > 0", who);
     PDU_REQUIRE((long)batch * coils <= 65535L * 64, "%s: too many planes", who);
@@ -1067,6 +1073,267 @@ static int check_call(const pdu_nufft_plan* p, const void* a, const void* b, con
     int dev = -1;
     PDU_CUDA(cudaGetDevice(&dev));
     PDU_REQUIRE(dev == p->device, "%s: plan was created on device %d, current device is %d", who, p->device, dev);
+    return PDU_OK;
+}
+
+// ------------------------------------------------------------------ Toeplitz-embedded normal operator (pdu_toep_*)
+// T x = crop(ifft2(kernel . fft2(zero_pad_2N(x))))  -- A^H W A of the NUFFT without any interpolation ([RECALL]
+// torchkbnufft ToepNufft / calc_toeplitz_kernel).  The kernel is the 2-D DFT of the point-spread function p in
+// circulant layout (DESIGN.md section 3.4).
+
+// p_circ [kernels][2 n0][2 n1] from q1 = A^H w (omega) and q2 = A^H w (omega0 negated), both with n_shift 0:
+//   q1[a, b] = p[a, b], q2[a, b] = p[-a, b], p[-a, -b] = conj p[a, b] (real weights); the row i0 = n0 and the column
+//   i1 = n1 are zero
+__global__ void __launch_bounds__(256)
+    tz_assemble_kernel(const float2* __restrict__ q1, const float2* __restrict__ q2, float2* __restrict__ out, int n0, int n1,
+                       float scale, long total) {
+    const int l0 = 2 * n0, l1 = 2 * n1;
+    const long plane = (long)n0 * n1;
+    for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
+        const int i1 = (int)(i % l1);
+        const long t = i / l1;
+        const int i0 = (int)(t % l0);
+        const long b = t / l0;
+        float2 v = make_float2(0.f, 0.f);
+        if (i0 != n0 && i1 != n1) {
+            const bool lo0 = i0 < n0, lo1 = i1 < n1;
+            const int a0 = lo0 ? i0 : l0 - i0, a1 = lo1 ? i1 : l1 - i1;
+            v = __ldg((lo0 == lo1 ? q1 : q2) + b * plane + (long)a0 * n1 + a1);
+            if (!lo1) v.y = -v.y;
+        }
+        out[i] = make_float2(v.x * scale, v.y * scale);
+    }
+}
+
+// generic path: grid [planes][k0][k1] *= kernel (or its conjugate); plane p uses kernel p / coils (batch element) when
+// there is one kernel per batch element
+__global__ void __launch_bounds__(256)
+    tz_mul_kernel(float2* __restrict__ grid, const float2* __restrict__ kern, long cells, int coils, int kernel_batch, int conj,
+                  long total) {
+    for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
+        const long p = i / cells, c = i - p * cells;
+        float2 k = __ldg(kern + (kernel_batch == 1 ? 0 : p / coils) * cells + c);
+        if (conj) k.y = -k.y;
+        grid[i] = cmul(grid[i], k);
+    }
+}
+
+// fast path, pass 2: SEQ neighbouring columns of T [planes][N][K] (the row pass's output) per CTA, the layout of
+// ff_cols_fwd_kernel.  Per column: forward FFT of the N stored rows (HALF_IN), x kernel column on the way into shared
+// memory (ST_BUF), inverse FFT from there (LD_BUF) keeping the first N outputs (HALF_OUT), written back in place -- the
+// CTA owns its columns across every row, so no other CTA reads them.
+template <int K, int SEQ>
+__global__ void __launch_bounds__(SEQ* FastFft<K>::TPS)
+    tz_cols_kernel(float2* __restrict__ T, const float2* __restrict__ kern, const float2* __restrict__ tw_g, int coils,
+                   int kernel_batch, int conj) {
+    using F = FastFft<K>;
+    constexpr int N = K / 2, TPS = F::TPS, NS3 = F::NS3, PITCH = F::template pitch<3>();
+    float2* buf = pf_smem<float2>();
+    float2* tw = buf + SEQ * PITCH;
+    const int tid = threadIdx.x, t = tid / SEQ, s = tid - t * SEQ;
+    const int p = blockIdx.y;
+    const int col = blockIdx.x * SEQ + s;          // K is a multiple of SEQ: every column exists
+    for (int i = tid; i < K; i += SEQ * TPS) tw[i] = __ldg(tw_g + i);
+    float2* colp = T + (long)p * N * K + col;
+    const float2* kc = kern + (long)(kernel_batch == 1 ? 0 : p / coils) * K * K + col;
+    float2* seq = buf + s * PITCH;
+    {
+        const float2* src = colp + (long)t * K;
+        auto ld = [&](int r) { return __ldcs(src + r * (TPS * K)); };
+        // output element e = j + r NS3 (row frequency) at its padded position pos(j) + r (NS3 + NS3 / 8)
+        auto st = [&](int j, int r, float2 v) {
+            float2 k = __ldg(kc + (long)(j + r * NS3) * K);
+            if (conj) k.y = -k.y;
+            seq[(j + (j >> 3)) + r * (NS3 + NS3 / 8)] = cmul(v, k);
+        };
+        ff_transform<K, 3, false, true, false, false, true>(seq, tw, t, ld, st);
+    }
+    __syncthreads();                               // every product is in shared memory
+    {
+        const float2* in = seq + (t + (t >> 3));   // input element t + r TPS at pos(t) + r (TPS + TPS / 8)
+        auto ld = [&](int r) { return in[r * (TPS + TPS / 8)]; };
+        auto st = [&](int j, int r, float2 v) { __stcs(colp + (long)(j + r * NS3) * K, v); };
+        ff_transform<K, 3, true, false, true, true>(seq, tw, t, ld, st);
+    }
+}
+
+// fast path, pass 3: SEQ rows of one output plane per CTA: pruned inverse row FFT of T's N rows (first N outputs),
+// x scale; with coil maps the CTA walks the batch element's coils in a fixed order and sums conj(S_c) T_c in registers
+// (bit-reproducible; no cropped intermediate, no crop_apod_kernel pass)
+template <int K, int SEQ>
+__global__ void __launch_bounds__(SEQ* FastFft<K>::TPS)
+    tz_rows_out_kernel(const float2* __restrict__ T, const float2* __restrict__ smaps, float2* __restrict__ out,
+                       const float2* __restrict__ tw_g, int coils, int smaps_batch, float scale) {
+    using F = FastFft<K>;
+    constexpr int N = K / 2, TPS = F::TPS, NS3 = F::NS3, R3 = F::R3;
+    constexpr int PER = TPS >= NS3 ? 1 : NS3 / TPS;     // last-pass butterflies per thread (ff_transform)
+    static_assert(PER <= 2, "outputs j = t or t + TPS");
+    float2* buf = pf_smem<float2>();
+    float2* tw = buf + SEQ * F::template pitch<4>();
+    const int tid = threadIdx.x, s = tid / TPS, t = tid - s * TPS;
+    const int q = blockIdx.y;                            // batch element (coil maps) or plane
+    const int row = blockIdx.x * SEQ + s;
+    for (int i = tid; i < K; i += SEQ * TPS) tw[i] = __ldg(tw_g + i);
+    const bool live = row < N;
+    float2 acc[PER][R3];
+#pragma unroll
+    for (int i = 0; i < PER; ++i)
+#pragma unroll
+        for (int r = 0; r < R3; ++r) acc[i][r] = make_float2(0.f, 0.f);
+    const int nc = smaps ? coils : 1;
+    const float2* sm = smaps ? smaps + ((long)(smaps_batch == 1 ? 0 : q) * coils * N + row) * N : nullptr;
+    for (int c = 0; c < nc; ++c) {
+        const long p = smaps ? (long)q * coils + c : q;
+        const float2* src = T + (p * N + row) * K + t;
+        const float2* smc = sm ? sm + (long)c * N * N : nullptr;
+        auto ld = [&](int r) { return live ? __ldcs(src + r * TPS) : make_float2(0.f, 0.f); };
+        auto st = [&](int j, int r, float2 v) {
+            if (!live) return;
+            if (smc) v = cmul_conj(v, __ldg(smc + j + r * NS3));
+            if (PER == 1 || j < TPS) {
+                acc[0][r].x += v.x;
+                acc[0][r].y += v.y;
+            } else {
+                acc[PER - 1][r].x += v.x;
+                acc[PER - 1][r].y += v.y;
+            }
+        };
+        ff_transform<K, 4, true, false, true, false, false, true>(buf + s * F::template pitch<4>(), tw, t, ld, st);
+        __syncthreads();                                 // the next coil's pass-1 stores reuse the buffer
+    }
+    if (!live) return;
+    float2* dst = out + ((long)q * N + row) * N;
+#pragma unroll
+    for (int i = 0; i < PER; ++i) {
+        const int j = t + i * TPS;
+        if (j < NS3) {
+#pragma unroll
+            for (int r = 0; r < R3 / 2; ++r) dst[j + r * NS3] = make_float2(acc[i][r].x * scale, acc[i][r].y * scale);
+        }
+    }
+}
+
+static bool tz_fast(const pdu_nufft_plan* p) { return p->n0 == p->n1 && p->k0 == p->k1 && fast_fft_size(p->k0); }
+
+// scratch per plane: T [N][K] on the fast path; grid + intermediate + cropped planes on the generic one
+static size_t tz_plane_bytes(const pdu_nufft_plan* p) {
+    if (tz_fast(p)) return (size_t)p->n0 * p->k1 * sizeof(float2);
+    const size_t mid = (size_t)std::max((long)p->n0 * p->k1, (long)p->k0 * p->n1);
+    return ((size_t)p->k0 * p->k1 + mid + (size_t)p->n0 * p->n1) * sizeof(float2);
+}
+
+// batch elements per chunk: the scratch stays under 512 MB (as the NUFFT's) and a chunk's planes fit gridDim.y;
+// pd_unet_b200/nufft.py::_ToepPlan.chunk repeats this arithmetic to size the workspace
+static int tz_batch_chunk(const pdu_nufft_plan* p, int batch, int coils) {
+    long planes = (long)(((size_t)512 << 20) / tz_plane_bytes(p));
+    if (planes > 65535) planes = 65535;
+    long cb = planes / coils;
+    if (cb < 1) cb = 1;
+    return (int)(cb < batch ? cb : batch);
+}
+
+constexpr int TZ_SEQ_ROWS = 4;
+template <int K>
+static constexpr int tz_seq_rows_out() { return K == 2048 ? 2 : TZ_SEQ_ROWS; }
+
+template <int K>
+static int tz_apply_fast(pdu_nufft_plan* p, const float2* image, float2* out, const float2* kern, int kernel_batch,
+                         const float2* smaps, int batch, int coils, int smaps_batch, int conj, float2* T, cudaStream_t st) {
+    constexpr int N = K / 2, SC = ff_seq_cols<K>(), SO = tz_seq_rows_out<K>();
+    const int planes = batch * coils;
+    PDU_CUDA((ensure_dyn_smem<ff_rows_fwd_kernel<K, FF_SEQ_ROWS>>((int)ff_smem_bytes<K>(FF_SEQ_ROWS))));
+    PDU_CUDA((ensure_dyn_smem<tz_cols_kernel<K, SC>>((int)ff_smem_bytes<K>(SC))));
+    PDU_CUDA((ensure_dyn_smem<tz_rows_out_kernel<K, SO>>((int)ff_smem_bytes<K>(SO))));
+    ff_rows_fwd_kernel<K, FF_SEQ_ROWS><<<dim3((unsigned)cdiv(N, FF_SEQ_ROWS), (unsigned)planes), FF_SEQ_ROWS * FastFft<K>::TPS,
+                                         ff_smem_bytes<K>(FF_SEQ_ROWS), st>>>(image, smaps, T, p->d_s0, p->d_s1, p->d_w1,
+                                                                              dims_of(p), coils, smaps_batch);
+    PDU_LAUNCHED();
+    tz_cols_kernel<K, SC><<<dim3((unsigned)(K / SC), (unsigned)planes), SC * FastFft<K>::TPS, ff_smem_bytes<K>(SC), st>>>(
+        T, kern, p->d_w0, coils, kernel_batch, conj);
+    PDU_LAUNCHED();
+    const int out_planes = smaps ? batch : planes;
+    tz_rows_out_kernel<K, SO><<<dim3((unsigned)cdiv(N, SO), (unsigned)out_planes), SO * FastFft<K>::TPS, ff_smem_bytes<K>(SO),
+                                 st>>>(T, smaps, out, p->d_w1, coils, smaps_batch, 1.f / ((float)K * (float)K));
+    PDU_LAUNCHED();
+    note_kernel(OP_TOEP, "ff_rows_fwd_kernel<%d,%d> + tz_cols_kernel<%d,%d> + tz_rows_out_kernel<%d,%d> (fast path, %d planes of %dx%d)",
+                K, FF_SEQ_ROWS, K, SC, K, SO, planes, N, N);
+    return PDU_OK;
+}
+
+// the generic passes' column SEQ: 8 where it fits shared memory, 2 otherwise (2048-point columns)
+static bool tz_cols_seq8(const pdu_nufft_plan* p) { return pf_smem_bytes(PF_SEQ_COLS, p->k0) <= 200 * 1024; }
+
+template <int SC>
+static int tz_apply_generic(pdu_nufft_plan* p, const float2* image, float2* out, const float2* kern, int kernel_batch,
+                            const float2* smaps, int batch, int coils, int smaps_batch, int conj, float2* ws, cudaStream_t st) {
+    const int planes = batch * coils;
+    const long cells = (long)p->k0 * p->k1;
+    float2* grid = ws;
+    float2* T = grid + planes * cells;
+    float2* U = T + (long)planes * std::max((long)p->n0 * p->k1, (long)p->k0 * p->n1);
+    const NufftDims d = dims_of(p);
+    const int pitch1 = pfft_pitch(p->k1), pitch0 = pfft_pitch(p->k0);
+    int rc = pf_set_smem(pfft_rows_fwd_kernel<PF_SEQ_ROWS>, pf_smem_bytes(PF_SEQ_ROWS, p->k1));
+    if (!rc) rc = pf_set_smem(pfft_cols_fwd_kernel<SC>, pf_smem_bytes(SC, p->k0));
+    if (!rc) rc = pf_set_smem(pfft_rows_adj_kernel<PF_SEQ_ROWS>, pf_smem_bytes(PF_SEQ_ROWS, p->k1));
+    if (!rc) rc = pf_set_smem(pfft_cols_adj_kernel<SC>, pf_smem_bytes(SC, p->k0));
+    if (rc) return rc;
+    pfft_rows_fwd_kernel<PF_SEQ_ROWS><<<dim3((unsigned)cdiv(p->n0, PF_SEQ_ROWS), (unsigned)planes), 256,
+                                        pf_smem_bytes(PF_SEQ_ROWS, p->k1), st>>>(image, smaps, T, p->d_s0, p->d_s1, p->d_w1, p->pf1,
+                                                                                 d, coils, smaps_batch, pitch1);
+    PDU_LAUNCHED();
+    pfft_cols_fwd_kernel<SC><<<dim3((unsigned)cdiv(p->k1, SC), (unsigned)planes), 256, pf_smem_bytes(SC, p->k0), st>>>(
+        T, grid, p->d_w0, p->pf0, d, pitch0);
+    PDU_LAUNCHED();
+    tz_mul_kernel<<<stream_grid(planes * cells), 256, 0, st>>>(grid, kern, cells, coils, kernel_batch, conj, planes * cells);
+    PDU_LAUNCHED();
+    pfft_rows_adj_kernel<PF_SEQ_ROWS><<<dim3((unsigned)cdiv(p->k0, PF_SEQ_ROWS), (unsigned)planes), 256,
+                                        pf_smem_bytes(PF_SEQ_ROWS, p->k1), st>>>(grid, T, p->d_w1, p->pf1, d, pitch1);
+    PDU_LAUNCHED();
+    pfft_cols_adj_kernel<SC><<<dim3((unsigned)cdiv(p->n1, SC), (unsigned)planes), 256, pf_smem_bytes(SC, p->k0), st>>>(
+        T, U, p->d_w0, p->pf0, d, pitch0);
+    PDU_LAUNCHED();
+    const int out_planes = smaps ? batch : planes;
+    rc = launch_crop_apod(p, U, smaps, out, out_planes, coils, smaps_batch, 1.f / ((float)p->k0 * (float)p->k1), 0, st);
+    if (rc) return rc;
+    note_kernel(OP_TOEP, "pfft_rows_fwd_kernel<%d> + pfft_cols_fwd_kernel<%d> + tz_mul_kernel + pfft_rows_adj_kernel<%d> + "
+                "pfft_cols_adj_kernel<%d> + crop_apod_kernel (generic path, %d planes of %dx%d)",
+                PF_SEQ_ROWS, SC, PF_SEQ_ROWS, SC, planes, p->n0, p->n1);
+    return PDU_OK;
+}
+
+static int tz_apply_chunk(pdu_nufft_plan* p, const float2* image, float2* out, const float2* kern, int kernel_batch,
+                          const float2* smaps, int batch, int coils, int smaps_batch, int conj, float2* ws, cudaStream_t st) {
+    if (tz_fast(p)) {
+        switch (p->k0) {
+            case 256: return tz_apply_fast<256>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, st);
+            case 512: return tz_apply_fast<512>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, st);
+            case 640: return tz_apply_fast<640>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, st);
+            case 1024: return tz_apply_fast<1024>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, st);
+            default: return tz_apply_fast<2048>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, st);
+        }
+    }
+    if (tz_cols_seq8(p))
+        return tz_apply_generic<PF_SEQ_COLS>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, st);
+    return tz_apply_generic<2>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, st);
+}
+
+// kernel build, step 4: the full (unpruned) 2-D FFT of p_circ, in place in `kern` with T as the intermediate
+template <int SC>
+static int tz_kernel_fft(pdu_nufft_plan* p, float2* kern, float2* T, int kernels, cudaStream_t st) {
+    NufftDims d = dims_of(p);
+    d.n0 = p->k0;            // pruning off: every row of the input is stored, every column is transformed
+    d.n1 = p->k1;
+    int rc = pf_set_smem(pfft_rows_fwd_kernel<PF_SEQ_ROWS>, pf_smem_bytes(PF_SEQ_ROWS, p->k1));
+    if (!rc) rc = pf_set_smem(pfft_cols_fwd_kernel<SC>, pf_smem_bytes(SC, p->k0));
+    if (rc) return rc;
+    pfft_rows_fwd_kernel<PF_SEQ_ROWS><<<dim3((unsigned)cdiv(p->k0, PF_SEQ_ROWS), (unsigned)kernels), 256,
+                                        pf_smem_bytes(PF_SEQ_ROWS, p->k1), st>>>(kern, nullptr, T, p->d_s0, p->d_s1, p->d_w1, p->pf1,
+                                                                                 d, 1, 1, pfft_pitch(p->k1));
+    PDU_LAUNCHED();
+    pfft_cols_fwd_kernel<SC><<<dim3((unsigned)cdiv(p->k1, SC), (unsigned)kernels), 256, pf_smem_bytes(SC, p->k0), st>>>(
+        T, kern, p->d_w0, p->pf0, d, pfft_pitch(p->k0));
+    PDU_LAUNCHED();
     return PDU_OK;
 }
 
@@ -1347,12 +1614,14 @@ size_t pdu_nufft_csr_bytes2(const pdu_nufft_plan_t* p, long m, size_t* persist_b
 
 int pdu_nufft_csr_build(pdu_nufft_plan_t* p, const float* omega, long m, void* csr, size_t csr_bytes, pdu_stream_t stream) {
     PDU_REQUIRE(p && omega && m > 0, "pdu_nufft_csr_build: null pointer or m <= 0");
+    PDU_REQUIRE(!p->toep, "pdu_nufft_csr_build: a Toeplitz plan has no interpolation tables");
     return csr_build(p, omega, m, csr, csr_bytes, (cudaStream_t)stream);
 }
 
 int pdu_nufft_interp_adj_csr_c64(pdu_nufft_plan_t* p, const float* kdata, float* grid, const void* csr, int planes, long m,
                                  pdu_stream_t stream) {
     PDU_REQUIRE(p && kdata && grid && csr && planes > 0 && m > 0, "pdu_nufft_interp_adj_csr_c64: null pointer or empty problem");
+    PDU_REQUIRE(!p->toep, "pdu_nufft_interp_adj_csr_c64: a Toeplitz plan has no interpolation tables");
     return launch_interp_adj_csr(p, (const float2*)kdata, (float2*)grid, csr, planes, m, (cudaStream_t)stream);
 }
 
@@ -1456,6 +1725,120 @@ int pdu_nufft_interp_adj_c64(pdu_nufft_plan_t* p, const float* kdata, float* gri
     int rc = check_call(p, kdata, grid, omega, planes, 1, 1, nullptr, m, "pdu_nufft_interp_adj_c64");
     if (rc) return rc;
     return launch_interp_adj(p, (const float2*)kdata, (float2*)grid, omega, planes, m, (cudaStream_t)stream);
+}
+
+int pdu_toep_plan_create(pdu_nufft_plan_t** plan, int n0, int n1) {
+    PDU_REQUIRE(plan != nullptr, "pdu_toep_plan_create: plan is null");
+    *plan = nullptr;
+    PDU_REQUIRE(n0 > 0 && n1 > 0 && n0 <= 2048 && n1 <= 2048, "pdu_toep_plan_create: need 0 < n <= 2048 per axis (got %d x %d)", n0, n1);
+    const int k0 = 2 * n0, k1 = 2 * n1;
+    PfftPlan pf0, pf1;
+    // the kernel build's FFT and the generic apply run the run-time-radix passes: 2, 3, 5 sizes whose rows (4 per CTA)
+    // and columns (2 per CTA) fit shared memory; the fast path's sizes are among them
+    if (!pfft_factor(k0, &pf0) || !pfft_factor(k1, &pf1) || pf_smem_bytes(PF_SEQ_ROWS, k1) > 200 * 1024 ||
+        pf_smem_bytes(2, k0) > 200 * 1024) {
+        set_error("pdu_toep_plan_create: no Toeplitz path for %d x %d (the embedding grid %d x %d must factor into 2, 3, 5 "
+                  "and fit the shared-memory FFT)", n0, n1, k0, k1);
+        return PDU_EUNSUPPORTED;
+    }
+    pdu_nufft_plan* p = new (std::nothrow) pdu_nufft_plan();
+    if (!p) {
+        set_error("pdu_toep_plan_create: out of host memory");
+        return PDU_ENOMEM;
+    }
+    p->n0 = n0; p->n1 = n1; p->k0 = k0; p->k1 = k1; p->J = 0; p->L = 0;
+    p->shift0 = p->shift1 = 0;
+    p->d_t0 = p->d_t1 = nullptr;
+    p->d_s0 = p->d_s1 = nullptr;
+    p->d_w0 = p->d_w1 = nullptr;
+    p->pfft_ok = true;
+    p->pf0 = pf0;
+    p->pf1 = pf1;
+    p->toep = true;
+    cudaError_t e = cudaGetDevice(&p->device);
+    for (int ax = 0; ax < 2 && e == cudaSuccess; ++ax) {
+        const int K = ax == 0 ? k0 : k1;
+        std::vector<float> ones((size_t)K, 1.f);        // unit apodisation (every entry a row / column pass may read)
+        std::vector<float2> w((size_t)K);
+        for (int i = 0; i < K; ++i) {
+            const double a = -2.0 * 3.14159265358979323846 * (double)i / (double)K;
+            w[i] = make_float2((float)cos(a), (float)sin(a));
+        }
+        float** s = ax == 0 ? &p->d_s0 : &p->d_s1;
+        float2** tw = ax == 0 ? &p->d_w0 : &p->d_w1;
+        e = cudaMalloc(s, (size_t)K * sizeof(float));
+        if (e == cudaSuccess) e = cudaMemcpy(*s, ones.data(), (size_t)K * sizeof(float), cudaMemcpyHostToDevice);
+        if (e == cudaSuccess) e = cudaMalloc(tw, (size_t)K * sizeof(float2));
+        if (e == cudaSuccess) e = cudaMemcpy(*tw, w.data(), (size_t)K * sizeof(float2), cudaMemcpyHostToDevice);
+    }
+    if (e != cudaSuccess) {
+        set_error("pdu_toep_plan_create: %s", cudaGetErrorString(e));
+        pdu_nufft_plan_destroy(p);
+        return PDU_ECUDA;
+    }
+    *plan = p;
+    return PDU_OK;
+}
+
+size_t pdu_toep_workspace_bytes(const pdu_nufft_plan_t* p, int planes) {
+    if (!p || !p->toep || planes <= 0) return 0;
+    return (size_t)planes * tz_plane_bytes(p);
+}
+
+int pdu_toep_kernel_c64(pdu_nufft_plan_t* p, const float* q1, const float* q2, float* kernel, int kernels, float scale,
+                        void* ws, size_t ws_bytes, pdu_stream_t stream) {
+    PDU_REQUIRE(p != nullptr, "pdu_toep_kernel_c64: plan is null");
+    PDU_REQUIRE(p->toep, "pdu_toep_kernel_c64: not a Toeplitz plan (use pdu_toep_plan_create)");
+    PDU_REQUIRE(q1 && q2 && kernel, "pdu_toep_kernel_c64: null pointer");
+    PDU_REQUIRE(kernels > 0 && kernels <= 65535, "pdu_toep_kernel_c64: kernels must be in 1..65535");
+    const size_t need = (size_t)kernels * p->k0 * p->k1 * sizeof(float2);
+    if (!ws || ws_bytes < need) {
+        set_error("pdu_toep_kernel_c64: workspace of %zu bytes required, got %zu", need, ws ? ws_bytes : (size_t)0);
+        return PDU_ENOMEM;
+    }
+    int dev = -1;
+    PDU_CUDA(cudaGetDevice(&dev));
+    PDU_REQUIRE(dev == p->device, "pdu_toep_kernel_c64: plan was created on device %d, current device is %d", p->device, dev);
+    PDU_CHECK_DEVICE("pdu_toep_kernel_c64");
+    cudaStream_t st = (cudaStream_t)stream;
+    const long total = (long)kernels * p->k0 * p->k1;
+    tz_assemble_kernel<<<stream_grid(total), 256, 0, st>>>((const float2*)q1, (const float2*)q2, (float2*)kernel, p->n0, p->n1,
+                                                           scale, total);
+    PDU_LAUNCHED();
+    if (tz_cols_seq8(p)) return tz_kernel_fft<PF_SEQ_COLS>(p, (float2*)kernel, (float2*)ws, kernels, st);
+    return tz_kernel_fft<2>(p, (float2*)kernel, (float2*)ws, kernels, st);
+}
+
+int pdu_toep_apply_c64(pdu_nufft_plan_t* p, const float* image, float* out, const float* kernel, int kernel_batch,
+                       const float* smaps, int batch, int coils, int smaps_batch, int conj_kernel, void* ws, size_t ws_bytes,
+                       pdu_stream_t stream) {
+    PDU_REQUIRE(p != nullptr, "pdu_toep_apply_c64: plan is null");
+    PDU_REQUIRE(p->toep, "pdu_toep_apply_c64: not a Toeplitz plan (use pdu_toep_plan_create)");
+    PDU_REQUIRE(image && out && kernel, "pdu_toep_apply_c64: null pointer");
+    PDU_REQUIRE(batch > 0 && coils > 0 && coils <= 65535, "pdu_toep_apply_c64: batch must be > 0 and coils in 1..65535");
+    PDU_REQUIRE(kernel_batch == 1 || kernel_batch == batch, "pdu_toep_apply_c64: kernel batch must be 1 or batch");
+    if (smaps) PDU_REQUIRE(smaps_batch == 1 || smaps_batch == batch, "pdu_toep_apply_c64: smaps batch must be 1 or batch");
+    const int cb = tz_batch_chunk(p, batch, coils);
+    const size_t need = pdu_toep_workspace_bytes(p, cb * coils);
+    if (!ws || ws_bytes < need) {
+        set_error("pdu_toep_apply_c64: workspace of %zu bytes required, got %zu", need, ws ? ws_bytes : (size_t)0);
+        return PDU_ENOMEM;
+    }
+    int dev = -1;
+    PDU_CUDA(cudaGetDevice(&dev));
+    PDU_REQUIRE(dev == p->device, "pdu_toep_apply_c64: plan was created on device %d, current device is %d", p->device, dev);
+    PDU_CHECK_DEVICE("pdu_toep_apply_c64");
+    const long plane = (long)p->n0 * p->n1, cells = (long)p->k0 * p->k1;
+    const long img_b = (smaps ? 1 : coils) * plane, out_b = img_b, smap_b = smaps_batch == 1 ? 0 : coils * plane;
+    for (int b0 = 0; b0 < batch; b0 += cb) {
+        const int nb = b0 + cb <= batch ? cb : batch - b0;
+        int rc = tz_apply_chunk(p, (const float2*)image + b0 * img_b, (float2*)out + b0 * out_b,
+                                (const float2*)kernel + (kernel_batch == 1 ? 0 : b0 * cells), kernel_batch == 1 ? 1 : nb,
+                                smaps ? (const float2*)smaps + b0 * smap_b : nullptr, nb, coils, smaps_batch == 1 ? 1 : nb,
+                                conj_kernel ? 1 : 0, (float2*)ws, (cudaStream_t)stream);
+        if (rc) return rc;
+    }
+    return PDU_OK;
 }
 
 }  // extern "C"

@@ -25,6 +25,9 @@ struct pdu_nufft_plan {
     pdu::PfftPlan pf0, pf1;
     float2* d_w0;
     float2* d_w1;
+    // a plan of the Toeplitz-embedded normal operator (pdu_toep_plan_create): grid 2 n, no interpolation tables, unit
+    // apodisation tables of k0 / k1 entries; accepted only by the pdu_toep_* entry points
+    bool toep;
 };
 
 namespace pdu {

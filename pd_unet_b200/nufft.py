@@ -6,6 +6,7 @@ the reference reaches the library through its unmounted MRI branch, /root/refere
     KbNufftAdjoint(...)(data, omega, interp_mats=None, smaps=None, norm=None)
     KbInterp(...)(image, omega) / KbInterpAdjoint(...)(data, omega)
     calc_density_compensation_function(ktraj, im_size, num_iterations=10, ...)
+    calc_toeplitz_kernel(omega, im_size, weights=None, norm=None, ...) / ToepNufft()(image, kernel, smaps=None, norm=None)
 
 image: complex64 [B, C, N0, N1]; omega: float32 [2, M] radians (or [B, 2, M]); data: complex64
 [B, C, M].  With smaps [1 or B, coils, N0, N1] the forward expands a one-channel image to the
@@ -26,7 +27,7 @@ import numpy as np
 import torch
 from torch import nn
 
-from ._lib import NUFFT_IMAGE_SPLIT, NUFFT_KDATA_SPLIT, PduError, check, lib, require_cuda, stream_ptr
+from ._lib import NUFFT_IMAGE_SPLIT, NUFFT_KDATA_SPLIT, PDU_EUNSUPPORTED, PduError, check, lib, require_cuda, stream_ptr
 
 
 # ----------------------------------------------------------------------------- tables (host, float64)
@@ -534,3 +535,186 @@ def calc_density_compensation_function(ktraj: torch.Tensor, im_size: Sequence[in
         new = plan.interp(plan.interp_adjoint(w, omega), omega)
         w = w / new.abs()
     return w
+
+
+# ----------------------------------------------------------------------------- Toeplitz-embedded normal operator
+class _ToepPlan:
+    """Owns one Toeplitz pdu_nufft_plan_t (grid 2 N, unit apodisation, no tables) per device for one image size."""
+
+    def __init__(self, im_size: Tuple[int, int]):
+        self.im_size = im_size
+        self._handles: Dict[int, C.c_void_p] = {}
+
+    def handle(self, device: torch.device) -> C.c_void_p:
+        idx = device.index if device.index is not None else torch.cuda.current_device()
+        h = self._handles.get(idx)
+        if h is None:
+            h = C.c_void_p()
+            with torch.cuda.device(idx):
+                rc = lib().pdu_toep_plan_create(C.byref(h), self.im_size[0], self.im_size[1])
+            if rc == PDU_EUNSUPPORTED:
+                raise NotImplementedError(f"no Toeplitz path for a {self.im_size[0]} x {self.im_size[1]} image (the 2 N "
+                                          "embedding grid must factor into 2, 3, 5); there is no CPU fallback")
+            check(rc, "pdu_toep_plan_create")
+            self._handles[idx] = h
+        return h
+
+    def workspace_bytes(self, h, batch: int, coils: int) -> int:
+        """Scratch of one batch chunk: the arithmetic of csrc/nufft.cu::tz_batch_chunk (512 MB, 65535 planes)."""
+        L = lib()
+        per = int(L.pdu_toep_workspace_bytes(h, 1))
+        cb = min(batch, max(1, min((512 << 20) // per, 65535) // coils))
+        return int(L.pdu_toep_workspace_bytes(h, cb * coils))
+
+    def __del__(self):
+        # the same deferred destruction as _Plan: a collection during a CUDA-graph capture must not free device memory
+        try:
+            if not self._handles:
+                return
+            _DEFERRED_DESTROY.extend(self._handles.values())
+            if torch.cuda.is_current_stream_capturing():
+                return
+            while _DEFERRED_DESTROY:
+                lib().pdu_nufft_plan_destroy(_DEFERRED_DESTROY.pop())
+        except Exception:
+            pass
+
+
+_TOEP_PLANS: Dict[Tuple[int, int], _ToepPlan] = {}
+
+
+def _toep_plan(im_size) -> _ToepPlan:
+    key = tuple(int(v) for v in im_size)
+    if len(key) != 2:
+        raise NotImplementedError("only 2-D Toeplitz operators are implemented (radial MRI slices)")
+    tp = _TOEP_PLANS.get(key)
+    if tp is None:
+        tp = _TOEP_PLANS[key] = _ToepPlan(key)
+    return tp
+
+
+def _check_norm(norm: Optional[str]) -> None:
+    if norm not in (None, "ortho"):
+        raise ValueError("norm must be None or 'ortho'")
+
+
+def _toep_apply(image: torch.Tensor, kernel: torch.Tensor, smaps: Optional[torch.Tensor], conj: bool) -> torch.Tensor:
+    image = require_cuda(image, torch.complex64, "image")
+    kernel = require_cuda(kernel, torch.complex64, "kernel")
+    if image.dim() != 4:
+        raise ValueError(f"image must be [B, C, N0, N1], got {tuple(image.shape)}")
+    B, ci, N0, N1 = image.shape
+    if kernel.dim() == 2:
+        kernel = kernel[None]
+    if kernel.dim() != 3 or tuple(kernel.shape[1:]) != (2 * N0, 2 * N1) or kernel.shape[0] not in (1, B):
+        raise ValueError(f"kernel must be [2 N0, 2 N1] = [{2 * N0}, {2 * N1}] or [1 or {B}, {2 * N0}, {2 * N1}] for this image, "
+                         f"got {tuple(kernel.shape)}")
+    coils, sb = ci, 1
+    if smaps is not None:
+        smaps = require_cuda(smaps, torch.complex64, "smaps")
+        if smaps.dim() == 3:
+            smaps = smaps[None]
+        if smaps.dim() != 4 or tuple(smaps.shape[-2:]) != (N0, N1) or smaps.shape[0] not in (1, B):
+            raise ValueError(f"smaps must be [1 or {B}, coils, {N0}, {N1}]")
+        if ci != 1:
+            raise ValueError("with smaps the image must have one channel")
+        coils, sb = smaps.shape[1], smaps.shape[0]
+    out = torch.empty_like(image)
+    if out.numel() == 0:
+        return out
+    with torch.cuda.device(image.device):
+        tp = _toep_plan((N0, N1))
+        h = tp.handle(image.device)
+        L = lib()
+        ws = torch.empty(tp.workspace_bytes(h, B, coils), dtype=torch.uint8, device=image.device)
+        check(L.pdu_toep_apply_c64(h, image.data_ptr(), out.data_ptr(), kernel.data_ptr(), kernel.shape[0],
+                                   smaps.data_ptr() if smaps is not None else None, B, coils, sb, 1 if conj else 0,
+                                   ws.data_ptr(), ws.numel(), stream_ptr()), "pdu_toep_apply_c64")
+    return out
+
+
+class _ToepFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, kernel, smaps):
+        ctx.save_for_backward(kernel, smaps) if smaps is not None else ctx.save_for_backward(kernel)
+        return _toep_apply(x, kernel, smaps, False)
+
+    @staticmethod
+    def backward(ctx, grad):
+        saved = ctx.saved_tensors
+        kernel, smaps = saved[0], (saved[1] if len(saved) > 1 else None)
+        # T = P^T F^-1 diag(k) F P (with coil maps: sum_c S_c^H T S_c), so T^H is the same apply with conj(k): exact for
+        # any complex kernel
+        return _toep_apply(grad.contiguous(), kernel, smaps, True), None, None
+
+
+class ToepNufft(nn.Module):
+    """The NUFFT normal operator A^H W A by Toeplitz embedding.  [RECALL] torchkbnufft.ToepNufft.
+
+    forward(image, kernel, smaps=None, norm=None): image complex64 [B, C, N0, N1]; kernel complex64 [2 N0, 2 N1] or
+    [1 or B, 2 N0, 2 N1] from calc_toeplitz_kernel.  Returns ifft2(kernel * fft2(zero_pad(x)))[..., :N0, :N1] for every
+    channel, or with smaps [1 or B, coils, N0, N1] (image [B, 1, N0, N1]) sum_c conj(S_c) T(S_c x).  No interpolation:
+    the cost does not depend on the trajectory length.
+
+    norm is accepted with torchkbnufft's values and does not change the result [RECALL]: the FFT pair's normalisations
+    multiply to the same total either way, and the NUFFT's scaling lives in the kernel (calc_toeplitz_kernel(norm=...)).
+    Differentiable in the image (the backward is the same apply with the conjugate kernel, exact for any complex
+    kernel); no gradient flows to the kernel.  No parameters, no buffers."""
+
+    def forward(self, image, kernel, smaps=None, norm: Optional[str] = None):
+        _check_norm(norm)
+        return _ToepFn.apply(image, kernel, smaps)
+
+
+def calc_toeplitz_kernel(omega: torch.Tensor, im_size: Sequence[int], weights: Optional[torch.Tensor] = None,
+                         norm: Optional[str] = None, grid_size: Optional[Sequence[int]] = None, numpoints=6,
+                         n_shift: Optional[Sequence[int]] = None, table_oversamp=2 ** 10, kbwidth: float = 2.34,
+                         order=0.0) -> torch.Tensor:
+    """The Toeplitz kernel of A^H W A for trajectory omega [2, M] (or [B, 2, M]: one kernel per trajectory).
+    [RECALL] torchkbnufft.calc_toeplitz_kernel; returns complex64 [2 N0, 2 N1] (or [B, 2 N0, 2 N1]).
+
+    kernel = fft2(p_circ), p[r] = s * sum_m w_m exp(i omega_m . r) for |r| < N in circulant layout; the point-spread
+    function comes from two adjoint NUFFTs of the weights (omega, and omega with its first row negated) at the user's
+    grid_size / numpoints / table, so it carries their Kaiser-Bessel approximation error.  s = 1 / (K0 K1) of the NUFFT
+    grid for norm="ortho", 1 for None.  weights: real, float32 [M] / [1, 1, M] (or [B, 1, M] for a batched omega), or
+    complex64 with a zero imaginary part (what calc_density_compensation_function returns); None means all ones.
+    n_shift is accepted and ignored: the normal operator does not depend on it."""
+    del n_shift
+    _check_norm(norm)
+    im_size = tuple(int(v) for v in im_size)
+    tp = _toep_plan(im_size)
+    omega = require_cuda(omega, torch.float32, "omega")
+    h = tp.handle(omega.device)               # an unsupported size fails here, before any NUFFT work
+    om = omega if omega.dim() == 3 else omega[None]
+    if om.dim() != 3 or om.shape[1] != 2:
+        raise ValueError(f"omega must be [2, M] or [B, 2, M], got {tuple(omega.shape)}")
+    nk, M = om.shape[0], om.shape[2]
+    if weights is None:
+        w = torch.ones((nk, 1, M), dtype=torch.float32, device=omega.device)
+    else:
+        if not isinstance(weights, torch.Tensor) or not weights.is_cuda:
+            raise PduError("weights must be a CUDA tensor (no CPU fallback)")
+        if weights.is_complex():
+            if bool((weights.imag != 0).any()):        # one read-back per kernel build
+                raise ValueError("weights must be real: the kernel's Hermitian assembly assumes p(-r) = conj p(r)")
+            weights = weights.real
+        w = weights.to(torch.float32)
+        if w.numel() == M:
+            w = w.reshape(1, 1, M).expand(nk, 1, M)
+        elif w.numel() == nk * M:
+            w = w.reshape(nk, 1, M)
+        else:
+            raise ValueError(f"weights must have {M} entries (or {nk} x {M} for a batched omega), got {tuple(weights.shape)}")
+    w = torch.complex(w, torch.zeros_like(w)).contiguous()
+    plan = _Plan(im_size, grid_size, numpoints, (0, 0), table_oversamp, kbwidth, float(order if np.isscalar(order) else order[0]))
+    scale = 1.0 / (plan.grid_size[0] * plan.grid_size[1]) if norm == "ortho" else 1.0
+    flip = torch.tensor([-1.0, 1.0], dtype=torch.float32, device=omega.device)[:, None]
+    q1 = _per_trajectory(plan.adjoint, w, omega, None, None).contiguous()
+    q2 = _per_trajectory(plan.adjoint, w, (omega * flip).contiguous(), None, None).contiguous()
+    N0, N1 = im_size
+    kernel = torch.empty((nk, 2 * N0, 2 * N1), dtype=torch.complex64, device=omega.device)
+    with torch.cuda.device(omega.device):
+        ws = torch.empty(nk * 4 * N0 * N1 * 8, dtype=torch.uint8, device=omega.device)
+        check(lib().pdu_toep_kernel_c64(h, q1.data_ptr(), q2.data_ptr(), kernel.data_ptr(), nk, scale, ws.data_ptr(),
+                                        ws.numel(), stream_ptr()), "pdu_toep_kernel_c64")
+    return kernel if omega.dim() == 3 else kernel[0]

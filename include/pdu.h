@@ -70,8 +70,8 @@ PDU_API long pdu_launch_count(int reset);
  * their loads so that the path can be tested. */
 PDU_API int pdu_device_error(int reset);
 /* Name and shape of the kernel the dispatcher of an operator chose in this thread's most recent
- * call: op in {"radon_fwd", "radon_adj", "filter", "nufft_fwd", "nufft_adj", "toep"}; "" before the
- * first call.  The string stays valid until the thread's next call of that operator. */
+ * call: op in {"radon_fwd", "radon_adj", "filter", "nufft_fwd", "nufft_adj", "toep", "cg"}; "" before
+ * the first call.  The string stays valid until the thread's next call of that operator. */
 PDU_API const char* pdu_last_kernel(const char* op);
 
 /* ------------------------------------------------------------------ CT ---- */
@@ -245,6 +245,32 @@ PDU_API int pdu_toep_kernel_c64(pdu_nufft_plan_t* plan, const float* q1, const f
 PDU_API int pdu_toep_apply_c64(pdu_nufft_plan_t* plan, const float* image, float* out, const float* kernel,
                                int kernel_batch, const float* smaps, int batch, int coils, int smaps_batch,
                                int conj_kernel, void* ws, size_t ws_bytes, pdu_stream_t stream);
+
+/* Conjugate gradient on the Toeplitz normal operator: solves (T + lam I) x = b, T = pdu_toep_apply_c64's operator, for
+ * every system at once -- a plane [batch, coils, n0, n1] without smaps; a batch element b [batch, 1, n0, n1] with smaps
+ * [smaps_batch (1 or batch), coils, n0, n1] (CG-SENSE).  kernel / kernel_batch / conj_kernel as pdu_toep_apply_c64
+ * (conj_kernel != 0 solves the adjoint system).  lam: device float32 [lam_count], lam_count 1 or batch (channels of a
+ * batch element share its lam); null means 0.  x0: the warm start, null for zero; it may equal x.  Per system, in
+ * float64 scalars and complex64 vectors:
+ *     r = b - (T + lam) x0 (r = b without x0);  p = r;  rho = ||r||^2;  bb = ||b||^2
+ *     max_iter times:
+ *         q = (T + lam) p;  pi = Re<p, q>
+ *         if frozen or rho == 0 or pi <= 0: freeze (x and r stay as they are from then on)
+ *         alpha = rho / pi;  x += alpha p;  r -= alpha q;  rho' = ||r||^2
+ *         if rho' <= tol^2 bb: freeze
+ *         p = r + (rho' / rho) p;  rho = rho'
+ * tol never ends the call early: every call launches max_iter iterations, reads nothing back and can be captured in
+ * a CUDA graph.  The sums add in a fixed order without atomics: a system's x is bit-identical whatever else is in
+ * the batch and however it is chunked.  Per iteration 5 launches on the fast path (the apply's three, the last with
+ * the lam p term and the Re<p, q> partials fused in, + cg_update_kernel + cg_direction_kernel) and 9 on the generic
+ * one (+ cg_lam_dot_kernel); set-up is cg_init_kernel, after one apply when x0 is given.  pdu_last_kernel("cg").
+ * PDU_EINVAL for a Kaiser-Bessel plan, max_iter < 0, tol < 0, a bad lam_count or a workspace shorter than
+ * pdu_toep_cg_workspace_bytes (the Toeplitz scratch, r, p and q and the partial sums of one batch chunk). */
+PDU_API size_t pdu_toep_cg_workspace_bytes(const pdu_nufft_plan_t* plan, int batch, int coils, int has_smaps);
+PDU_API int pdu_toep_cg_c64(pdu_nufft_plan_t* plan, const float* b, const float* x0, float* x, const float* kernel,
+                            int kernel_batch, const float* smaps, int batch, int coils, int smaps_batch, const float* lam,
+                            int lam_count, int max_iter, float tol, int conj_kernel, void* ws, size_t ws_bytes,
+                            pdu_stream_t stream);
 
 /* The layout change on its own, for the generic (complex64) entry points: split [planes, 2, n] float32 <-> complex64
  * [planes, n]; `weight` (nullable, float32 [n]) multiplies element e of every plane (the density compensation). */

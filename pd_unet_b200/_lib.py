@@ -73,6 +73,9 @@ SIGNATURES = {
     "pdu_toep_workspace_bytes": (C.c_size_t, [_p, C.c_int]),
     "pdu_toep_kernel_c64": (C.c_int, [_p, _p, _p, _p, C.c_int, C.c_float, _p, C.c_size_t, _p]),
     "pdu_toep_apply_c64": (C.c_int, [_p, _p, _p, _p, C.c_int, _p, C.c_int, C.c_int, C.c_int, C.c_int, _p, C.c_size_t, _p]),
+    "pdu_toep_cg_workspace_bytes": (C.c_size_t, [_p, C.c_int, C.c_int, C.c_int]),
+    "pdu_toep_cg_c64": (C.c_int, [_p, _p, _p, _p, _p, C.c_int, _p, C.c_int, C.c_int, C.c_int, _p, C.c_int, C.c_int, C.c_float,
+                                  C.c_int, _p, C.c_size_t, _p]),
     "pdu_complex_from_split_f32": (C.c_int, [_p, _p, _p, C.c_long, C.c_long, _p]),
     "pdu_split_from_complex_f32": (C.c_int, [_p, _p, C.c_long, C.c_long, _p]),
     "pdu_nufft_csr_build": (C.c_int, [_p, _p, C.c_long, _p, C.c_size_t, _p]),

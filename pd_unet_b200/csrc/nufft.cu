@@ -24,6 +24,7 @@
 #include <math.h>
 
 #include <algorithm>
+#include <initializer_list>
 #include <map>
 #include <mutex>
 #include <vector>
@@ -1157,13 +1158,40 @@ __global__ void __launch_bounds__(SEQ* FastFft<K>::TPS)
     }
 }
 
+// The conjugate-gradient epilogue of an apply (pdu_toep_cg_c64): q = T p + lam p and, per CTA, the float64 partial of
+// Re<p, q> in the slot part[system * gridDim.x + blockIdx.x].  A system is a plane, or a batch element with coil maps;
+// its lam is lam[system / lam_div] (lam_div 0: lam[0]; lam null: 0).
+struct TzCg {
+    const float2* p;          // the apply's input, laid out as its output
+    const float* lam;
+    int lam_div;
+    double* part;
+};
+
+__device__ __forceinline__ float cg_lam(const float* lam, int lam_div, int sys) {
+    return lam ? __ldg(lam + (lam_div ? sys / lam_div : 0)) : 0.f;
+}
+
+// sum of one double per thread over the CTA in a fixed order: a shuffle tree in each warp, then the warps in index
+// order; the result is valid in thread 0 (blockDim.x a multiple of 32, `red` 32 doubles of shared memory)
+__device__ __forceinline__ double cg_block_sum(double v, double* red) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+    __syncthreads();
+    double s = 0.0;
+    if (threadIdx.x == 0)
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += red[w];
+    return s;
+}
+
 // fast path, pass 3: SEQ rows of one output plane per CTA: pruned inverse row FFT of T's N rows (first N outputs),
 // x scale; with coil maps the CTA walks the batch element's coils in a fixed order and sums conj(S_c) T_c in registers
-// (bit-reproducible; no cropped intermediate, no crop_apod_kernel pass)
-template <int K, int SEQ>
+// (bit-reproducible; no cropped intermediate, no crop_apod_kernel pass).  CG: the TzCg epilogue at the output store.
+template <int K, int SEQ, bool CG = false>
 __global__ void __launch_bounds__(SEQ* FastFft<K>::TPS)
     tz_rows_out_kernel(const float2* __restrict__ T, const float2* __restrict__ smaps, float2* __restrict__ out,
-                       const float2* __restrict__ tw_g, int coils, int smaps_batch, float scale) {
+                       const float2* __restrict__ tw_g, int coils, int smaps_batch, float scale, TzCg cg) {
     using F = FastFft<K>;
     constexpr int N = K / 2, TPS = F::TPS, NS3 = F::NS3, R3 = F::R3;
     constexpr int PER = TPS >= NS3 ? 1 : NS3 / TPS;     // last-pass butterflies per thread (ff_transform)
@@ -1201,15 +1229,260 @@ __global__ void __launch_bounds__(SEQ* FastFft<K>::TPS)
         ff_transform<K, 4, true, false, true, false, false, true>(buf + s * F::template pitch<4>(), tw, t, ld, st);
         __syncthreads();                                 // the next coil's pass-1 stores reuse the buffer
     }
-    if (!live) return;
-    float2* dst = out + ((long)q * N + row) * N;
+    if constexpr (!CG) {
+        if (!live) return;
+        float2* dst = out + ((long)q * N + row) * N;
 #pragma unroll
-    for (int i = 0; i < PER; ++i) {
-        const int j = t + i * TPS;
-        if (j < NS3) {
+        for (int i = 0; i < PER; ++i) {
+            const int j = t + i * TPS;
+            if (j < NS3) {
 #pragma unroll
-            for (int r = 0; r < R3 / 2; ++r) dst[j + r * NS3] = make_float2(acc[i][r].x * scale, acc[i][r].y * scale);
+                for (int r = 0; r < R3 / 2; ++r) dst[j + r * NS3] = make_float2(acc[i][r].x * scale, acc[i][r].y * scale);
+            }
         }
+    } else {
+        __shared__ double red[32];
+        const float lam = cg_lam(cg.lam, cg.lam_div, q);
+        double dot = 0.0;
+        if (live) {
+            float2* dst = out + ((long)q * N + row) * N;
+            const float2* src = cg.p + ((long)q * N + row) * N;
+#pragma unroll
+            for (int i = 0; i < PER; ++i) {
+                const int j = t + i * TPS;
+                if (j < NS3) {
+#pragma unroll
+                    for (int r = 0; r < R3 / 2; ++r) {
+                        const float2 pv = __ldg(src + j + r * NS3);
+                        const float2 v = make_float2(fmaf(lam, pv.x, acc[i][r].x * scale), fmaf(lam, pv.y, acc[i][r].y * scale));
+                        dst[j + r * NS3] = v;
+                        dot = fma((double)pv.x, (double)v.x, dot);
+                        dot = fma((double)pv.y, (double)v.y, dot);
+                    }
+                }
+            }
+        }
+        dot = cg_block_sum(dot, red);
+        if (tid == 0) cg.part[(long)q * gridDim.x + blockIdx.x] = dot;
+    }
+}
+
+// ------------------------------------------------------------------ conjugate gradient on T + lam I (pdu_toep_cg_c64)
+// Per system (a plane, or a batch element with coil maps), every launch does the same work whatever the data: the
+// scalars live on the device, a frozen system's kernels return early, and nothing is read back to the host.  Each CTA
+// of the vector kernels first sums its system's partial slots in a fixed order, derives the same alpha / beta / freeze
+// decision as every other CTA of the system, does its share of the vector work and writes its own partial of the next
+// reduction.  No atomics: a system's result is bit-identical whatever else is in the batch.
+constexpr int CG_THREADS = 256;
+
+// CTAs per system of the vector kernels, and slots of their partial sums: a function of the system size alone, so that
+// a system's sums add in the same order however the batch is made up or chunked
+static int cg_ctas(long n) { return (int)std::min(std::max(cdiv(cdiv(n, 2), 2 * CG_THREADS), 1L), 256L); }
+
+// 16-byte accesses when n is even and every vector of the call is 16-byte aligned; the element pairs, and so the
+// order of every sum, are the same either way
+static int cg_v4(long n, std::initializer_list<const void*> ptrs) {
+    if (n & 1) return 0;
+    for (const void* q : ptrs)
+        if (q && ((uintptr_t)q & 15)) return 0;
+    return 1;
+}
+
+// element pair k of a system's vector: elements 2 k and 2 k + 1 (zero past the end of an odd n)
+__device__ __forceinline__ void cg_ld(const float2* v, long k, long n, int v4, float2& a, float2& b) {
+    if (v4) {
+        const float4 t = reinterpret_cast<const float4*>(v)[k];
+        a = make_float2(t.x, t.y);
+        b = make_float2(t.z, t.w);
+    } else {
+        a = v[2 * k];
+        b = 2 * k + 1 < n ? v[2 * k + 1] : make_float2(0.f, 0.f);
+    }
+}
+__device__ __forceinline__ void cg_st(float2* v, long k, long n, int v4, float2 a, float2 b) {
+    if (v4) {
+        reinterpret_cast<float4*>(v)[k] = make_float4(a.x, a.y, b.x, b.y);
+    } else {
+        v[2 * k] = a;
+        if (2 * k + 1 < n) v[2 * k + 1] = b;
+    }
+}
+// acc + Re(conj(a) b), in float64
+__device__ __forceinline__ double cg_dot(double acc, float2 a, float2 b) {
+    return fma((double)a.y, (double)b.y, fma((double)a.x, (double)b.x, acc));
+}
+__device__ __forceinline__ float2 cg_axpy(float a, float2 x, float2 y) { return make_float2(fmaf(a, x.x, y.x), fmaf(a, x.y, y.y)); }
+
+// a system's `count` partial slots (written by an earlier kernel) summed in a fixed order by one warp: lane l adds
+// slots l, l + 32, ..., then a shuffle tree; every lane gets the result
+__device__ __forceinline__ double cg_slots(const double* s, int count) {
+    double v = 0.0;
+    for (int i = threadIdx.x & 31; i < count; i += 32) v += __ldcg(s + i);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+    return __shfl_sync(0xffffffffu, v, 0);
+}
+
+// the iteration runs for a system that is not frozen, has rho != 0 and a positive curvature pi = Re<p, (T + lam) p>
+__device__ __forceinline__ bool cg_runs(int frozen, double rho, double pi) { return !frozen && rho != 0.0 && pi > 0.0; }
+
+// generic path: q += lam p on the apply's cropped output, and per-CTA partials of Re<p, q> (the fast path does this in
+// tz_rows_out_kernel's epilogue).  Grid (cg_ctas(n), systems).
+__global__ void __launch_bounds__(CG_THREADS)
+    cg_lam_dot_kernel(float2* __restrict__ q, const float2* __restrict__ p, const float* __restrict__ lam, int lam_div,
+                      double* __restrict__ part, long n, int v4) {
+    __shared__ double red[32];
+    const int sys = blockIdx.y;
+    const long base = (long)sys * n, pairs = (n + 1) / 2;
+    const float l = cg_lam(lam, lam_div, sys);
+    double dot = 0.0;
+    for (long k = (long)blockIdx.x * CG_THREADS + threadIdx.x; k < pairs; k += (long)gridDim.x * CG_THREADS) {
+        float2 p0, p1, q0, q1;
+        cg_ld(p + base, k, n, v4, p0, p1);
+        cg_ld(q + base, k, n, v4, q0, q1);
+        q0 = cg_axpy(l, p0, q0);
+        q1 = cg_axpy(l, p1, q1);
+        cg_st(q + base, k, n, v4, q0, q1);
+        dot = cg_dot(cg_dot(dot, p0, q0), p1, q1);
+    }
+    dot = cg_block_sum(dot, red);
+    if (threadIdx.x == 0) part[(long)sys * gridDim.x + blockIdx.x] = dot;
+}
+
+// set-up: x = x0 (zero when x0 is null; untouched when x0 == x), r = b - q (q = (T + lam) x0; r = b when q is null),
+// p = r, and per-CTA partials of ||r||^2 and ||b||^2.  Grid (cg_ctas(n), systems).
+__global__ void __launch_bounds__(CG_THREADS)
+    cg_init_kernel(const float2* __restrict__ b, const float2* x0, float2* x, const float2* __restrict__ q, float2* __restrict__ r,
+                   float2* __restrict__ p, double* __restrict__ rr_part, double* __restrict__ bb_part, long n, int v4) {
+    __shared__ double red[2][32];
+    const int sys = blockIdx.y;
+    const long base = (long)sys * n, pairs = (n + 1) / 2;
+    double rr = 0.0, bb = 0.0;
+    for (long k = (long)blockIdx.x * CG_THREADS + threadIdx.x; k < pairs; k += (long)gridDim.x * CG_THREADS) {
+        float2 b0, b1, r0, r1;
+        cg_ld(b + base, k, n, v4, b0, b1);
+        if (x0 != x) {
+            float2 x00 = make_float2(0.f, 0.f), x01 = x00;
+            if (x0) cg_ld(x0 + base, k, n, v4, x00, x01);
+            cg_st(x + base, k, n, v4, x00, x01);
+        }
+        r0 = b0;
+        r1 = b1;
+        if (q) {
+            float2 q0, q1;
+            cg_ld(q + base, k, n, v4, q0, q1);
+            r0 = make_float2(b0.x - q0.x, b0.y - q0.y);
+            r1 = make_float2(b1.x - q1.x, b1.y - q1.y);
+        }
+        cg_st(r + base, k, n, v4, r0, r1);
+        cg_st(p + base, k, n, v4, r0, r1);
+        rr = cg_dot(cg_dot(rr, r0, r0), r1, r1);
+        bb = cg_dot(cg_dot(bb, b0, b0), b1, b1);
+    }
+    rr = cg_block_sum(rr, red[0]);
+    bb = cg_block_sum(bb, red[1]);
+    if (threadIdx.x == 0) {
+        rr_part[(long)sys * gridDim.x + blockIdx.x] = rr;
+        bb_part[(long)sys * gridDim.x + blockIdx.x] = bb;
+    }
+}
+
+// the scalars of one iteration, by warp 0 of every CTA of a system: pi from the apply's slots; rho and the frozen flag
+// from the previous iteration's direction kernel, or on the first iteration (rr_first non-null) rho from the set-up's
+// slots with the flag clear
+__device__ __forceinline__ void cg_scalars(int sys, const double* pi_part, int pi_slots, const double* rr_first,
+                                           const double* rho_in, const int* frz_in, double& pi, double& rho, int& frozen) {
+    pi = cg_slots(pi_part + (long)sys * pi_slots, pi_slots);
+    rho = rr_first ? cg_slots(rr_first + (long)sys * gridDim.x, gridDim.x) : __ldcg(rho_in + sys);
+    frozen = rr_first ? 0 : __ldcg(frz_in + sys);
+}
+
+// x += alpha p, r -= alpha q with alpha = rho / pi, and per-CTA partials of the new ||r||^2 (rr_out); a system whose
+// iteration does not run (cg_runs) is left as it is.  Grid (cg_ctas(n), systems).
+__global__ void __launch_bounds__(CG_THREADS)
+    cg_update_kernel(float2* __restrict__ x, float2* __restrict__ r, const float2* __restrict__ p, const float2* __restrict__ q,
+                     const double* __restrict__ pi_part, int pi_slots, const double* __restrict__ rr_first,
+                     const double* __restrict__ rho_in, const int* __restrict__ frz_in, double* __restrict__ rr_out, long n,
+                     int v4) {
+    __shared__ double red[32];
+    __shared__ double s_alpha;
+    __shared__ int s_run;
+    const int sys = blockIdx.y;
+    if (threadIdx.x < 32) {
+        double pi, rho;
+        int frozen;
+        cg_scalars(sys, pi_part, pi_slots, rr_first, rho_in, frz_in, pi, rho, frozen);
+        if (threadIdx.x == 0) {
+            s_run = cg_runs(frozen, rho, pi);
+            s_alpha = s_run ? rho / pi : 0.0;
+        }
+    }
+    __syncthreads();
+    if (!s_run) return;                                  // uniform over the CTA
+    const float a = (float)s_alpha;
+    const long base = (long)sys * n, pairs = (n + 1) / 2;
+    double rr = 0.0;
+    for (long k = (long)blockIdx.x * CG_THREADS + threadIdx.x; k < pairs; k += (long)gridDim.x * CG_THREADS) {
+        float2 x0, x1, r0, r1, p0, p1, q0, q1;
+        cg_ld(p + base, k, n, v4, p0, p1);
+        cg_ld(q + base, k, n, v4, q0, q1);
+        cg_ld(x + base, k, n, v4, x0, x1);
+        cg_ld(r + base, k, n, v4, r0, r1);
+        cg_st(x + base, k, n, v4, cg_axpy(a, p0, x0), cg_axpy(a, p1, x1));
+        r0 = cg_axpy(-a, q0, r0);
+        r1 = cg_axpy(-a, q1, r1);
+        cg_st(r + base, k, n, v4, r0, r1);
+        rr = cg_dot(cg_dot(rr, r0, r0), r1, r1);
+    }
+    rr = cg_block_sum(rr, red);
+    if (threadIdx.x == 0) rr_out[(long)sys * gridDim.x + blockIdx.x] = rr;
+}
+
+// p = r + beta p with beta = rho' / rho, rho' the sum of cg_update_kernel's partials (rr_new).  The system freezes
+// instead when this iteration's update did not run (the same decision from the same slots) or rho' <= tol^2 ||b||^2.
+// CTA 0 writes rho and the flag of the next iteration (rho_out / frz_out: the other parity's buffers, which no CTA of
+// this launch reads) and, on the first iteration, ||b||^2 (bb_io, read on the later ones).  Grid (cg_ctas(n), systems).
+__global__ void __launch_bounds__(CG_THREADS)
+    cg_direction_kernel(float2* __restrict__ p, const float2* __restrict__ r, const double* __restrict__ pi_part, int pi_slots,
+                        const double* __restrict__ rr_first, const double* __restrict__ bb_first, const double* __restrict__ rho_in,
+                        const int* __restrict__ frz_in, double* bb_io, const double* __restrict__ rr_new,
+                        double* __restrict__ rho_out, int* __restrict__ frz_out, double tol2, long n, int v4) {
+    __shared__ double s_beta;
+    __shared__ int s_frozen;
+    const int sys = blockIdx.y;
+    if (threadIdx.x < 32) {
+        double pi, rho;
+        int frozen;
+        cg_scalars(sys, pi_part, pi_slots, rr_first, rho_in, frz_in, pi, rho, frozen);
+        const double bb = rr_first ? cg_slots(bb_first + (long)sys * gridDim.x, gridDim.x) : __ldcg(bb_io + sys);
+        double rho_next = rho, beta = 0.0;
+        int frozen_next = 1;
+        if (cg_runs(frozen, rho, pi)) {
+            rho_next = cg_slots(rr_new + (long)sys * gridDim.x, gridDim.x);
+            if (!(rho_next <= tol2 * bb)) {
+                frozen_next = 0;
+                beta = rho_next / rho;
+            }
+        }
+        if (threadIdx.x == 0) {
+            s_beta = beta;
+            s_frozen = frozen_next;
+            if (blockIdx.x == 0) {
+                rho_out[sys] = rho_next;
+                frz_out[sys] = frozen_next;
+                if (rr_first) bb_io[sys] = bb;
+            }
+        }
+    }
+    __syncthreads();
+    if (s_frozen) return;                                // uniform over the CTA
+    const float be = (float)s_beta;
+    const long base = (long)sys * n, pairs = (n + 1) / 2;
+    for (long k = (long)blockIdx.x * CG_THREADS + threadIdx.x; k < pairs; k += (long)gridDim.x * CG_THREADS) {
+        float2 r0, r1, p0, p1;
+        cg_ld(r + base, k, n, v4, r0, r1);
+        cg_ld(p + base, k, n, v4, p0, p1);
+        cg_st(p + base, k, n, v4, cg_axpy(be, p0, r0), cg_axpy(be, p1, r1));
     }
 }
 
@@ -1236,14 +1509,17 @@ constexpr int TZ_SEQ_ROWS = 4;
 template <int K>
 static constexpr int tz_seq_rows_out() { return K == 2048 ? 2 : TZ_SEQ_ROWS; }
 
+// cg: the conjugate-gradient epilogue (tz_rows_out_kernel<K, SO, true>), or null for the plain apply
 template <int K>
 static int tz_apply_fast(pdu_nufft_plan* p, const float2* image, float2* out, const float2* kern, int kernel_batch,
-                         const float2* smaps, int batch, int coils, int smaps_batch, int conj, float2* T, cudaStream_t st) {
+                         const float2* smaps, int batch, int coils, int smaps_batch, int conj, float2* T, const TzCg* cg,
+                         cudaStream_t st) {
     constexpr int N = K / 2, SC = ff_seq_cols<K>(), SO = tz_seq_rows_out<K>();
     const int planes = batch * coils;
     PDU_CUDA((ensure_dyn_smem<ff_rows_fwd_kernel<K, FF_SEQ_ROWS>>((int)ff_smem_bytes<K>(FF_SEQ_ROWS))));
     PDU_CUDA((ensure_dyn_smem<tz_cols_kernel<K, SC>>((int)ff_smem_bytes<K>(SC))));
-    PDU_CUDA((ensure_dyn_smem<tz_rows_out_kernel<K, SO>>((int)ff_smem_bytes<K>(SO))));
+    if (cg) PDU_CUDA((ensure_dyn_smem<tz_rows_out_kernel<K, SO, true>>((int)ff_smem_bytes<K>(SO))));
+    else PDU_CUDA((ensure_dyn_smem<tz_rows_out_kernel<K, SO>>((int)ff_smem_bytes<K>(SO))));
     ff_rows_fwd_kernel<K, FF_SEQ_ROWS><<<dim3((unsigned)cdiv(N, FF_SEQ_ROWS), (unsigned)planes), FF_SEQ_ROWS * FastFft<K>::TPS,
                                          ff_smem_bytes<K>(FF_SEQ_ROWS), st>>>(image, smaps, T, p->d_s0, p->d_s1, p->d_w1,
                                                                               dims_of(p), coils, smaps_batch);
@@ -1252,8 +1528,18 @@ static int tz_apply_fast(pdu_nufft_plan* p, const float2* image, float2* out, co
         T, kern, p->d_w0, coils, kernel_batch, conj);
     PDU_LAUNCHED();
     const int out_planes = smaps ? batch : planes;
-    tz_rows_out_kernel<K, SO><<<dim3((unsigned)cdiv(N, SO), (unsigned)out_planes), SO * FastFft<K>::TPS, ff_smem_bytes<K>(SO),
-                                 st>>>(T, smaps, out, p->d_w1, coils, smaps_batch, 1.f / ((float)K * (float)K));
+    const dim3 grid_out((unsigned)cdiv(N, SO), (unsigned)out_planes);
+    const float scale = 1.f / ((float)K * (float)K);
+    if (cg) {
+        tz_rows_out_kernel<K, SO, true><<<grid_out, SO * FastFft<K>::TPS, ff_smem_bytes<K>(SO), st>>>(
+            T, smaps, out, p->d_w1, coils, smaps_batch, scale, *cg);
+        PDU_LAUNCHED();
+        note_kernel(OP_CG, "ff_rows_fwd_kernel<%d,%d> + tz_cols_kernel<%d,%d> + tz_rows_out_kernel<%d,%d,cg> + cg_update_kernel + "
+                    "cg_direction_kernel (fast path, %d systems of %dx%d)", K, FF_SEQ_ROWS, K, SC, K, SO, out_planes, N, N);
+        return PDU_OK;
+    }
+    tz_rows_out_kernel<K, SO><<<grid_out, SO * FastFft<K>::TPS, ff_smem_bytes<K>(SO), st>>>(T, smaps, out, p->d_w1, coils,
+                                                                                            smaps_batch, scale, TzCg{});
     PDU_LAUNCHED();
     note_kernel(OP_TOEP, "ff_rows_fwd_kernel<%d,%d> + tz_cols_kernel<%d,%d> + tz_rows_out_kernel<%d,%d> (fast path, %d planes of %dx%d)",
                 K, FF_SEQ_ROWS, K, SC, K, SO, planes, N, N);
@@ -1265,7 +1551,8 @@ static bool tz_cols_seq8(const pdu_nufft_plan* p) { return pf_smem_bytes(PF_SEQ_
 
 template <int SC>
 static int tz_apply_generic(pdu_nufft_plan* p, const float2* image, float2* out, const float2* kern, int kernel_batch,
-                            const float2* smaps, int batch, int coils, int smaps_batch, int conj, float2* ws, cudaStream_t st) {
+                            const float2* smaps, int batch, int coils, int smaps_batch, int conj, float2* ws, const TzCg* cg,
+                            cudaStream_t st) {
     const int planes = batch * coils;
     const long cells = (long)p->k0 * p->k1;
     float2* grid = ws;
@@ -1296,6 +1583,16 @@ static int tz_apply_generic(pdu_nufft_plan* p, const float2* image, float2* out,
     const int out_planes = smaps ? batch : planes;
     rc = launch_crop_apod(p, U, smaps, out, out_planes, coils, smaps_batch, 1.f / ((float)p->k0 * (float)p->k1), 0, st);
     if (rc) return rc;
+    if (cg) {
+        const long n = (long)p->n0 * p->n1;
+        cg_lam_dot_kernel<<<dim3((unsigned)cg_ctas(n), (unsigned)out_planes), CG_THREADS, 0, st>>>(out, cg->p, cg->lam, cg->lam_div,
+                                                                                                  cg->part, n, cg_v4(n, {(const void*)out, (const void*)cg->p}));
+        PDU_LAUNCHED();
+        note_kernel(OP_CG, "pfft_rows_fwd_kernel<%d> + pfft_cols_fwd_kernel<%d> + tz_mul_kernel + pfft_rows_adj_kernel<%d> + "
+                    "pfft_cols_adj_kernel<%d> + crop_apod_kernel + cg_lam_dot_kernel + cg_update_kernel + cg_direction_kernel "
+                    "(generic path, %d systems of %dx%d)", PF_SEQ_ROWS, SC, PF_SEQ_ROWS, SC, out_planes, p->n0, p->n1);
+        return PDU_OK;
+    }
     note_kernel(OP_TOEP, "pfft_rows_fwd_kernel<%d> + pfft_cols_fwd_kernel<%d> + tz_mul_kernel + pfft_rows_adj_kernel<%d> + "
                 "pfft_cols_adj_kernel<%d> + crop_apod_kernel (generic path, %d planes of %dx%d)",
                 PF_SEQ_ROWS, SC, PF_SEQ_ROWS, SC, planes, p->n0, p->n1);
@@ -1303,19 +1600,20 @@ static int tz_apply_generic(pdu_nufft_plan* p, const float2* image, float2* out,
 }
 
 static int tz_apply_chunk(pdu_nufft_plan* p, const float2* image, float2* out, const float2* kern, int kernel_batch,
-                          const float2* smaps, int batch, int coils, int smaps_batch, int conj, float2* ws, cudaStream_t st) {
+                          const float2* smaps, int batch, int coils, int smaps_batch, int conj, float2* ws, cudaStream_t st,
+                          const TzCg* cg = nullptr) {
     if (tz_fast(p)) {
         switch (p->k0) {
-            case 256: return tz_apply_fast<256>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, st);
-            case 512: return tz_apply_fast<512>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, st);
-            case 640: return tz_apply_fast<640>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, st);
-            case 1024: return tz_apply_fast<1024>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, st);
-            default: return tz_apply_fast<2048>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, st);
+            case 256: return tz_apply_fast<256>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st);
+            case 512: return tz_apply_fast<512>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st);
+            case 640: return tz_apply_fast<640>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st);
+            case 1024: return tz_apply_fast<1024>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st);
+            default: return tz_apply_fast<2048>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st);
         }
     }
     if (tz_cols_seq8(p))
-        return tz_apply_generic<PF_SEQ_COLS>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, st);
-    return tz_apply_generic<2>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, st);
+        return tz_apply_generic<PF_SEQ_COLS>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st);
+    return tz_apply_generic<2>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st);
 }
 
 // kernel build, step 4: the full (unpruned) 2-D FFT of p_circ, in place in `kern` with T as the intermediate
@@ -1334,6 +1632,82 @@ static int tz_kernel_fft(pdu_nufft_plan* p, float2* kern, float2* T, int kernels
     pfft_cols_fwd_kernel<SC><<<dim3((unsigned)cdiv(p->k1, SC), (unsigned)kernels), 256, pf_smem_bytes(SC, p->k0), st>>>(
         T, kern, p->d_w0, p->pf0, d, pfft_pitch(p->k0));
     PDU_LAUNCHED();
+    return PDU_OK;
+}
+
+// ------------------------------------------------------------------ pdu_toep_cg_c64: the solve's workspace and loop
+// slots of the Re<p, q> partials per system: tz_rows_out_kernel's CTAs per plane on the fast path (its SEQ is
+// tz_seq_rows_out), cg_lam_dot_kernel's on the generic one
+static int cg_pi_slots(const pdu_nufft_plan* p) {
+    if (tz_fast(p)) return (int)cdiv(p->n0, p->k0 == 2048 ? tz_seq_rows_out<2048>() : tz_seq_rows_out<256>());
+    return cg_ctas((long)p->n0 * p->n1);
+}
+
+// one chunk of cb batch elements: the apply's scratch; r, p, q; the partial slots of Re<p, q>, of ||r||^2 (two sets,
+// by iteration parity) and of ||b||^2; rho and the frozen flag by parity; ||b||^2
+struct CgWs {
+    float2 *tz, *r, *p, *q;
+    double *pi, *rr[2], *bb, *rho[2], *bbv;
+    int* frz[2];
+    size_t bytes;
+};
+
+static CgWs cg_layout(const pdu_nufft_plan* p, int cb, int coils, bool has_smaps, void* base) {
+    const size_t S = (size_t)cb * (has_smaps ? 1 : coils), n = (size_t)p->n0 * p->n1;
+    const size_t G = (size_t)cg_ctas((long)n), GP = (size_t)cg_pi_slots(p);
+    size_t off = 0;
+    auto take = [&](size_t bytes) {
+        void* q = (void*)((uintptr_t)base + off);
+        off += align256(bytes);
+        return q;
+    };
+    CgWs w;
+    w.tz = (float2*)take((size_t)cb * coils * tz_plane_bytes(p));
+    w.r = (float2*)take(S * n * sizeof(float2));
+    w.p = (float2*)take(S * n * sizeof(float2));
+    w.q = (float2*)take(S * n * sizeof(float2));
+    w.pi = (double*)take(S * GP * sizeof(double));
+    for (int e = 0; e < 2; ++e) w.rr[e] = (double*)take(S * G * sizeof(double));
+    w.bb = (double*)take(S * G * sizeof(double));
+    for (int e = 0; e < 2; ++e) w.rho[e] = (double*)take(S * sizeof(double));
+    w.bbv = (double*)take(S * sizeof(double));
+    for (int e = 0; e < 2; ++e) w.frz[e] = (int*)take(S * sizeof(int));
+    w.bytes = off;
+    return w;
+}
+
+// the whole solve of one chunk (nb batch elements): [x0: one apply] + cg_init_kernel, then per iteration the apply with
+// the CG epilogue, cg_update_kernel and cg_direction_kernel -- 5 launches on the fast path, 9 on the generic one
+static int tz_cg_chunk(pdu_nufft_plan* p, const float2* b, const float2* x0, float2* x, const float2* kern, int kernel_batch,
+                       const float2* smaps, int nb, int coils, int smaps_batch, const float* lam, int lam_div, int max_iter,
+                       double tol2, int conj, const CgWs& w, cudaStream_t st) {
+    const int S = smaps ? nb : nb * coils, G = cg_ctas((long)p->n0 * p->n1), GP = cg_pi_slots(p);
+    const long n = (long)p->n0 * p->n1;
+    const dim3 grid((unsigned)G, (unsigned)S);
+    const int v4 = cg_v4(n, {(const void*)b, (const void*)x0, (const void*)x, (const void*)w.r, (const void*)w.p, (const void*)w.q});
+    TzCg cg{x0, lam, lam_div, w.pi};
+    const float2* q0 = nullptr;
+    if (x0 && max_iter > 0) {                            // q = (T + lam) x0 for r = b - q
+        int rc = tz_apply_chunk(p, x0, w.q, kern, kernel_batch, smaps, nb, coils, smaps_batch, conj, w.tz, st, &cg);
+        if (rc) return rc;
+        q0 = w.q;
+    }
+    cg_init_kernel<<<grid, CG_THREADS, 0, st>>>(b, x0, x, q0, w.r, w.p, w.rr[0], w.bb, n, v4);
+    PDU_LAUNCHED();
+    cg.p = w.p;
+    for (int it = 0; it < max_iter; ++it) {
+        const int e = it & 1;
+        const double* first = it == 0 ? w.rr[0] : nullptr;
+        int rc = tz_apply_chunk(p, w.p, w.q, kern, kernel_batch, smaps, nb, coils, smaps_batch, conj, w.tz, st, &cg);
+        if (rc) return rc;
+        cg_update_kernel<<<grid, CG_THREADS, 0, st>>>(x, w.r, w.p, w.q, w.pi, GP, first, w.rho[e], w.frz[e], w.rr[e ^ 1], n, v4);
+        PDU_LAUNCHED();
+        cg_direction_kernel<<<grid, CG_THREADS, 0, st>>>(w.p, w.r, w.pi, GP, first, w.bb, w.rho[e], w.frz[e], w.bbv, w.rr[e ^ 1],
+                                                         w.rho[e ^ 1], w.frz[e ^ 1], tol2, n, v4);
+        PDU_LAUNCHED();
+    }
+    if (max_iter == 0)
+        note_kernel(OP_CG, "cg_init_kernel only (max_iter 0, %d systems of %dx%d)", S, p->n0, p->n1);
     return PDU_OK;
 }
 
@@ -1836,6 +2210,47 @@ int pdu_toep_apply_c64(pdu_nufft_plan_t* p, const float* image, float* out, cons
                                 (const float2*)kernel + (kernel_batch == 1 ? 0 : b0 * cells), kernel_batch == 1 ? 1 : nb,
                                 smaps ? (const float2*)smaps + b0 * smap_b : nullptr, nb, coils, smaps_batch == 1 ? 1 : nb,
                                 conj_kernel ? 1 : 0, (float2*)ws, (cudaStream_t)stream);
+        if (rc) return rc;
+    }
+    return PDU_OK;
+}
+
+size_t pdu_toep_cg_workspace_bytes(const pdu_nufft_plan_t* p, int batch, int coils, int has_smaps) {
+    if (!p || !p->toep || batch <= 0 || coils <= 0 || coils > 65535) return 0;
+    return cg_layout(p, tz_batch_chunk(p, batch, coils), coils, has_smaps != 0, nullptr).bytes;
+}
+
+int pdu_toep_cg_c64(pdu_nufft_plan_t* p, const float* b, const float* x0, float* x, const float* kernel, int kernel_batch,
+                    const float* smaps, int batch, int coils, int smaps_batch, const float* lam, int lam_count, int max_iter,
+                    float tol, int conj_kernel, void* ws, size_t ws_bytes, pdu_stream_t stream) {
+    PDU_REQUIRE(p != nullptr, "pdu_toep_cg_c64: plan is null");
+    PDU_REQUIRE(p->toep, "pdu_toep_cg_c64: not a Toeplitz plan (use pdu_toep_plan_create)");
+    PDU_REQUIRE(b && x && kernel, "pdu_toep_cg_c64: null pointer");
+    PDU_REQUIRE(batch > 0 && coils > 0 && coils <= 65535, "pdu_toep_cg_c64: batch must be > 0 and coils in 1..65535");
+    PDU_REQUIRE(kernel_batch == 1 || kernel_batch == batch, "pdu_toep_cg_c64: kernel batch must be 1 or batch");
+    if (smaps) PDU_REQUIRE(smaps_batch == 1 || smaps_batch == batch, "pdu_toep_cg_c64: smaps batch must be 1 or batch");
+    PDU_REQUIRE(lam_count == 1 || lam_count == batch, "pdu_toep_cg_c64: lam_count must be 1 or batch (got %d)", lam_count);
+    PDU_REQUIRE(max_iter >= 0, "pdu_toep_cg_c64: max_iter must be >= 0 (got %d)", max_iter);
+    PDU_REQUIRE(tol >= 0.f, "pdu_toep_cg_c64: tol must be >= 0");
+    const int cb = tz_batch_chunk(p, batch, coils);
+    const CgWs w = cg_layout(p, cb, coils, smaps != nullptr, ws);
+    PDU_REQUIRE(ws && ws_bytes >= w.bytes, "pdu_toep_cg_c64: workspace of %zu bytes required, got %zu", w.bytes,
+                ws ? ws_bytes : (size_t)0);
+    int dev = -1;
+    PDU_CUDA(cudaGetDevice(&dev));
+    PDU_REQUIRE(dev == p->device, "pdu_toep_cg_c64: plan was created on device %d, current device is %d", p->device, dev);
+    PDU_CHECK_DEVICE("pdu_toep_cg_c64");
+    const long plane = (long)p->n0 * p->n1, cells = (long)p->k0 * p->k1;
+    const long img_b = (smaps ? 1 : coils) * plane, smap_b = smaps_batch == 1 ? 0 : coils * plane;
+    const int lam_div = lam_count == 1 ? 0 : (smaps ? 1 : coils);   // system -> batch element within a chunk
+    const double tol2 = (double)tol * (double)tol;
+    for (int b0 = 0; b0 < batch; b0 += cb) {
+        const int nb = b0 + cb <= batch ? cb : batch - b0;
+        int rc = tz_cg_chunk(p, (const float2*)b + b0 * img_b, x0 ? (const float2*)x0 + b0 * img_b : nullptr,
+                             (float2*)x + b0 * img_b, (const float2*)kernel + (kernel_batch == 1 ? 0 : b0 * cells),
+                             kernel_batch == 1 ? 1 : nb, smaps ? (const float2*)smaps + b0 * smap_b : nullptr, nb, coils,
+                             smaps_batch == 1 ? 1 : nb, lam ? lam + (lam_count == 1 ? 0 : b0) : nullptr, lam_div, max_iter,
+                             tol2, conj_kernel ? 1 : 0, w, (cudaStream_t)stream);
         if (rc) return rc;
     }
     return PDU_OK;

@@ -7,6 +7,7 @@ the reference reaches the library through its unmounted MRI branch, /root/refere
     KbInterp(...)(image, omega) / KbInterpAdjoint(...)(data, omega)
     calc_density_compensation_function(ktraj, im_size, num_iterations=10, ...)
     calc_toeplitz_kernel(omega, im_size, weights=None, norm=None, ...) / ToepNufft()(image, kernel, smaps=None, norm=None)
+    toep_cg(b, kernel, smaps=None, lam=0.0, x0=None, max_iter=10, tol=0.0): CG on (ToepNufft + lam I) x = b
 
 image: complex64 [B, C, N0, N1]; omega: float32 [2, M] radians (or [B, 2, M]); data: complex64
 [B, C, M].  With smaps [1 or B, coils, N0, N1] the forward expands a one-channel image to the
@@ -598,11 +599,12 @@ def _check_norm(norm: Optional[str]) -> None:
         raise ValueError("norm must be None or 'ortho'")
 
 
-def _toep_apply(image: torch.Tensor, kernel: torch.Tensor, smaps: Optional[torch.Tensor], conj: bool) -> torch.Tensor:
-    image = require_cuda(image, torch.complex64, "image")
+def _toep_args(image: torch.Tensor, kernel: torch.Tensor, smaps: Optional[torch.Tensor], name: str = "image"):
+    """Checked operands of a Toeplitz call: (image, kernel [1 or B, 2 N0, 2 N1], smaps or None, coils, smaps batch)."""
+    image = require_cuda(image, torch.complex64, name)
     kernel = require_cuda(kernel, torch.complex64, "kernel")
     if image.dim() != 4:
-        raise ValueError(f"image must be [B, C, N0, N1], got {tuple(image.shape)}")
+        raise ValueError(f"{name} must be [B, C, N0, N1], got {tuple(image.shape)}")
     B, ci, N0, N1 = image.shape
     if kernel.dim() == 2:
         kernel = kernel[None]
@@ -617,8 +619,14 @@ def _toep_apply(image: torch.Tensor, kernel: torch.Tensor, smaps: Optional[torch
         if smaps.dim() != 4 or tuple(smaps.shape[-2:]) != (N0, N1) or smaps.shape[0] not in (1, B):
             raise ValueError(f"smaps must be [1 or {B}, coils, {N0}, {N1}]")
         if ci != 1:
-            raise ValueError("with smaps the image must have one channel")
+            raise ValueError(f"with smaps the {name} must have one channel")
         coils, sb = smaps.shape[1], smaps.shape[0]
+    return image, kernel, smaps, coils, sb
+
+
+def _toep_apply(image: torch.Tensor, kernel: torch.Tensor, smaps: Optional[torch.Tensor], conj: bool) -> torch.Tensor:
+    image, kernel, smaps, coils, sb = _toep_args(image, kernel, smaps)
+    B, _, N0, N1 = image.shape
     out = torch.empty_like(image)
     if out.numel() == 0:
         return out
@@ -718,3 +726,114 @@ def calc_toeplitz_kernel(omega: torch.Tensor, im_size: Sequence[int], weights: O
         check(lib().pdu_toep_kernel_c64(h, q1.data_ptr(), q2.data_ptr(), kernel.data_ptr(), nk, scale, ws.data_ptr(),
                                         ws.numel(), stream_ptr()), "pdu_toep_kernel_c64")
     return kernel if omega.dim() == 3 else kernel[0]
+
+
+# ----------------------------------------------------------------------------- conjugate gradient on the normal operator
+def _cg_lam(lam, B: int, device: torch.device):
+    """(device float32 lam or None for 0, lam_count).  A Python number becomes a one-entry tensor by a fill kernel."""
+    if isinstance(lam, torch.Tensor):
+        if not lam.is_cuda:
+            raise PduError(f"lam is on {lam.device}: the pd_unet_b200 operators run on CUDA only (no CPU fallback)")
+        if lam.dtype != torch.float32:
+            raise TypeError(f"a tensor lam must be float32, got {lam.dtype}")
+        if lam.numel() not in (1, B):
+            raise ValueError(f"a tensor lam must have 1 or B = {B} entries, got {tuple(lam.shape)}")
+        return lam.detach().reshape(-1).contiguous(), lam.numel()
+    if isinstance(lam, bool) or not isinstance(lam, (int, float)):
+        raise ValueError(f"lam must be a float >= 0 or a float32 CUDA tensor, got {type(lam).__name__}")
+    if not float(lam) >= 0.0:
+        raise ValueError(f"lam must be >= 0, got {lam}")
+    if float(lam) == 0.0:
+        return None, 1
+    return torch.full((1,), float(lam), dtype=torch.float32, device=device), 1
+
+
+def _toep_cg_solve(b, kernel, smaps, lam_dev, lam_count: int, x0, max_iter: int, tol: float, conj: bool) -> torch.Tensor:
+    b, kernel, smaps, coils, sb = _toep_args(b, kernel, smaps, "b")
+    B, _, N0, N1 = b.shape
+    if x0 is not None:
+        x0 = require_cuda(x0, torch.complex64, "x0")
+        if x0.shape != b.shape:
+            raise ValueError(f"x0 must have the shape of b {tuple(b.shape)}, got {tuple(x0.shape)}")
+    x = torch.empty_like(b)
+    if x.numel() == 0:
+        return x
+    with torch.cuda.device(b.device):
+        tp = _toep_plan((N0, N1))
+        h = tp.handle(b.device)
+        L = lib()
+        ws = torch.empty(int(L.pdu_toep_cg_workspace_bytes(h, B, coils, 1 if smaps is not None else 0)), dtype=torch.uint8,
+                         device=b.device)
+        check(L.pdu_toep_cg_c64(h, b.data_ptr(), x0.data_ptr() if x0 is not None else None, x.data_ptr(), kernel.data_ptr(),
+                                kernel.shape[0], smaps.data_ptr() if smaps is not None else None, B, coils, sb,
+                                lam_dev.data_ptr() if lam_dev is not None else None, lam_count, max_iter, tol, 1 if conj else 0,
+                                ws.data_ptr(), ws.numel(), stream_ptr()), "pdu_toep_cg_c64")
+    return x
+
+
+class _ToepCgFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, b, lam_t, kernel, smaps, x0, lam_dev, lam_count, max_iter, tol):
+        x = _toep_cg_solve(b, kernel, smaps, lam_dev, lam_count, x0, max_iter, tol, False)
+        ctx.save_for_backward(kernel, x, smaps)
+        ctx.cg = (lam_dev, lam_count, max_iter, tol)
+        ctx.lam_shape = lam_t.shape if lam_t is not None else None
+        return x
+
+    @staticmethod
+    def backward(ctx, g):
+        kernel, x, smaps = ctx.saved_tensors
+        lam_dev, lam_count, max_iter, tol = ctx.cg
+        # implicit differentiation of x = M^-1 b, M = T + lam I: grad_b = M^-H g (the conj-kernel system), and
+        # dx / dlam = -M^-1 x, so grad_lam = -Re <M^-H g, x> per lam entry
+        gb = _toep_cg_solve(g.contiguous(), kernel, smaps, lam_dev, lam_count, None, max_iter, tol, True)
+        glam = None
+        if ctx.needs_input_grad[1]:
+            prod = (gb.conj() * x).real
+            glam = -(prod.sum() if lam_count == 1 else prod.sum(dim=(1, 2, 3))).reshape(ctx.lam_shape)
+        return (gb if ctx.needs_input_grad[0] else None), glam, None, None, None, None, None, None, None
+
+
+def toep_cg(b: torch.Tensor, kernel: torch.Tensor, smaps: Optional[torch.Tensor] = None, lam=0.0,
+            x0: Optional[torch.Tensor] = None, max_iter: int = 10, tol: float = 0.0) -> torch.Tensor:
+    """Conjugate gradient on the Toeplitz normal operator: solves (T + lam I) x = b with T(v) = ToepNufft()(v, kernel,
+    smaps=smaps), for every system of the batch at once, entirely on the device.
+
+    b: complex64 [B, C, N0, N1], every (batch, channel) plane its own system; with smaps [1 or B, coils, N0, N1], b is
+    [B, 1, N0, N1] and each batch element is one system (CG-SENSE).  kernel: [2 N0, 2 N1] or [1 or B, 2 N0, 2 N1] from
+    calc_toeplitz_kernel.  lam: a float >= 0, or a float32 CUDA tensor with 1 or B entries (channels of a batch element
+    share its lam; a tensor is not checked for sign, which would need a read-back).  x0: the warm start, shape of b;
+    None starts from zero.  max_iter: iterations run, an int >= 0 (0 returns x0, or zeros).  tol >= 0: relative to
+    ||b|| per system, like scipy's rtol.
+
+    Per system, with float64 scalars and complex64 vectors:
+        r = b - (T + lam) x0  (r = b without x0);  p = r;  rho = ||r||^2;  bb = ||b||^2
+        repeat max_iter times:
+            q = (T + lam) p;  pi = Re<p, q>
+            if frozen or rho == 0 or pi <= 0:  freeze (x and r stay as they are from then on)
+            alpha = rho / pi;  x += alpha p;  r -= alpha q;  rho' = ||r||^2
+            if rho' <= tol^2 bb:  freeze
+            p = r + (rho' / rho) p;  rho = rho'
+    tol freezes a converged system but never ends the call early: every call runs max_iter iterations of device work,
+    so a looser tol does not make it faster.  In exchange there is no host synchronisation and the whole solve can be
+    captured in a CUDA graph.  The sums add in a fixed order without atomics, so a system's result is bit-identical
+    whatever else is in the batch, however the batch is chunked, and under graph replay; no NaN or Inf is written (a
+    zero right-hand side gives 0, a zero operator gives x0).
+
+    Differentiable in b and in a tensor lam by implicit differentiation (the MoDL convention): grad_b solves the
+    adjoint system (conj kernel) with the same lam, max_iter and tol, and grad_lam = -Re sum conj(grad_b) x per lam
+    entry.  That is the gradient of the exact solution, which x approximates, not of the truncated iteration.  No
+    gradient reaches kernel, smaps or x0."""
+    if isinstance(max_iter, bool) or not isinstance(max_iter, int) or max_iter < 0:
+        raise ValueError(f"max_iter must be an int >= 0, got {max_iter!r}")
+    if isinstance(tol, bool) or not isinstance(tol, (int, float)) or not float(tol) >= 0.0:
+        raise ValueError(f"tol must be a float >= 0, got {tol!r}")
+    if not isinstance(b, torch.Tensor):
+        raise TypeError("b must be a torch.Tensor")
+    if not b.is_cuda:
+        raise PduError(f"b is on {b.device}: the pd_unet_b200 operators run on CUDA only (no CPU fallback)")
+    if b.dim() != 4:
+        raise ValueError(f"b must be [B, C, N0, N1], got {tuple(b.shape)}")
+    lam_dev, lam_count = _cg_lam(lam, b.shape[0], b.device)
+    lam_t = lam if isinstance(lam, torch.Tensor) else None
+    return _ToepCgFn.apply(b, lam_t, kernel, smaps, x0, lam_dev, lam_count, max_iter, float(tol))

@@ -70,7 +70,7 @@ PDU_API long pdu_launch_count(int reset);
  * their loads so that the path can be tested. */
 PDU_API int pdu_device_error(int reset);
 /* Name and shape of the kernel the dispatcher of an operator chose in this thread's most recent
- * call: op in {"radon_fwd", "radon_adj", "filter", "nufft_fwd", "nufft_adj", "toep", "cg"}; "" before
+ * call: op in {"radon_fwd", "radon_adj", "filter", "nufft_fwd", "nufft_adj", "toep", "cg", "smaps_grad"}; "" before
  * the first call.  The string stays valid until the thread's next call of that operator. */
 PDU_API const char* pdu_last_kernel(const char* op);
 
@@ -215,6 +215,21 @@ PDU_API int pdu_nufft_adj_binned_c64(pdu_nufft_plan_t* plan, const float* kdata,
                                      const float* smaps, const float* kweight, int batch, int coils,
                                      int smaps_batch, long m, float scale, const void* bins, int flags,
                                      void* workspace, size_t workspace_bytes, pdu_stream_t stream);
+/* Gradient of the coil maps through the adjoint: gs [smaps_batch, coils, n0, n1] complex64 (+)= the adjoint of kdata
+ * [batch, coils, m] WITHOUT the coil combination, U[b, c] = A^H(kweight . kdata[b, c]) (times scale, as
+ * pdu_nufft_adj_c64), reduced as   gs[s, c] = sum_{b : s(b) = s} U[b, c] . conj(q[b]),  s(b) = 0 for smaps_batch 1, else b.
+ * q: [batch, 1, n0, n1] complex64, or [batch, 2, n0, n1] float32 with PDU_NUFFT_IMAGE_SPLIT in flags.  The path is the
+ * one the adjoint entry points would take: bins non-NULL -- the fused row-binned path (pdu_nufft_adj_binned_c64's
+ * workspace, kweight and PDU_NUFFT_KDATA_SPLIT allowed); otherwise omega with the CSR gather when csr is non-NULL,
+ * the atomic scatter when it is NULL (pdu_nufft_workspace_bytes of one batch chunk, complex64 kdata, no kweight).  The
+ * last pass is smaps_grad_kernel in place of crop_apod_kernel: b runs in increasing order in registers, no atomics,
+ * and accumulate != 0 adds to gs (a batch cut into calls carries a shared map's sum from call to call).
+ * pdu_last_kernel("smaps_grad").  The gradient torch autograd wants for the maps of KbNufft (kdata = the incoming
+ * gradient, q = the image) and of KbNufftAdjoint (kdata = its input, q = the incoming gradient). */
+PDU_API int pdu_nufft_adj_smaps_grad_c64(pdu_nufft_plan_t* plan, const float* kdata, const float* q, float* gs,
+                                         const float* omega, const void* csr, const void* bins, const float* kweight,
+                                         int batch, int coils, int smaps_batch, long m, float scale, int flags,
+                                         int accumulate, void* workspace, size_t workspace_bytes, pdu_stream_t stream);
 
 /* Toeplitz-embedded normal operator A^H W A of the NUFFT: no interpolation, one zero-padded 2n0 x 2n1
  * FFT, a pointwise multiply by a kernel and one cropped inverse FFT, whatever the trajectory length.
@@ -245,6 +260,16 @@ PDU_API int pdu_toep_kernel_c64(pdu_nufft_plan_t* plan, const float* q1, const f
 PDU_API int pdu_toep_apply_c64(pdu_nufft_plan_t* plan, const float* image, float* out, const float* kernel,
                                int kernel_batch, const float* smaps, int batch, int coils, int smaps_batch,
                                int conj_kernel, void* ws, size_t ws_bytes, pdu_stream_t stream);
+/* Gradient of the coil maps through pdu_toep_apply_c64 with smaps: for x, g [batch, 1, n0, n1] c64,
+ *     gs[s, c] (+)= out_scale * sum_{b : s(b) = s} [ T(S_c x_b) . conj(g_b) + T^H(S_c g_b) . conj(x_b) ]
+ * (T^H: the conjugate kernel; conj_kernel != 0 swaps the two).  Two apply launch sets, one per term; the last pass walks
+ * the batch elements sharing a map in increasing order instead of the coils (tz_rows_out_kernel's map-gradient mode on
+ * the fast sizes, smaps_grad_kernel on the generic ones).  out_scale = -1 gives the conjugate-gradient solve's map
+ * gradient at (x, M^-H g).  Workspace as pdu_toep_apply_c64.  pdu_last_kernel("smaps_grad"). */
+PDU_API int pdu_toep_smaps_grad_c64(pdu_nufft_plan_t* plan, const float* x, const float* g, float* gs, const float* kernel,
+                                    int kernel_batch, const float* smaps, int batch, int coils, int smaps_batch,
+                                    int conj_kernel, float out_scale, int accumulate, void* ws, size_t ws_bytes,
+                                    pdu_stream_t stream);
 
 /* Conjugate gradient on the Toeplitz normal operator: solves (T + lam I) x = b, T = pdu_toep_apply_c64's operator, for
  * every system at once -- a plane [batch, coils, n0, n1] without smaps; a batch element b [batch, 1, n0, n1] with smaps

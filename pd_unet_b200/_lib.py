@@ -69,10 +69,14 @@ SIGNATURES = {
                                            C.c_size_t, _p]),
     "pdu_nufft_adj_binned_c64": (C.c_int, [_p, _p, _p, _p, _p, C.c_int, C.c_int, C.c_int, C.c_long, C.c_float, _p, C.c_int, _p,
                                            C.c_size_t, _p]),
+    "pdu_nufft_adj_smaps_grad_c64": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, _p, C.c_int, C.c_int, C.c_int, C.c_long, C.c_float,
+                                               C.c_int, C.c_int, _p, C.c_size_t, _p]),
     "pdu_toep_plan_create": (C.c_int, [C.POINTER(_p), C.c_int, C.c_int]),
     "pdu_toep_workspace_bytes": (C.c_size_t, [_p, C.c_int]),
     "pdu_toep_kernel_c64": (C.c_int, [_p, _p, _p, _p, C.c_int, C.c_float, _p, C.c_size_t, _p]),
     "pdu_toep_apply_c64": (C.c_int, [_p, _p, _p, _p, C.c_int, _p, C.c_int, C.c_int, C.c_int, C.c_int, _p, C.c_size_t, _p]),
+    "pdu_toep_smaps_grad_c64": (C.c_int, [_p, _p, _p, _p, _p, C.c_int, _p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float,
+                                          C.c_int, _p, C.c_size_t, _p]),
     "pdu_toep_cg_workspace_bytes": (C.c_size_t, [_p, C.c_int, C.c_int, C.c_int]),
     "pdu_toep_cg_c64": (C.c_int, [_p, _p, _p, _p, _p, C.c_int, _p, C.c_int, C.c_int, C.c_int, _p, C.c_int, C.c_int, C.c_float,
                                   C.c_int, _p, C.c_size_t, _p]),

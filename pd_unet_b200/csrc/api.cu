@@ -152,7 +152,7 @@ int pdu_device_error(int reset) {
 
 const char* pdu_last_kernel(const char* op) {
     static const char* names[pdu::OP_COUNT] = {"radon_fwd", "radon_adj", "filter", "nufft_fwd", "nufft_adj",
-                                               "toep", "cg"};
+                                               "toep", "cg", "smaps_grad"};
     if (!op) return "";
     for (int i = 0; i < pdu::OP_COUNT; ++i)
         if (!strcmp(op, names[i])) return pdu::g_kernel[i];

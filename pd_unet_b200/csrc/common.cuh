@@ -26,7 +26,7 @@ int check_device_error(const char* who);
 
 // the kernel the dispatcher of an operator chose most recently (this thread): pdu_last_kernel()
 enum Op { OP_RADON_FWD = 0, OP_RADON_ADJ = 1, OP_FILTER = 2, OP_NUFFT_FWD = 3, OP_NUFFT_ADJ = 4, OP_TOEP = 5, OP_CG = 6,
-          OP_COUNT };
+          OP_SMAPS_GRAD = 7, OP_COUNT };
 void note_kernel(int op, const char* fmt, ...);
 
 #define PDU_CHECK_DEVICE(who)                          \

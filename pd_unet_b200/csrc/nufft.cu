@@ -129,6 +129,61 @@ __global__ void __launch_bounds__(256)
     }
 }
 
+// ------------------------------------------------------------------ crop + apodise, coil-map gradient (SmapsGrad)
+// the sibling of crop_apod_kernel for the gradient of the coil maps: the same per-plane grid (or cropped planes U), but
+// summed over the batch elements sharing a map instead of over the coils, each times conj(q[b]); b in increasing order
+__device__ __forceinline__ float2 sg_q(const float* q, int q_split, long b, long plane, long pix) {
+    if (q_split) return make_float2(__ldg(q + 2 * b * plane + pix), __ldg(q + (2 * b + 1) * plane + pix));
+    return __ldg(reinterpret_cast<const float2*>(q) + b * plane + pix);
+}
+
+__global__ void __launch_bounds__(256)
+    smaps_grad_kernel(const float2* __restrict__ grid, const float* __restrict__ q, float2* __restrict__ gs,
+                      const float* __restrict__ s0, const float* __restrict__ s1, NufftDims d, int coils, int batch,
+                      int per_batch, int q_split, int accumulate, float scale, long total) {
+    const long plane = (long)d.n0 * d.n1;
+    const long gplane = (long)d.k0 * d.k1;
+    for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long)gridDim.x * blockDim.x) {
+        const int c1 = (int)(i % d.n1);
+        const long t = i / d.n1;
+        const int c0 = (int)(t % d.n0);
+        const long o = t / d.n0;          // gs plane: s * coils + c
+        const long s = o / coils, c = o - s * coils;
+        const long b_lo = per_batch ? s : 0, b_hi = per_batch ? s + 1 : batch;
+        const float w = __ldg(s0 + c0) * __ldg(s1 + c1) * scale;
+        const long pix = (long)c0 * d.n1 + c1;
+        const float2* gc = grid + c * gplane + (long)c0 * d.k1 + c1;     // plane b * coils + c
+        float2 acc = make_float2(0.f, 0.f);
+        long b = b_lo;
+        for (; b + 4 <= b_hi; b += 4) {   // four batch elements' loads in flight, added in order
+            float2 gv[4], qv[4];
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                gv[u] = __ldg(gc + (b + u) * coils * gplane);
+                qv[u] = sg_q(q, q_split, b + u, plane, pix);
+            }
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                const float2 z = cmul_conj(gv[u], qv[u]);
+                acc.x += z.x;
+                acc.y += z.y;
+            }
+        }
+        for (; b < b_hi; ++b) {
+            const float2 z = cmul_conj(__ldg(gc + b * coils * gplane), sg_q(q, q_split, b, plane, pix));
+            acc.x += z.x;
+            acc.y += z.y;
+        }
+        float2 v = make_float2(acc.x * w, acc.y * w);
+        if (accumulate) {
+            const float2 old = gs[i];
+            v.x += old.x;
+            v.y += old.y;
+        }
+        gs[i] = v;
+    }
+}
+
 // ------------------------------------------------------------------ interpolation (gather)
 // thread = one sample m; loops over the PC planes of its plane chunk (blockIdx.y)
 template <int JT>
@@ -1063,6 +1118,16 @@ int launch_crop_apod(pdu_nufft_plan* p, const float2* U, const float2* smaps, fl
     return PDU_OK;
 }
 
+// grid or cropped planes U [batch][coils] with plane geometry d (k0 x k1 planes, the n0 x n1 corner kept) -> sg.gs
+int launch_smaps_grad(pdu_nufft_plan* p, const float2* U, NufftDims d, int coils, float scale, const SmapsGrad& sg,
+                      cudaStream_t st) {
+    const long total = (long)(sg.per_batch ? sg.batch : 1) * coils * p->n0 * p->n1;
+    smaps_grad_kernel<<<stream_grid(total), 256, 0, st>>>(U, sg.q, sg.gs, p->d_s0, p->d_s1, d, coils, sg.batch, sg.per_batch,
+                                                          sg.q_split, sg.accumulate, scale * sg.scale, total);
+    PDU_LAUNCHED();
+    return PDU_OK;
+}
+
 static int check_call(const pdu_nufft_plan* p, const void* a, const void* b, const void* omega, int batch, int coils,
                       int smaps_batch, const void* smaps, long m, const char* who) {
     PDU_REQUIRE(p != nullptr, "%s: plan is null", who);
@@ -1188,10 +1253,13 @@ __device__ __forceinline__ double cg_block_sum(double v, double* red) {
 // fast path, pass 3: SEQ rows of one output plane per CTA: pruned inverse row FFT of T's N rows (first N outputs),
 // x scale; with coil maps the CTA walks the batch element's coils in a fixed order and sums conj(S_c) T_c in registers
 // (bit-reproducible; no cropped intermediate, no crop_apod_kernel pass).  CG: the TzCg epilogue at the output store.
-template <int K, int SEQ, bool CG = false>
+// GS (the coil-map gradient, SmapsGrad): the CTA owns rows of coil c of gs plane blockIdx.y = s * coils + c and walks the
+// other axis instead -- the batch elements b sharing that map, in increasing order -- summing T_{b, c} conj(q_b); out
+// is gs.
+template <int K, int SEQ, bool CG = false, bool GS = false>
 __global__ void __launch_bounds__(SEQ* FastFft<K>::TPS)
     tz_rows_out_kernel(const float2* __restrict__ T, const float2* __restrict__ smaps, float2* __restrict__ out,
-                       const float2* __restrict__ tw_g, int coils, int smaps_batch, float scale, TzCg cg) {
+                       const float2* __restrict__ tw_g, int coils, int smaps_batch, float scale, TzCg cg, SmapsGrad sg) {
     using F = FastFft<K>;
     constexpr int N = K / 2, TPS = F::TPS, NS3 = F::NS3, R3 = F::R3;
     constexpr int PER = TPS >= NS3 ? 1 : NS3 / TPS;     // last-pass butterflies per thread (ff_transform)
@@ -1208,10 +1276,14 @@ __global__ void __launch_bounds__(SEQ* FastFft<K>::TPS)
     for (int i = 0; i < PER; ++i)
 #pragma unroll
         for (int r = 0; r < R3; ++r) acc[i][r] = make_float2(0.f, 0.f);
-    const int nc = smaps ? coils : 1;
-    const float2* sm = smaps ? smaps + ((long)(smaps_batch == 1 ? 0 : q) * coils * N + row) * N : nullptr;
-    for (int c = 0; c < nc; ++c) {
-        const long p = smaps ? (long)q * coils + c : q;
+    // GS: the walk runs over b in [b_lo, b_hi) for coil gc, reading q_b's row where the apply reads S_c's
+    const int gc = GS ? q % coils : 0;
+    const int b_lo = GS ? (sg.per_batch ? q / coils : 0) : 0;
+    const int nc = GS ? (sg.per_batch ? b_lo + 1 : sg.batch) : (smaps ? coils : 1);
+    const float2* sm = GS ? reinterpret_cast<const float2*>(sg.q) + (long)row * N
+                          : (smaps ? smaps + ((long)(smaps_batch == 1 ? 0 : q) * coils * N + row) * N : nullptr);
+    for (int c = b_lo; c < nc; ++c) {
+        const long p = GS ? (long)c * coils + gc : (smaps ? (long)q * coils + c : q);
         const float2* src = T + (p * N + row) * K + t;
         const float2* smc = sm ? sm + (long)c * N * N : nullptr;
         auto ld = [&](int r) { return live ? __ldcs(src + r * TPS) : make_float2(0.f, 0.f); };
@@ -1237,7 +1309,17 @@ __global__ void __launch_bounds__(SEQ* FastFft<K>::TPS)
             const int j = t + i * TPS;
             if (j < NS3) {
 #pragma unroll
-                for (int r = 0; r < R3 / 2; ++r) dst[j + r * NS3] = make_float2(acc[i][r].x * scale, acc[i][r].y * scale);
+                for (int r = 0; r < R3 / 2; ++r) {
+                    float2 v = make_float2(acc[i][r].x * scale, acc[i][r].y * scale);
+                    if constexpr (GS) {
+                        if (sg.accumulate) {
+                            const float2 old = dst[j + r * NS3];
+                            v.x += old.x;
+                            v.y += old.y;
+                        }
+                    }
+                    dst[j + r * NS3] = v;
+                }
             }
         }
     } else {
@@ -1509,16 +1591,18 @@ constexpr int TZ_SEQ_ROWS = 4;
 template <int K>
 static constexpr int tz_seq_rows_out() { return K == 2048 ? 2 : TZ_SEQ_ROWS; }
 
-// cg: the conjugate-gradient epilogue (tz_rows_out_kernel<K, SO, true>), or null for the plain apply
+// cg: the conjugate-gradient epilogue (tz_rows_out_kernel<K, SO, true>), or null for the plain apply; sg: the coil-map
+// gradient walk (tz_rows_out_kernel<K, SO, false, true>) into sg->gs instead of out
 template <int K>
 static int tz_apply_fast(pdu_nufft_plan* p, const float2* image, float2* out, const float2* kern, int kernel_batch,
                          const float2* smaps, int batch, int coils, int smaps_batch, int conj, float2* T, const TzCg* cg,
-                         cudaStream_t st) {
+                         cudaStream_t st, const SmapsGrad* sg) {
     constexpr int N = K / 2, SC = ff_seq_cols<K>(), SO = tz_seq_rows_out<K>();
     const int planes = batch * coils;
     PDU_CUDA((ensure_dyn_smem<ff_rows_fwd_kernel<K, FF_SEQ_ROWS>>((int)ff_smem_bytes<K>(FF_SEQ_ROWS))));
     PDU_CUDA((ensure_dyn_smem<tz_cols_kernel<K, SC>>((int)ff_smem_bytes<K>(SC))));
     if (cg) PDU_CUDA((ensure_dyn_smem<tz_rows_out_kernel<K, SO, true>>((int)ff_smem_bytes<K>(SO))));
+    else if (sg) PDU_CUDA((ensure_dyn_smem<tz_rows_out_kernel<K, SO, false, true>>((int)ff_smem_bytes<K>(SO))));
     else PDU_CUDA((ensure_dyn_smem<tz_rows_out_kernel<K, SO>>((int)ff_smem_bytes<K>(SO))));
     ff_rows_fwd_kernel<K, FF_SEQ_ROWS><<<dim3((unsigned)cdiv(N, FF_SEQ_ROWS), (unsigned)planes), FF_SEQ_ROWS * FastFft<K>::TPS,
                                          ff_smem_bytes<K>(FF_SEQ_ROWS), st>>>(image, smaps, T, p->d_s0, p->d_s1, p->d_w1,
@@ -1532,14 +1616,24 @@ static int tz_apply_fast(pdu_nufft_plan* p, const float2* image, float2* out, co
     const float scale = 1.f / ((float)K * (float)K);
     if (cg) {
         tz_rows_out_kernel<K, SO, true><<<grid_out, SO * FastFft<K>::TPS, ff_smem_bytes<K>(SO), st>>>(
-            T, smaps, out, p->d_w1, coils, smaps_batch, scale, *cg);
+            T, smaps, out, p->d_w1, coils, smaps_batch, scale, *cg, SmapsGrad{});
         PDU_LAUNCHED();
         note_kernel(OP_CG, "ff_rows_fwd_kernel<%d,%d> + tz_cols_kernel<%d,%d> + tz_rows_out_kernel<%d,%d,cg> + cg_update_kernel + "
                     "cg_direction_kernel (fast path, %d systems of %dx%d)", K, FF_SEQ_ROWS, K, SC, K, SO, out_planes, N, N);
         return PDU_OK;
     }
+    if (sg) {
+        const dim3 grid_gs((unsigned)cdiv(N, SO), (unsigned)((sg->per_batch ? batch : 1) * coils));
+        tz_rows_out_kernel<K, SO, false, true><<<grid_gs, SO * FastFft<K>::TPS, ff_smem_bytes<K>(SO), st>>>(
+            T, nullptr, sg->gs, p->d_w1, coils, 1, scale * sg->scale, TzCg{}, *sg);
+        PDU_LAUNCHED();
+        note_kernel(OP_SMAPS_GRAD, "ff_rows_fwd_kernel<%d,%d> + tz_cols_kernel<%d,%d> + tz_rows_out_kernel<%d,%d,smaps_grad> per "
+                    "term (fast path, %d planes of %dx%d)", K, FF_SEQ_ROWS, K, SC, K, SO, planes, N, N);
+        return PDU_OK;
+    }
     tz_rows_out_kernel<K, SO><<<grid_out, SO * FastFft<K>::TPS, ff_smem_bytes<K>(SO), st>>>(T, smaps, out, p->d_w1, coils,
-                                                                                            smaps_batch, scale, TzCg{});
+                                                                                            smaps_batch, scale, TzCg{},
+                                                                                            SmapsGrad{});
     PDU_LAUNCHED();
     note_kernel(OP_TOEP, "ff_rows_fwd_kernel<%d,%d> + tz_cols_kernel<%d,%d> + tz_rows_out_kernel<%d,%d> (fast path, %d planes of %dx%d)",
                 K, FF_SEQ_ROWS, K, SC, K, SO, planes, N, N);
@@ -1552,7 +1646,7 @@ static bool tz_cols_seq8(const pdu_nufft_plan* p) { return pf_smem_bytes(PF_SEQ_
 template <int SC>
 static int tz_apply_generic(pdu_nufft_plan* p, const float2* image, float2* out, const float2* kern, int kernel_batch,
                             const float2* smaps, int batch, int coils, int smaps_batch, int conj, float2* ws, const TzCg* cg,
-                            cudaStream_t st) {
+                            cudaStream_t st, const SmapsGrad* sg) {
     const int planes = batch * coils;
     const long cells = (long)p->k0 * p->k1;
     float2* grid = ws;
@@ -1580,6 +1674,17 @@ static int tz_apply_generic(pdu_nufft_plan* p, const float2* image, float2* out,
     pfft_cols_adj_kernel<SC><<<dim3((unsigned)cdiv(p->n1, SC), (unsigned)planes), 256, pf_smem_bytes(SC, p->k0), st>>>(
         T, U, p->d_w0, p->pf0, d, pitch0);
     PDU_LAUNCHED();
+    if (sg) {
+        NufftDims dc = d;          // the cropped result is a dense [n0][n1] "grid"
+        dc.k0 = d.n0;
+        dc.k1 = d.n1;
+        rc = launch_smaps_grad(p, U, dc, coils, 1.f / ((float)p->k0 * (float)p->k1), *sg, st);
+        if (rc) return rc;
+        note_kernel(OP_SMAPS_GRAD, "pfft_rows_fwd_kernel<%d> + pfft_cols_fwd_kernel<%d> + tz_mul_kernel + pfft_rows_adj_kernel<%d> + "
+                    "pfft_cols_adj_kernel<%d> + smaps_grad_kernel per term (generic path, %d planes of %dx%d)",
+                    PF_SEQ_ROWS, SC, PF_SEQ_ROWS, SC, planes, p->n0, p->n1);
+        return PDU_OK;
+    }
     const int out_planes = smaps ? batch : planes;
     rc = launch_crop_apod(p, U, smaps, out, out_planes, coils, smaps_batch, 1.f / ((float)p->k0 * (float)p->k1), 0, st);
     if (rc) return rc;
@@ -1601,19 +1706,19 @@ static int tz_apply_generic(pdu_nufft_plan* p, const float2* image, float2* out,
 
 static int tz_apply_chunk(pdu_nufft_plan* p, const float2* image, float2* out, const float2* kern, int kernel_batch,
                           const float2* smaps, int batch, int coils, int smaps_batch, int conj, float2* ws, cudaStream_t st,
-                          const TzCg* cg = nullptr) {
+                          const TzCg* cg = nullptr, const SmapsGrad* sg = nullptr) {
     if (tz_fast(p)) {
         switch (p->k0) {
-            case 256: return tz_apply_fast<256>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st);
-            case 512: return tz_apply_fast<512>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st);
-            case 640: return tz_apply_fast<640>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st);
-            case 1024: return tz_apply_fast<1024>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st);
-            default: return tz_apply_fast<2048>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st);
+            case 256: return tz_apply_fast<256>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st, sg);
+            case 512: return tz_apply_fast<512>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st, sg);
+            case 640: return tz_apply_fast<640>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st, sg);
+            case 1024: return tz_apply_fast<1024>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st, sg);
+            default: return tz_apply_fast<2048>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st, sg);
         }
     }
     if (tz_cols_seq8(p))
-        return tz_apply_generic<PF_SEQ_COLS>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st);
-    return tz_apply_generic<2>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st);
+        return tz_apply_generic<PF_SEQ_COLS>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st, sg);
+    return tz_apply_generic<2>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st, sg);
 }
 
 // kernel build, step 4: the full (unpruned) 2-D FFT of p_circ, in place in `kern` with T as the intermediate
@@ -1862,7 +1967,7 @@ static int nufft_fwd_chunk(pdu_nufft_plan_t* p, const float2* image, float2* kda
 
 static int nufft_adj_chunk(pdu_nufft_plan_t* p, const float2* kdata, float2* image, const float* omega, const float2* smaps,
                            int batch, int coils, int smaps_batch, long m, float scale, float2* grid, const void* csr,
-                           cudaStream_t st) {
+                           cudaStream_t st, const SmapsGrad* sg = nullptr) {
     const int planes = batch * coils;
     int rc;
     int variant = option(OPT_NUFFT_ADJ);
@@ -1886,7 +1991,7 @@ static int nufft_adj_chunk(pdu_nufft_plan_t* p, const float2* kdata, float2* ima
     if (rc) return rc;
     const int out_planes = smaps ? batch : planes;
     const long total = (long)out_planes * p->n0 * p->n1;
-    note_kernel(OP_NUFFT_ADJ, "%s + %s + crop_apod_kernel (%d planes of %dx%d, M=%ld)",
+    note_kernel(sg ? OP_SMAPS_GRAD : OP_NUFFT_ADJ, "%s + %s + %s (%d planes of %dx%d, M=%ld)",
                 csr ? (compact ? "transpose_kdata_kernel + interp_adj_csrT_kernel (sorted gather: 4 lanes per cell x 16 planes, long rows by warps, non-empty cells only)"
                                : "transpose_kdata_kernel + interp_adj_csrT_kernel (sorted gather: 4 lanes per cell x 16 planes, long rows by warps)")
                     : "interp_adj_kernel (float2 atomics)",
@@ -1894,7 +1999,7 @@ static int nufft_adj_chunk(pdu_nufft_plan_t* p, const float2* kdata, float2* ima
                                         : "ff_rows_adj_kernel + ff_cols_adj_kernel (register-resident pruned FFT)")
                              : (variant == 1 && p->pfft_ok ? "pfft_rows_adj_kernel + pfft_cols_adj_kernel (generic pruned FFT)"
                                                            : "cuFFT C2C"),
-                planes, p->k0, p->k1, m);
+                sg ? "smaps_grad_kernel" : "crop_apod_kernel", planes, p->k0, p->k1, m);
     if (variant == 2) {
         float2* T = grid + (long)planes * p->k0 * p->k1;
         float2* U = T + (long)planes * std::max((long)p->n0 * p->k1, (long)p->k0 * p->n1);
@@ -1911,6 +2016,7 @@ static int nufft_adj_chunk(pdu_nufft_plan_t* p, const float2* kdata, float2* ima
         NufftDims dc = dims_of(p);          // the cropped result is a dense [n0][n1] "grid"
         dc.k0 = dc.n0;
         dc.k1 = dc.n1;
+        if (sg) return launch_smaps_grad(p, U, dc, coils, scale, *sg, st);
         crop_apod_kernel<<<stream_grid(total), 256, 0, st>>>(U, smaps, image, p->d_s0, p->d_s1, dc, coils, smaps_batch, scale,
                                                              total);
         PDU_LAUNCHED();
@@ -1935,6 +2041,7 @@ static int nufft_adj_chunk(pdu_nufft_plan_t* p, const float2* kdata, float2* ima
         NufftDims dc = d;          // the cropped result is a dense [n0][n1] "grid"
         dc.k0 = d.n0;
         dc.k1 = d.n1;
+        if (sg) return launch_smaps_grad(p, U, dc, coils, scale, *sg, st);
         crop_apod_kernel<<<stream_grid(total), 256, 0, st>>>(U, smaps, image, p->d_s0, p->d_s1, dc, coils, smaps_batch, scale,
                                                              total);
         PDU_LAUNCHED();
@@ -1942,6 +2049,7 @@ static int nufft_adj_chunk(pdu_nufft_plan_t* p, const float2* kdata, float2* ima
     }
     rc = run_fft(p, grid, planes, CUFFT_INVERSE, st);
     if (rc) return rc;
+    if (sg) return launch_smaps_grad(p, grid, dims_of(p), coils, scale, *sg, st);
     crop_apod_kernel<<<stream_grid(total), 256, 0, st>>>(grid, smaps, image, p->d_s0, p->d_s1, dims_of(p), coils, smaps_batch,
                                                          scale, total);
     PDU_LAUNCHED();
@@ -2071,6 +2179,53 @@ int pdu_nufft_adj_binned_c64(pdu_nufft_plan_t* p, const float* kdata, float* ima
     }
     return fused_adjoint(p, kdata, image, smaps, kweight, batch, coils, smaps_batch, m, scale, bins, flags, workspace,
                          (cudaStream_t)stream);
+}
+
+int pdu_nufft_adj_smaps_grad_c64(pdu_nufft_plan_t* p, const float* kdata, const float* q, float* gs, const float* omega,
+                                 const void* csr, const void* bins, const float* kweight, int batch, int coils,
+                                 int smaps_batch, long m, float scale, int flags, int accumulate, void* workspace,
+                                 size_t workspace_bytes, pdu_stream_t stream) {
+    const char* who = "pdu_nufft_adj_smaps_grad_c64";
+    int rc = check_call(p, kdata, gs, bins ? bins : (const void*)omega, batch, coils, smaps_batch, q, m, who);
+    if (rc) return rc;
+    PDU_REQUIRE(q != nullptr, "%s: q is null", who);
+    PDU_REQUIRE((flags & ~(PDU_NUFFT_IMAGE_SPLIT | PDU_NUFFT_KDATA_SPLIT)) == 0, "%s: unknown flags %d", who, flags);
+    PDU_CHECK_DEVICE(who);
+    const int q_split = (flags & PDU_NUFFT_IMAGE_SPLIT) ? 1 : 0, per_batch = smaps_batch == 1 ? 0 : 1;
+    if (bins) {
+        if (!fused_supported(p)) {
+            set_error("%s: grid %d x %d (J = %d) has no fused path; pass bins = NULL", who, p->k0, p->k1, p->J);
+            return PDU_EUNSUPPORTED;
+        }
+        const size_t need = fused_workspace_bytes(p, batch * coils, m);
+        if (!workspace || workspace_bytes < need || ((uintptr_t)workspace & 255)) {
+            set_error("%s: workspace of %zu bytes (256-byte aligned) required, got %zu", who, need,
+                      workspace ? workspace_bytes : (size_t)0);
+            return PDU_ENOMEM;
+        }
+        const SmapsGrad sg{(float2*)gs, q, batch, per_batch, q_split, accumulate ? 1 : 0, 1.f};
+        return fused_adjoint(p, kdata, nullptr, nullptr, kweight, batch, coils, 1, m, scale, bins, flags, workspace,
+                             (cudaStream_t)stream, &sg);
+    }
+    // the plain-omega / CSR paths take complex64 kdata without weights, as pdu_nufft_adj_csr_c64 does
+    PDU_REQUIRE(!kweight && !(flags & PDU_NUFFT_KDATA_SPLIT), "%s: kweight and split kdata need the row-binned path (bins)", who);
+    const int cb = batch_chunk(p, batch, coils);
+    const size_t need = pdu_nufft_workspace_bytes(p, cb * coils);
+    if (!workspace || workspace_bytes < need) {
+        set_error("%s: workspace of %zu bytes required, got %zu", who, need, workspace ? workspace_bytes : (size_t)0);
+        return PDU_ENOMEM;
+    }
+    const long plane = (long)p->n0 * p->n1;
+    for (int b0 = 0; b0 < batch; b0 += cb) {
+        const int nb = b0 + cb <= batch ? cb : batch - b0;
+        // a shared map's sum continues from chunk to chunk
+        const SmapsGrad sg{(float2*)gs + (per_batch ? (long)b0 * coils * plane : 0), q + (long)b0 * 2 * plane, nb, per_batch,
+                           q_split, (accumulate || (!per_batch && b0 > 0)) ? 1 : 0, 1.f};
+        rc = nufft_adj_chunk(p, (const float2*)kdata + (long)b0 * coils * m, nullptr, omega, nullptr, nb, coils, 1, m, scale,
+                             (float2*)workspace, csr, (cudaStream_t)stream, &sg);
+        if (rc) return rc;
+    }
+    return PDU_OK;
 }
 
 int pdu_complex_from_split_f32(const float* split, float* out, const float* weight, long planes, long n, pdu_stream_t stream) {
@@ -2211,6 +2366,46 @@ int pdu_toep_apply_c64(pdu_nufft_plan_t* p, const float* image, float* out, cons
                                 smaps ? (const float2*)smaps + b0 * smap_b : nullptr, nb, coils, smaps_batch == 1 ? 1 : nb,
                                 conj_kernel ? 1 : 0, (float2*)ws, (cudaStream_t)stream);
         if (rc) return rc;
+    }
+    return PDU_OK;
+}
+
+int pdu_toep_smaps_grad_c64(pdu_nufft_plan_t* p, const float* x, const float* g, float* gs, const float* kernel,
+                            int kernel_batch, const float* smaps, int batch, int coils, int smaps_batch, int conj_kernel,
+                            float out_scale, int accumulate, void* ws, size_t ws_bytes, pdu_stream_t stream) {
+    PDU_REQUIRE(p != nullptr, "pdu_toep_smaps_grad_c64: plan is null");
+    PDU_REQUIRE(p->toep, "pdu_toep_smaps_grad_c64: not a Toeplitz plan (use pdu_toep_plan_create)");
+    PDU_REQUIRE(x && g && gs && kernel && smaps, "pdu_toep_smaps_grad_c64: null pointer");
+    PDU_REQUIRE(batch > 0 && coils > 0 && coils <= 65535, "pdu_toep_smaps_grad_c64: batch must be > 0 and coils in 1..65535");
+    PDU_REQUIRE(kernel_batch == 1 || kernel_batch == batch, "pdu_toep_smaps_grad_c64: kernel batch must be 1 or batch");
+    PDU_REQUIRE(smaps_batch == 1 || smaps_batch == batch, "pdu_toep_smaps_grad_c64: smaps batch must be 1 or batch");
+    const int cb = tz_batch_chunk(p, batch, coils);
+    const size_t need = pdu_toep_workspace_bytes(p, cb * coils);
+    if (!ws || ws_bytes < need) {
+        set_error("pdu_toep_smaps_grad_c64: workspace of %zu bytes required, got %zu", need, ws ? ws_bytes : (size_t)0);
+        return PDU_ENOMEM;
+    }
+    int dev = -1;
+    PDU_CUDA(cudaGetDevice(&dev));
+    PDU_REQUIRE(dev == p->device, "pdu_toep_smaps_grad_c64: plan was created on device %d, current device is %d", p->device, dev);
+    PDU_CHECK_DEVICE("pdu_toep_smaps_grad_c64");
+    const long plane = (long)p->n0 * p->n1, cells = (long)p->k0 * p->k1;
+    const int per_batch = smaps_batch == 1 ? 0 : 1;
+    const long smap_b = per_batch ? coils * plane : 0;
+    for (int b0 = 0; b0 < batch; b0 += cb) {
+        const int nb = b0 + cb <= batch ? cb : batch - b0;
+        // term 0: T(S_c x_b) conj(g_b); term 1: T^H(S_c g_b) conj(x_b), added on top
+        for (int term = 0; term < 2; ++term) {
+            const float* image = term ? g : x;
+            const float* q = term ? x : g;
+            const int acc = (accumulate || term == 1 || (!per_batch && b0 > 0)) ? 1 : 0;
+            const SmapsGrad sg{(float2*)gs + b0 * smap_b, q + 2 * b0 * plane, nb, per_batch, 0, acc, out_scale};
+            int rc = tz_apply_chunk(p, (const float2*)image + b0 * plane, nullptr,
+                                    (const float2*)kernel + (kernel_batch == 1 ? 0 : b0 * cells), kernel_batch == 1 ? 1 : nb,
+                                    (const float2*)smaps + b0 * smap_b, nb, coils, per_batch ? nb : 1,
+                                    (conj_kernel != 0) != (term == 1) ? 1 : 0, (float2*)ws, (cudaStream_t)stream, nullptr, &sg);
+            if (rc) return rc;
+        }
     }
     return PDU_OK;
 }

@@ -90,12 +90,29 @@ static inline NufftDims dims_of(const pdu_nufft_plan* p) {
 
 static inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 
+// The coil-map gradient ending of an adjoint (pdu_nufft_adj_smaps_grad_c64, pdu_toep_smaps_grad_c64): instead of
+// combining the coils of the cropped planes U [batch][coils], gs[s][c] (+)= scale' * sum_{b : s(b) = s} U[b][c] conj(q[b]),
+// s(b) = 0 with one shared map, b with one map per batch element; b runs in increasing order, in registers.
+struct SmapsGrad {
+    float2* gs;           // [per_batch ? batch : 1][coils][n0][n1] of this chunk
+    const float* q;       // [batch][n0][n1] complex64, or [batch][2][n0][n1] float32 (q_split)
+    int batch;            // batch elements of this chunk
+    int per_batch;        // 0: every b sums into gs[0]; 1: b writes gs[b]
+    int q_split;
+    int accumulate;       // add to gs instead of overwriting it
+    float scale;          // multiplies the transform's own scale (-1 for the conjugate-gradient solve)
+};
+int launch_smaps_grad(pdu_nufft_plan* p, const float2* U, NufftDims d, int coils, float scale, const SmapsGrad& sg,
+                      cudaStream_t st);
+
 // nufft_fused.cu
 bool fused_supported(const pdu_nufft_plan* p);
 size_t fused_workspace_bytes(const pdu_nufft_plan* p, int planes, long m);
 int fused_forward(pdu_nufft_plan* p, const float* image, float* kdata, const float* smaps, int batch, int coils, int smaps_batch,
                   long m, float scale, const void* bins, int flags, void* ws, cudaStream_t st);
+// sg: end in smaps_grad_kernel (smaps null) instead of writing the image
 int fused_adjoint(pdu_nufft_plan* p, const float* kdata, float* image, const float* smaps, const float* kweight, int batch,
-                  int coils, int smaps_batch, long m, float scale, const void* bins, int flags, void* ws, cudaStream_t st);
+                  int coils, int smaps_batch, long m, float scale, const void* bins, int flags, void* ws, cudaStream_t st,
+                  const SmapsGrad* sg = nullptr);
 
 }  // namespace pdu

@@ -643,7 +643,7 @@ int launch_crop_apod(pdu_nufft_plan* p, const float2* U, const float2* smaps, fl
 template <int K, int PG>
 static int fused_adjoint_k(pdu_nufft_plan* p, const float* kdata, float* image, const float2* smaps, const float* kweight,
                            int batch, int coils, int smaps_batch, long m, float scale, const BinsView& v, int flags, void* ws,
-                           cudaStream_t st) {
+                           cudaStream_t st, const SmapsGrad* sg) {
     constexpr int FZ_SEQ_COLS = fz_seq<K>();
     const NufftDims d = dims_of(p);
     const int planes = batch * coils;
@@ -661,7 +661,7 @@ static int fused_adjoint_k(pdu_nufft_plan* p, const float* kdata, float* image, 
     }
     const int split = (flags & PDU_NUFFT_IMAGE_SPLIT) ? 1 : 0;
     const dim3 gc((unsigned)cdiv(d.n1, FZ_SEQ_COLS), (unsigned)planes);
-    if (!smaps) {
+    if (!smaps && !sg) {
         fz_cols_adj_kernel<K, FZ_SEQ_COLS><<<gc, FZ_SEQ_COLS * FastFft<K>::TPS, fz_cols_smem<K>(), st>>>(
             T, image, p->d_s0, p->d_s1, p->d_w0, d, scale, 1, split);
         PDU_LAUNCHED();
@@ -669,12 +669,18 @@ static int fused_adjoint_k(pdu_nufft_plan* p, const float* kdata, float* image, 
         fz_cols_adj_kernel<K, FZ_SEQ_COLS><<<gc, FZ_SEQ_COLS * FastFft<K>::TPS, fz_cols_smem<K>(), st>>>(
             T, (float*)U, p->d_s0, p->d_s1, p->d_w0, d, 1.f, 0, 0);
         PDU_LAUNCHED();
-        int rc = launch_crop_apod(p, U, smaps, (float2*)image, batch, coils, smaps_batch, scale, split, st);
+        NufftDims dc = d;          // the cropped result is a dense [n0][n1] "grid"
+        dc.k0 = d.n0;
+        dc.k1 = d.n1;
+        int rc = sg ? launch_smaps_grad(p, U, dc, coils, scale, *sg, st)
+                    : launch_crop_apod(p, U, smaps, (float2*)image, batch, coils, smaps_batch, scale, split, st);
         if (rc) return rc;
     }
-    note_kernel(OP_NUFFT_ADJ, "fz_rows_adj_kernel<%d,%d,%d> (in-row gather + inverse row FFT) + fz_cols_adj_kernel<%d,%d>%s "
-                "(%d planes of %dx%d, M=%ld; own register-resident pruned FFT, grid never materialised, no atomics)", K, PG, FZ_EC, K,
-                FZ_SEQ_COLS, smaps ? " + crop_apod_kernel (coil combine)" : " (crop + apodisation fused)", planes, K, K, m);
+    note_kernel(sg ? OP_SMAPS_GRAD : OP_NUFFT_ADJ, "fz_rows_adj_kernel<%d,%d,%d> (in-row gather + inverse row FFT) + "
+                "fz_cols_adj_kernel<%d,%d>%s (%d planes of %dx%d, M=%ld; own register-resident pruned FFT, grid never "
+                "materialised, no atomics)", K, PG, FZ_EC, K, FZ_SEQ_COLS,
+                sg ? " + smaps_grad_kernel (fused path)" : (smaps ? " + crop_apod_kernel (coil combine)" : " (crop + apodisation fused)"),
+                planes, K, K, m);
     return PDU_OK;
 }
 
@@ -697,18 +703,19 @@ int fused_forward(pdu_nufft_plan* p, const float* image, float* kdata, const flo
 }
 
 int fused_adjoint(pdu_nufft_plan* p, const float* kdata, float* image, const float* smaps, const float* kweight, int batch,
-                  int coils, int smaps_batch, long m, float scale, const void* bins, int flags, void* ws, cudaStream_t st) {
+                  int coils, int smaps_batch, long m, float scale, const void* bins, int flags, void* ws, cudaStream_t st,
+                  const SmapsGrad* sg) {
     int rc = check_bins(p, bins, m, "pdu_nufft_adj_binned_c64");
     if (rc) return rc;
     const BinsView v = bins_layout(p, m, const_cast<void*>(bins), false);
     const float2* sm = (const float2*)smaps;
     const int pg = option(OPT_NUFFT_ADJ) == 8 ? 8 : (option(OPT_NUFFT_ADJ) == 2 ? 2 : 4);     // A/B: planes per CTA (default 4)
     switch (p->k0) {
-        case 256: return pg == 8 ? fused_adjoint_k<256, 8>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : (pg == 2 ? fused_adjoint_k<256, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : fused_adjoint_k<256, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st));
-        case 512: return pg == 8 ? fused_adjoint_k<512, 8>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : (pg == 2 ? fused_adjoint_k<512, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : fused_adjoint_k<512, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st));
-        case 640: return pg == 8 ? fused_adjoint_k<640, 8>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : (pg == 2 ? fused_adjoint_k<640, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : fused_adjoint_k<640, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st));
-        case 1024: return pg == 8 ? fused_adjoint_k<1024, 8>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : (pg == 2 ? fused_adjoint_k<1024, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : fused_adjoint_k<1024, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st));
-        case 2048: return pg == 2 ? fused_adjoint_k<2048, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : fused_adjoint_k<2048, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st);
+        case 256: return pg == 8 ? fused_adjoint_k<256, 8>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : (pg == 2 ? fused_adjoint_k<256, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : fused_adjoint_k<256, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg));
+        case 512: return pg == 8 ? fused_adjoint_k<512, 8>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : (pg == 2 ? fused_adjoint_k<512, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : fused_adjoint_k<512, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg));
+        case 640: return pg == 8 ? fused_adjoint_k<640, 8>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : (pg == 2 ? fused_adjoint_k<640, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : fused_adjoint_k<640, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg));
+        case 1024: return pg == 8 ? fused_adjoint_k<1024, 8>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : (pg == 2 ? fused_adjoint_k<1024, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : fused_adjoint_k<1024, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg));
+        case 2048: return pg == 2 ? fused_adjoint_k<2048, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : fused_adjoint_k<2048, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg);
     }
     set_error("pdu_nufft_adj_binned_c64: grid %d has no fused path", p->k0);
     return PDU_EUNSUPPORTED;

@@ -12,7 +12,7 @@ the reference reaches the library through its unmounted MRI branch, /root/refere
 image: complex64 [B, C, N0, N1]; omega: float32 [2, M] radians (or [B, 2, M]); data: complex64
 [B, C, M].  With smaps [1 or B, coils, N0, N1] the forward expands a one-channel image to the
 coils and the adjoint combines them.  Both directions are differentiable (each is the other's
-conjugate transpose).  The modules register no parameters and no persistent buffers, so a model
+conjugate transpose), in the maps too.  The modules register no parameters and no persistent buffers, so a model
 containing them has the same state_dict as one without.
 
 Everything numeric happens in libpdu_b200.so (pd_unet_b200/csrc/nufft.cu).  No CPU path.
@@ -383,6 +383,48 @@ class _Plan:
                                           ws.numel(), stream_ptr()), "pdu_nufft_adj_c64")
         return out
 
+    def smaps_grad(self, data, omega, q, gs, norm, split: bool = False, kweight: Optional[torch.Tensor] = None,
+                   accumulate: bool = False) -> None:
+        """gs [1 or B, coils, N0, N1] (+)= sum over b of the un-combined adjoint of data[b] (as adjoint() would run it)
+        times conj(q[b]); q is the image side [B, 1, N0, N1] (split: [B, 2, N0, N1] float32).  A shared map (gs[0])
+        sums the batch in increasing order, carried from chunk to chunk."""
+        omega = self._omega(omega)
+        data, q = data.contiguous(), q.contiguous()
+        if kweight is not None:
+            kweight = require_cuda(kweight, torch.float32, "kweight").reshape(-1)
+        B, M = data.shape[0], data.shape[2]
+        coils = data.shape[1] // 2 if split else data.shape[1]
+        per_batch = gs.shape[0] != 1
+        if B == 0 or M == 0:
+            if not accumulate:
+                gs.zero_()
+            return
+        L, h = lib(), self.handle(data.device)
+        bins = self._bins_for(omega, B * coils, adjoint=True, split=split)
+        if bins is not None:
+            flags = (NUFFT_IMAGE_SPLIT | NUFFT_KDATA_SPLIT) if split else 0
+            for b0, b1 in self._chunks(L, h, B, coils, M):
+                nb = b1 - b0
+                ws = torch.empty(L.pdu_nufft_binned_workspace_bytes(h, nb * coils, M), dtype=torch.uint8, device=data.device)
+                g = gs[b0:b1] if per_batch else gs
+                check(L.pdu_nufft_adj_smaps_grad_c64(h, data[b0:b1].data_ptr(), q[b0:b1].data_ptr(), g.data_ptr(), None, None,
+                                                     bins.data_ptr(), kweight.data_ptr() if kweight is not None else None, nb,
+                                                     coils, g.shape[0], M, self.scale(norm), flags,
+                                                     1 if (accumulate or (b0 > 0 and not per_batch)) else 0, ws.data_ptr(),
+                                                     ws.numel(), stream_ptr()), "pdu_nufft_adj_smaps_grad_c64")
+            return
+        # generic path: complex64 kdata with the weights applied, as adjoint() feeds pdu_nufft_adj_csr_c64
+        if split:
+            data = self._split_to_complex(data, kweight)
+        elif kweight is not None:
+            data = data * kweight
+        ws = torch.empty(L.pdu_nufft_workspace_bytes(h, B * coils), dtype=torch.uint8, device=data.device)
+        csr = self._csr_for(omega, B * coils)
+        check(L.pdu_nufft_adj_smaps_grad_c64(h, data.data_ptr(), q.data_ptr(), gs.data_ptr(), omega.data_ptr(),
+                                             csr.data_ptr() if csr is not None else None, None, None, B, coils, gs.shape[0], M,
+                                             self.scale(norm), NUFFT_IMAGE_SPLIT if split else 0, 1 if accumulate else 0,
+                                             ws.data_ptr(), ws.numel(), stream_ptr()), "pdu_nufft_adj_smaps_grad_c64")
+
     def interp(self, grid, omega):
         grid = require_cuda(grid, torch.complex64, "grid")
         if grid.dim() != 4 or tuple(grid.shape[-2:]) != self.grid_size:
@@ -432,11 +474,31 @@ def _per_trajectory(fn, x, omega, smaps, *rest):
     return torch.cat(outs, dim=0)
 
 
+def _nufft_smaps_grad(plan: _Plan, data, omega, q, smaps, norm, split, kweight) -> torch.Tensor:
+    """The coil-map gradient sum_b A^H(w data[b, c]) conj(q[b]) in the shape of smaps (3-D or 4-D); a batched omega runs
+    per trajectory, a shared map summing the batch in increasing order."""
+    sm = smaps if smaps.dim() == 4 else smaps[None]
+    gs = torch.empty(sm.shape, dtype=torch.complex64, device=data.device)
+    with torch.cuda.device(data.device):
+        if omega.dim() == 2:
+            plan.smaps_grad(data, omega, q, gs, norm, split, kweight)
+        else:
+            for b in range(data.shape[0]):
+                plan.smaps_grad(data[b:b + 1], omega[b], q[b:b + 1], gs if gs.shape[0] == 1 else gs[b:b + 1], norm, split,
+                                kweight, accumulate=gs.shape[0] == 1 and b > 0)
+    return gs.reshape(smaps.shape)
+
+
 class _NufftFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, omega, smaps, plan, norm, adjoint, split=False, kweight=None):
         ctx.plan, ctx.norm, ctx.adjoint, ctx.split, ctx.kweight = plan, norm, adjoint, split, kweight
-        ctx.save_for_backward(omega, smaps) if smaps is not None else ctx.save_for_backward(omega)
+        if smaps is None:
+            ctx.save_for_backward(omega)
+        elif ctx.needs_input_grad[2]:        # the map gradient pairs the input with the incoming gradient
+            ctx.save_for_backward(omega, smaps, x)
+        else:
+            ctx.save_for_backward(omega, smaps)
         if adjoint:
             return _per_trajectory(plan.adjoint, x, omega, smaps, norm, split, kweight)
         return _per_trajectory(plan.forward, x, omega, smaps, norm, split)
@@ -445,13 +507,24 @@ class _NufftFn(torch.autograd.Function):
     def backward(ctx, grad):
         saved = ctx.saved_tensors
         omega, smaps = saved[0], (saved[1] if len(saved) > 1 else None)
-        if ctx.adjoint:       # x = A^H (w y)  =>  dy = w A dx
-            g = _per_trajectory(ctx.plan.forward, grad.contiguous(), omega, smaps, ctx.norm, ctx.split)
-            if ctx.kweight is not None:
-                g = g * ctx.kweight.reshape(-1)
-        else:
-            g = _per_trajectory(ctx.plan.adjoint, grad.contiguous(), omega, smaps, ctx.norm, ctx.split)
-        return g, None, None, None, None, None, None, None
+        grad = grad.contiguous()
+        g = gs = None
+        if ctx.needs_input_grad[0] or not ctx.needs_input_grad[2]:
+            if ctx.adjoint:       # x = A^H (w y)  =>  dy = w A dx
+                g = _per_trajectory(ctx.plan.forward, grad, omega, smaps, ctx.norm, ctx.split)
+                if ctx.kweight is not None:
+                    g = g * ctx.kweight.reshape(-1)
+            else:
+                g = _per_trajectory(ctx.plan.adjoint, grad, omega, smaps, ctx.norm, ctx.split)
+        if smaps is not None and ctx.needs_input_grad[2]:
+            x = saved[2]
+            # forward  y[b, c] = A(S_c x_b):              gS_c = sum_b A^H(g[b, c]) conj(x_b)
+            # adjoint  x_b = sum_c conj(S_c) A^H(w y[b, c]):  gS_c = sum_b A^H(w y[b, c]) conj(g_b)
+            if ctx.adjoint:
+                gs = _nufft_smaps_grad(ctx.plan, x, omega, grad, smaps, ctx.norm, ctx.split, ctx.kweight)
+            else:
+                gs = _nufft_smaps_grad(ctx.plan, grad, omega, x, smaps, ctx.norm, ctx.split, None)
+        return g, None, gs, None, None, None, None, None
 
 
 class _InterpFn(torch.autograd.Function):
@@ -487,7 +560,11 @@ class _KbModule(nn.Module):
 
 
 class KbNufft(_KbModule):
-    """image [B, C, N0, N1] -> k-space samples [B, C (or coils), M].  [RECALL] torchkbnufft.KbNufft."""
+    """image [B, C, N0, N1] -> k-space samples [B, C (or coils), M].  [RECALL] torchkbnufft.KbNufft.
+
+    Differentiable in the image and in smaps: grad_S[c] = sum_b A^H(g[b, c]) conj(x_b) over the batch elements sharing
+    a map, one adjoint launch set ending in the library's map-gradient kernel; maps that need no gradient cost
+    nothing extra."""
 
     def forward(self, image, omega, interp_mats=None, smaps=None, norm: Optional[str] = None, split: bool = False):
         """split=True (an extension): image float32 [B, 2 C, N0, N1] with (re, im) as neighbouring channels ->
@@ -497,7 +574,10 @@ class KbNufft(_KbModule):
 
 
 class KbNufftAdjoint(_KbModule):
-    """samples [B, C, M] -> image [B, C (or 1), N0, N1].  [RECALL] torchkbnufft.KbNufftAdjoint."""
+    """samples [B, C, M] -> image [B, C (or 1), N0, N1].  [RECALL] torchkbnufft.KbNufftAdjoint.
+
+    Differentiable in the samples and in smaps: grad_S[c] = sum_b A^H(kweight y[b, c]) conj(g_b) over the batch
+    elements sharing a map (the un-combined adjoint of the input, reduced by the library's map-gradient kernel)."""
 
     def forward(self, data, omega, interp_mats=None, smaps=None, norm: Optional[str] = None, split: bool = False,
                 kweight: Optional[torch.Tensor] = None):
@@ -641,19 +721,49 @@ def _toep_apply(image: torch.Tensor, kernel: torch.Tensor, smaps: Optional[torch
     return out
 
 
+def _toep_smaps_grad(x: torch.Tensor, g: torch.Tensor, kernel: torch.Tensor, smaps: torch.Tensor, out_scale: float) -> torch.Tensor:
+    """out_scale * sum_b [T(S_c x_b) conj(g_b) + T^H(S_c g_b) conj(x_b)], the coil-map gradient of ToepNufft at (x, g), in
+    the shape of smaps."""
+    x, kernel, sm, coils, sb = _toep_args(x, kernel, smaps)
+    g = require_cuda(g, torch.complex64, "grad").contiguous()
+    B, _, N0, N1 = x.shape
+    gs = torch.empty(sm.shape, dtype=torch.complex64, device=x.device)
+    if B == 0:
+        return gs.zero_().reshape(smaps.shape)
+    with torch.cuda.device(x.device):
+        tp = _toep_plan((N0, N1))
+        h = tp.handle(x.device)
+        ws = torch.empty(tp.workspace_bytes(h, B, coils), dtype=torch.uint8, device=x.device)
+        check(lib().pdu_toep_smaps_grad_c64(h, x.data_ptr(), g.data_ptr(), gs.data_ptr(), kernel.data_ptr(), kernel.shape[0],
+                                            sm.data_ptr(), B, coils, sb, 0, out_scale, 0, ws.data_ptr(), ws.numel(),
+                                            stream_ptr()), "pdu_toep_smaps_grad_c64")
+    return gs.reshape(smaps.shape)
+
+
 class _ToepFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, kernel, smaps):
-        ctx.save_for_backward(kernel, smaps) if smaps is not None else ctx.save_for_backward(kernel)
+        if smaps is None:
+            ctx.save_for_backward(kernel)
+        elif ctx.needs_input_grad[2]:
+            ctx.save_for_backward(kernel, smaps, x)
+        else:
+            ctx.save_for_backward(kernel, smaps)
         return _toep_apply(x, kernel, smaps, False)
 
     @staticmethod
     def backward(ctx, grad):
         saved = ctx.saved_tensors
         kernel, smaps = saved[0], (saved[1] if len(saved) > 1 else None)
-        # T = P^T F^-1 diag(k) F P (with coil maps: sum_c S_c^H T S_c), so T^H is the same apply with conj(k): exact for
-        # any complex kernel
-        return _toep_apply(grad.contiguous(), kernel, smaps, True), None, None
+        grad = grad.contiguous()
+        gx = gs = None
+        if ctx.needs_input_grad[0] or not ctx.needs_input_grad[2]:
+            # T = P^T F^-1 diag(k) F P (with coil maps: sum_c S_c^H T S_c), so T^H is the same apply with conj(k): exact
+            # for any complex kernel
+            gx = _toep_apply(grad, kernel, smaps, True)
+        if smaps is not None and ctx.needs_input_grad[2]:
+            gs = _toep_smaps_grad(saved[2], grad, kernel, smaps, 1.0)
+        return gx, None, gs
 
 
 class ToepNufft(nn.Module):
@@ -667,7 +777,9 @@ class ToepNufft(nn.Module):
     norm is accepted with torchkbnufft's values and does not change the result [RECALL]: the FFT pair's normalisations
     multiply to the same total either way, and the NUFFT's scaling lives in the kernel (calc_toeplitz_kernel(norm=...)).
     Differentiable in the image (the backward is the same apply with the conjugate kernel, exact for any complex
-    kernel); no gradient flows to the kernel.  No parameters, no buffers."""
+    kernel) and in smaps: grad_S[c] = sum_b [T(S_c x_b) conj(g_b) + T^H(S_c g_b) conj(x_b)], two apply launch sets
+    whose last pass walks the batch instead of the coils.  No gradient flows to the kernel.  No parameters, no
+    buffers."""
 
     def forward(self, image, kernel, smaps=None, norm: Optional[str] = None):
         _check_norm(norm)
@@ -787,11 +899,14 @@ class _ToepCgFn(torch.autograd.Function):
         # implicit differentiation of x = M^-1 b, M = T + lam I: grad_b = M^-H g (the conj-kernel system), and
         # dx / dlam = -M^-1 x, so grad_lam = -Re <M^-H g, x> per lam entry
         gb = _toep_cg_solve(g.contiguous(), kernel, smaps, lam_dev, lam_count, None, max_iter, tol, True)
-        glam = None
+        glam = gs = None
         if ctx.needs_input_grad[1]:
             prod = (gb.conj() * x).real
             glam = -(prod.sum() if lam_count == 1 else prod.sum(dim=(1, 2, 3))).reshape(ctx.lam_shape)
-        return (gb if ctx.needs_input_grad[0] else None), glam, None, None, None, None, None, None, None
+        if smaps is not None and ctx.needs_input_grad[3]:
+            # dx = -M^-1 (dM) x, so grad_S = -G(x, M^-H g) with G the ToepNufft map gradient
+            gs = _toep_smaps_grad(x, gb, kernel, smaps, -1.0)
+        return (gb if ctx.needs_input_grad[0] else None), glam, None, gs, None, None, None, None, None
 
 
 def toep_cg(b: torch.Tensor, kernel: torch.Tensor, smaps: Optional[torch.Tensor] = None, lam=0.0,
@@ -822,8 +937,9 @@ def toep_cg(b: torch.Tensor, kernel: torch.Tensor, smaps: Optional[torch.Tensor]
 
     Differentiable in b and in a tensor lam by implicit differentiation (the MoDL convention): grad_b solves the
     adjoint system (conj kernel) with the same lam, max_iter and tol, and grad_lam = -Re sum conj(grad_b) x per lam
-    entry.  That is the gradient of the exact solution, which x approximates, not of the truncated iteration.  No
-    gradient reaches kernel, smaps or x0."""
+    entry.  That is the gradient of the exact solution, which x approximates, not of the truncated iteration.  With
+    smaps requiring a gradient, grad_S = -G(x, grad_b), G the ToepNufft map gradient (the adjoint system is solved even
+    when b needs no gradient).  No gradient reaches kernel or x0."""
     if isinstance(max_iter, bool) or not isinstance(max_iter, int) or max_iter < 0:
         raise ValueError(f"max_iter must be an int >= 0, got {max_iter!r}")
     if isinstance(tol, bool) or not isinstance(tol, (int, float)) or not float(tol) >= 0.0:

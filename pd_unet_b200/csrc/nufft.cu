@@ -24,6 +24,7 @@
 #include <math.h>
 
 #include <algorithm>
+#include <climits>
 #include <initializer_list>
 #include <map>
 #include <mutex>
@@ -1105,20 +1106,15 @@ __global__ void __launch_bounds__(256)
     }
 }
 
-// cropped planes U [planes][n0][n1] -> image (x apodisation x scale, x conj(smaps) summed over coils); nufft_fused.cu
-int launch_crop_apod(pdu_nufft_plan* p, const float2* U, const float2* smaps, float2* image, int out_planes, int coils,
-                     int smaps_batch, float scale, int split, cudaStream_t st) {
-    NufftDims dc = dims_of(p);          // the cropped result is a dense [n0][n1] "grid"
-    dc.k0 = dc.n0;
-    dc.k1 = dc.n1;
+int launch_crop_apod(pdu_nufft_plan* p, const float2* U, NufftDims d, const float2* smaps, float2* image, int out_planes,
+                     int coils, int smaps_batch, float scale, int split, cudaStream_t st) {
     const long total = (long)out_planes * p->n0 * p->n1;
-    crop_apod_kernel<<<stream_grid(total), 256, 0, st>>>(U, smaps, image, p->d_s0, p->d_s1, dc, coils, smaps_batch, scale, total,
+    crop_apod_kernel<<<stream_grid(total), 256, 0, st>>>(U, smaps, image, p->d_s0, p->d_s1, d, coils, smaps_batch, scale, total,
                                                          split);
     PDU_LAUNCHED();
     return PDU_OK;
 }
 
-// grid or cropped planes U [batch][coils] with plane geometry d (k0 x k1 planes, the n0 x n1 corner kept) -> sg.gs
 int launch_smaps_grad(pdu_nufft_plan* p, const float2* U, NufftDims d, int coils, float scale, const SmapsGrad& sg,
                       cudaStream_t st) {
     const long total = (long)(sg.per_batch ? sg.batch : 1) * coils * p->n0 * p->n1;
@@ -1128,6 +1124,14 @@ int launch_smaps_grad(pdu_nufft_plan* p, const float2* U, NufftDims d, int coils
     return PDU_OK;
 }
 
+static int check_plan_device(const pdu_nufft_plan* p, const char* who) {
+    int dev = -1;
+    PDU_CUDA(cudaGetDevice(&dev));
+    PDU_REQUIRE(dev == p->device, "%s: plan was created on device %d, current device is %d", who, p->device, dev);
+    return PDU_OK;
+}
+
+// the argument checks of the NUFFT entry points
 static int check_call(const pdu_nufft_plan* p, const void* a, const void* b, const void* omega, int batch, int coils,
                       int smaps_batch, const void* smaps, long m, const char* who) {
     PDU_REQUIRE(p != nullptr, "%s: plan is null", who);
@@ -1136,9 +1140,47 @@ static int check_call(const pdu_nufft_plan* p, const void* a, const void* b, con
     PDU_REQUIRE(batch > 0 && coils > 0 && m > 0, "%s: batch, coils and m must be > 0", who);
     PDU_REQUIRE((long)batch * coils <= 65535L * 64, "%s: too many planes", who);
     if (smaps) PDU_REQUIRE(smaps_batch == 1 || smaps_batch == batch, "%s: smaps batch must be 1 or batch", who);
-    int dev = -1;
-    PDU_CUDA(cudaGetDevice(&dev));
-    PDU_REQUIRE(dev == p->device, "%s: plan was created on device %d, current device is %d", who, p->device, dev);
+    return check_plan_device(p, who);
+}
+
+// the argument checks of the pdu_toep_* entry points; ptrs: every pointer the entry point requires is set
+static int check_toep_call(const pdu_nufft_plan* p, bool ptrs, int batch, int coils, int kernel_batch, const void* smaps,
+                           int smaps_batch, const char* who) {
+    PDU_REQUIRE(p != nullptr, "%s: plan is null", who);
+    PDU_REQUIRE(p->toep, "%s: not a Toeplitz plan (use pdu_toep_plan_create)", who);
+    PDU_REQUIRE(ptrs, "%s: null pointer", who);
+    PDU_REQUIRE(batch > 0 && coils > 0 && coils <= 65535, "%s: batch must be > 0 and coils in 1..65535", who);
+    PDU_REQUIRE(kernel_batch == 1 || kernel_batch == batch, "%s: kernel batch must be 1 or batch", who);
+    if (smaps) PDU_REQUIRE(smaps_batch == 1 || smaps_batch == batch, "%s: smaps batch must be 1 or batch", who);
+    return check_plan_device(p, who);
+}
+
+// the caller's workspace: at least `need` bytes, 256-byte aligned if `aligned`; `code` when it is not
+static int check_workspace(const char* who, const void* ws, size_t bytes, size_t need, bool aligned, int code) {
+    if (ws && bytes >= need && !(aligned && ((uintptr_t)ws & 255))) return PDU_OK;
+    set_error("%s: workspace of %zu bytes%s required, got %zu", who, need, aligned ? " (256-byte aligned)" : "",
+              ws ? bytes : (size_t)0);
+    return code;
+}
+
+// A call is cut into batch chunks so that the scratch (plane_bytes per plane) stays under 512 MB and a chunk has at most
+// plane_cap planes.  Measured on B200: chunking the NUFFT down to L2-resident grids (56 MB) does NOT pay -- cuFFT runs at
+// ~3 TB/s either way and the gather / scatter lose parallelism -- so the budget only caps the workspace.
+static int batch_chunk(size_t plane_bytes, long plane_cap, int batch, int coils) {
+    long planes = (long)(((size_t)512 << 20) / plane_bytes);
+    if (planes > plane_cap) planes = plane_cap;
+    long cb = planes / coils;
+    if (cb < 1) cb = 1;
+    return (int)(cb < batch ? cb : batch);
+}
+
+// f(b0, nb) for the chunks [b0, b0 + nb) of cb batch elements (the last one shorter), stopping at the first error
+template <typename Fn>
+static int for_each_chunk(int batch, int cb, Fn&& f) {
+    for (int b0 = 0; b0 < batch; b0 += cb) {
+        const int rc = f(b0, b0 + cb <= batch ? cb : batch - b0);
+        if (rc) return rc;
+    }
     return PDU_OK;
 }
 
@@ -1577,14 +1619,10 @@ static size_t tz_plane_bytes(const pdu_nufft_plan* p) {
     return ((size_t)p->k0 * p->k1 + mid + (size_t)p->n0 * p->n1) * sizeof(float2);
 }
 
-// batch elements per chunk: the scratch stays under 512 MB (as the NUFFT's) and a chunk's planes fit gridDim.y;
-// pd_unet_b200/nufft.py::_ToepPlan.chunk repeats this arithmetic to size the workspace
+// batch elements per chunk: a chunk's planes also fit gridDim.y; pd_unet_b200/nufft.py::_ToepPlan.workspace_bytes
+// repeats this arithmetic to size the workspace
 static int tz_batch_chunk(const pdu_nufft_plan* p, int batch, int coils) {
-    long planes = (long)(((size_t)512 << 20) / tz_plane_bytes(p));
-    if (planes > 65535) planes = 65535;
-    long cb = planes / coils;
-    if (cb < 1) cb = 1;
-    return (int)(cb < batch ? cb : batch);
+    return batch_chunk(tz_plane_bytes(p), 65535, batch, coils);
 }
 
 constexpr int TZ_SEQ_ROWS = 4;
@@ -1675,10 +1713,7 @@ static int tz_apply_generic(pdu_nufft_plan* p, const float2* image, float2* out,
         T, U, p->d_w0, p->pf0, d, pitch0);
     PDU_LAUNCHED();
     if (sg) {
-        NufftDims dc = d;          // the cropped result is a dense [n0][n1] "grid"
-        dc.k0 = d.n0;
-        dc.k1 = d.n1;
-        rc = launch_smaps_grad(p, U, dc, coils, 1.f / ((float)p->k0 * (float)p->k1), *sg, st);
+        rc = launch_smaps_grad(p, U, cropped_dims(p), coils, 1.f / ((float)p->k0 * (float)p->k1), *sg, st);
         if (rc) return rc;
         note_kernel(OP_SMAPS_GRAD, "pfft_rows_fwd_kernel<%d> + pfft_cols_fwd_kernel<%d> + tz_mul_kernel + pfft_rows_adj_kernel<%d> + "
                     "pfft_cols_adj_kernel<%d> + smaps_grad_kernel per term (generic path, %d planes of %dx%d)",
@@ -1686,7 +1721,8 @@ static int tz_apply_generic(pdu_nufft_plan* p, const float2* image, float2* out,
         return PDU_OK;
     }
     const int out_planes = smaps ? batch : planes;
-    rc = launch_crop_apod(p, U, smaps, out, out_planes, coils, smaps_batch, 1.f / ((float)p->k0 * (float)p->k1), 0, st);
+    rc = launch_crop_apod(p, U, cropped_dims(p), smaps, out, out_planes, coils, smaps_batch, 1.f / ((float)p->k0 * (float)p->k1),
+                          0, st);
     if (rc) return rc;
     if (cg) {
         const long n = (long)p->n0 * p->n1;
@@ -1707,15 +1743,11 @@ static int tz_apply_generic(pdu_nufft_plan* p, const float2* image, float2* out,
 static int tz_apply_chunk(pdu_nufft_plan* p, const float2* image, float2* out, const float2* kern, int kernel_batch,
                           const float2* smaps, int batch, int coils, int smaps_batch, int conj, float2* ws, cudaStream_t st,
                           const TzCg* cg = nullptr, const SmapsGrad* sg = nullptr) {
-    if (tz_fast(p)) {
-        switch (p->k0) {
-            case 256: return tz_apply_fast<256>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st, sg);
-            case 512: return tz_apply_fast<512>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st, sg);
-            case 640: return tz_apply_fast<640>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st, sg);
-            case 1024: return tz_apply_fast<1024>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st, sg);
-            default: return tz_apply_fast<2048>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st, sg);
-        }
-    }
+    if (tz_fast(p))
+        return with_fast_fft_size(p->k0, [&](auto k) {
+            return tz_apply_fast<decltype(k)::value>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws,
+                                                     cg, st, sg);
+        });
     if (tz_cols_seq8(p))
         return tz_apply_generic<PF_SEQ_COLS>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st, sg);
     return tz_apply_generic<2>(p, image, out, kern, kernel_batch, smaps, batch, coils, smaps_batch, conj, ws, cg, st, sg);
@@ -1816,6 +1848,50 @@ static int tz_cg_chunk(pdu_nufft_plan* p, const float2* b, const float2* x0, flo
     return PDU_OK;
 }
 
+// n entries of `host` to a new device array *dst
+template <typename T>
+static cudaError_t upload(T** dst, const T* host, size_t n) {
+    cudaError_t e = cudaMalloc(dst, n * sizeof(T));
+    if (e == cudaSuccess) e = cudaMemcpy(*dst, host, n * sizeof(T), cudaMemcpyHostToDevice);
+    return e;
+}
+
+// the twiddle tables exp(-2 pi i j / K), j < K, of both axes (d_w0, d_w1), computed in float64
+static cudaError_t upload_twiddles(pdu_nufft_plan* p) {
+    cudaError_t e = cudaSuccess;
+    for (int ax = 0; ax < 2 && e == cudaSuccess; ++ax) {
+        const int K = ax == 0 ? p->k0 : p->k1;
+        std::vector<float2> w((size_t)K);
+        for (int i = 0; i < K; ++i) {
+            const double a = -2.0 * 3.14159265358979323846 * (double)i / (double)K;
+            w[i] = make_float2((float)cos(a), (float)sin(a));
+        }
+        e = upload(ax == 0 ? &p->d_w0 : &p->d_w1, w.data(), (size_t)K);
+    }
+    return e;
+}
+
+// a new plan of either kind for an n0 x n1 image on a k0 x k1 grid, on the current device; init(p) sets the rest and
+// uploads the kind's tables.  On an error the plan is destroyed and *plan stays null.
+template <typename Init>
+static int plan_create(pdu_nufft_plan_t** plan, int n0, int n1, int k0, int k1, const char* who, Init&& init) {
+    pdu_nufft_plan* p = new (std::nothrow) pdu_nufft_plan();
+    if (!p) {
+        set_error("%s: out of host memory", who);
+        return PDU_ENOMEM;
+    }
+    p->n0 = n0; p->n1 = n1; p->k0 = k0; p->k1 = k1;
+    cudaError_t e = cudaGetDevice(&p->device);
+    if (e == cudaSuccess) e = init(p);
+    if (e != cudaSuccess) {
+        set_error("%s: %s", who, cudaGetErrorString(e));
+        pdu_nufft_plan_destroy(p);
+        return PDU_ECUDA;
+    }
+    *plan = p;
+    return PDU_OK;
+}
+
 }  // namespace pdu
 
 using namespace pdu;
@@ -1833,48 +1909,21 @@ int pdu_nufft_plan_create(pdu_nufft_plan_t** plan, int n0, int n1, int k0, int k
     PDU_REQUIRE(table_oversamp >= 1 && (numpoints * table_oversamp) % 2 == 0,
                 "pdu_nufft_plan_create: numpoints * table_oversamp must be even");
     PDU_REQUIRE(table0 && table1 && scal0 && scal1, "pdu_nufft_plan_create: null table");
-    pdu_nufft_plan* p = new (std::nothrow) pdu_nufft_plan();
-    if (!p) {
-        set_error("pdu_nufft_plan_create: out of host memory");
-        return PDU_ENOMEM;
-    }
-    p->n0 = n0; p->n1 = n1; p->k0 = k0; p->k1 = k1; p->J = numpoints; p->L = table_oversamp;
-    p->shift0 = shift0; p->shift1 = shift1;
-    p->d_t0 = p->d_t1 = nullptr;
-    p->d_s0 = p->d_s1 = nullptr;
-    p->d_w0 = p->d_w1 = nullptr;
-    p->pfft_ok = pfft_factor(k0, &p->pf0) && pfft_factor(k1, &p->pf1) &&
-                 pf_smem_bytes(PF_SEQ_ROWS, k1) <= 200 * 1024 && pf_smem_bytes(PF_SEQ_COLS, k0) <= 200 * 1024;
-    const size_t tl = (size_t)numpoints * table_oversamp + 1;
-    cudaError_t e = cudaGetDevice(&p->device);
-    if (e == cudaSuccess) e = cudaMalloc(&p->d_t0, tl * sizeof(float2));
-    if (e == cudaSuccess) e = cudaMalloc(&p->d_t1, tl * sizeof(float2));
-    if (e == cudaSuccess) e = cudaMalloc(&p->d_s0, (size_t)n0 * sizeof(float));
-    if (e == cudaSuccess) e = cudaMalloc(&p->d_s1, (size_t)n1 * sizeof(float));
-    if (e == cudaSuccess) e = cudaMemcpy(p->d_t0, table0, tl * sizeof(float2), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(p->d_t1, table1, tl * sizeof(float2), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(p->d_s0, scal0, (size_t)n0 * sizeof(float), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(p->d_s1, scal1, (size_t)n1 * sizeof(float), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && (p->pfft_ok || (fast_fft_size(k0) && fast_fft_size(k1)))) {
-        for (int ax = 0; ax < 2 && e == cudaSuccess; ++ax) {
-            const int K = ax == 0 ? k0 : k1;
-            std::vector<float2> w((size_t)K);
-            for (int i = 0; i < K; ++i) {
-                const double a = -2.0 * 3.14159265358979323846 * (double)i / (double)K;
-                w[i] = make_float2((float)cos(a), (float)sin(a));
-            }
-            float2** dst = ax == 0 ? &p->d_w0 : &p->d_w1;
-            e = cudaMalloc(dst, (size_t)K * sizeof(float2));
-            if (e == cudaSuccess) e = cudaMemcpy(*dst, w.data(), (size_t)K * sizeof(float2), cudaMemcpyHostToDevice);
-        }
-    }
-    if (e != cudaSuccess) {
-        set_error("pdu_nufft_plan_create: %s", cudaGetErrorString(e));
-        pdu_nufft_plan_destroy(p);
-        return PDU_ECUDA;
-    }
-    *plan = p;
-    return PDU_OK;
+    return plan_create(plan, n0, n1, k0, k1, "pdu_nufft_plan_create", [&](pdu_nufft_plan* p) {
+        p->J = numpoints;
+        p->L = table_oversamp;
+        p->shift0 = shift0;
+        p->shift1 = shift1;
+        p->pfft_ok = pfft_factor(k0, &p->pf0) && pfft_factor(k1, &p->pf1) &&
+                     pf_smem_bytes(PF_SEQ_ROWS, k1) <= 200 * 1024 && pf_smem_bytes(PF_SEQ_COLS, k0) <= 200 * 1024;
+        const size_t tl = (size_t)numpoints * table_oversamp + 1;
+        cudaError_t e = upload(&p->d_t0, (const float2*)table0, tl);
+        if (e == cudaSuccess) e = upload(&p->d_t1, (const float2*)table1, tl);
+        if (e == cudaSuccess) e = upload(&p->d_s0, scal0, (size_t)n0);
+        if (e == cudaSuccess) e = upload(&p->d_s1, scal1, (size_t)n1);
+        if (e == cudaSuccess && (p->pfft_ok || (fast_fft_size(k0) && fast_fft_size(k1)))) e = upload_twiddles(p);
+        return e;
+    });
 }
 
 int pdu_nufft_plan_destroy(pdu_nufft_plan_t* p) {
@@ -1899,44 +1948,37 @@ size_t pdu_nufft_workspace_bytes(const pdu_nufft_plan_t* p, int planes) {
     return (size_t)planes * (grid + mid + crop) * sizeof(float2);
 }
 
-// A call is cut into batch chunks so that the scratch grids stay bounded (512 MB).  Measured on B200:
-// chunking down to L2-resident grids (56 MB) does NOT pay -- cuFFT runs at ~3 TB/s either way and the
-// gather / scatter lose parallelism -- so the budget only caps the workspace.
-static int batch_chunk(const pdu_nufft_plan* p, int batch, int coils) {
-    const size_t plane_bytes = (size_t)p->k0 * p->k1 * sizeof(float2);
-    const size_t budget = (size_t)512 << 20;
-    long planes = (long)(budget / plane_bytes);
-    long cb = planes / coils;
-    if (cb < 1) cb = 1;
-    return (int)(cb < batch ? cb : batch);
+// batch elements per chunk of the generic path, by its oversampled grids (no plane cap)
+static int nufft_batch_chunk(const pdu_nufft_plan* p, int batch, int coils) {
+    return batch_chunk((size_t)p->k0 * p->k1 * sizeof(float2), LONG_MAX, batch, coils);
+}
+
+// variant 2 = the register-resident pruned FFT (pfft_fast.cuh), 1 = the generic pruned FFT (pfft.cuh), 0 = pad + cuFFT;
+// opt: the A/B option of the direction.  Measured on B200 (64 planes of 640^2): the generic pruned passes move 2.5x fewer
+// bytes but are still ~1.7x slower than cuFFT's register-resident radix kernels (row+column 407 us vs 238 us).
+static int fft_variant(const pdu_nufft_plan* p, int opt) {
+    int variant = option(opt);
+    // default: the register-resident pruned FFT on the BASELINE grids, the generic pruned FFT on every other grid
+    // that factors into 2, 3, 5 (slower than cuFFT, but the library's own); cuFFT only for other prime factors
+    if (variant < 0) variant = ff_supported(p) ? 2 : (p->pfft_ok ? 1 : 0);
+    if ((variant == 2 && !ff_supported(p)) || (variant == 1 && !p->pfft_ok)) variant = 0;
+    return variant;
 }
 
 static int nufft_fwd_chunk(pdu_nufft_plan_t* p, const float2* image, float2* kdata, const float* omega, const float2* smaps,
                            int batch, int coils, int smaps_batch, long m, float scale, float2* grid, cudaStream_t st) {
     const int planes = batch * coils;
     const long total = (long)planes * p->k0 * p->k1;
-    // variant 1 = own pruned shared-memory FFT (pfft.cuh), variant 0 = pad + cuFFT.  Measured on B200 (64 planes of
-    // 640^2): the pruned passes move 2.5x fewer bytes but are still ~1.7x slower than cuFFT's register-resident
-    // radix kernels (row+column 407 us vs 238 us), so cuFFT stays the default until they are.
-    int variant = option(OPT_NUFFT_FWD);
-    // default: the register-resident pruned FFT on the BASELINE grids, the generic pruned FFT on every other grid
-    // that factors into 2, 3, 5 (slower than cuFFT, but the library's own); cuFFT only for other prime factors
-    if (variant < 0) variant = ff_supported(p) ? 2 : (p->pfft_ok ? 1 : 0);
+    const int variant = fft_variant(p, OPT_NUFFT_FWD);
+    float2* T = grid + total;
     int rc;
-    if (variant == 2 && !ff_supported(p)) variant = 0;
     if (variant == 2) {
-        float2* T = grid + total;
-        switch (p->k0) {
-            case 256: rc = ff_forward<256>(p, image, smaps, T, grid, planes, coils, smaps_batch, st); break;
-            case 512: rc = ff_forward<512>(p, image, smaps, T, grid, planes, coils, smaps_batch, st); break;
-            case 640: rc = ff_forward<640>(p, image, smaps, T, grid, planes, coils, smaps_batch, st); break;
-            case 1024: rc = ff_forward<1024>(p, image, smaps, T, grid, planes, coils, smaps_batch, st); break;
-            default: rc = ff_forward<2048>(p, image, smaps, T, grid, planes, coils, smaps_batch, st); break;
-        }
+        rc = with_fast_fft_size(p->k0, [&](auto k) {
+            return ff_forward<decltype(k)::value>(p, image, smaps, T, grid, planes, coils, smaps_batch, st);
+        });
         if (rc) return rc;
-    } else if (variant == 1 && p->pfft_ok) {
+    } else if (variant == 1) {
         // pruned FFT: apodise + pad + transform the n0 non-zero rows, then every column
-        float2* T = grid + total;
         const NufftDims d = dims_of(p);
         const int pitch1 = pfft_pitch(p->k1), pitch0 = pfft_pitch(p->k0);
         rc = pf_set_smem(pfft_rows_fwd_kernel<PF_SEQ_ROWS>, pf_smem_bytes(PF_SEQ_ROWS, p->k1));
@@ -1959,8 +2001,8 @@ static int nufft_fwd_chunk(pdu_nufft_plan_t* p, const float2* image, float2* kda
     }
     note_kernel(OP_NUFFT_FWD, "%s + interp_fwd_kernel<%d> (%d planes of %dx%d, M=%ld)",
                 variant == 2 ? "ff_rows_fwd_kernel + ff_cols_fwd_kernel (register-resident pruned FFT)"
-                             : (variant == 1 && p->pfft_ok ? "pfft_rows_fwd_kernel + pfft_cols_fwd_kernel (generic pruned FFT)"
-                                                           : "apod_pad_kernel + cuFFT C2C"),
+                             : (variant == 1 ? "pfft_rows_fwd_kernel + pfft_cols_fwd_kernel (generic pruned FFT)"
+                                             : "apod_pad_kernel + cuFFT C2C"),
                 p->J == 6 ? 6 : 0, planes, p->k0, p->k1, m);
     return launch_interp_fwd(p, grid, kdata, omega, planes, m, scale, st);
 }
@@ -1970,62 +2012,43 @@ static int nufft_adj_chunk(pdu_nufft_plan_t* p, const float2* kdata, float2* ima
                            cudaStream_t st, const SmapsGrad* sg = nullptr) {
     const int planes = batch * coils;
     int rc;
-    int variant = option(OPT_NUFFT_ADJ);
-    if (variant < 0) variant = ff_supported(p) ? 2 : (p->pfft_ok ? 1 : 0);      // see nufft_fwd_chunk
-    if (variant == 2 && !ff_supported(p)) variant = 0;
+    const int variant = fft_variant(p, OPT_NUFFT_ADJ);
     // the gridded samples stay compact (non-empty cells only) between the sorted gather and the register FFT's row pass
     // (only for sparse trajectories, at most 8 interpolation entries per cell on average: 48 radial spokes on 640^2 have
     //  2.7 and leave 61 % of the cells empty; a dense trajectory fills the grid and would only pay for the indirection)
     bool compact = csr && variant == 2 && (double)m * p->J * p->J <= 8.0 * (double)p->k0 * p->k1;
+    float2* T = grid + (long)planes * p->k0 * p->k1;
+    float2* U = T + (long)planes * std::max((long)p->n0 * p->k1, (long)p->k0 * p->n1);
     if (csr) {
-        // the FFT's intermediate buffer and the cropped result behind it are free until the transform starts: they hold the
-        // plane-interleaved kdata
-        float2* mid = grid + (long)planes * p->k0 * p->k1;
+        // the FFT's intermediate buffer T and the cropped result U behind it are free until the transform starts: they
+        // hold the plane-interleaved kdata
         const long mid_elems = (long)planes * (std::max((long)p->n0 * p->k1, (long)p->k0 * p->n1) + (long)p->n0 * p->n1);
         const bool fits = m * (long)((planes + 3) & ~3) <= mid_elems;
-        rc = launch_interp_adj_csr(p, kdata, grid, csr, planes, m, st, fits ? mid : nullptr, &compact);   // writes every cell: no memset
+        rc = launch_interp_adj_csr(p, kdata, grid, csr, planes, m, st, fits ? T : nullptr, &compact);   // writes every cell: no memset
     } else {
         PDU_CUDA(cudaMemsetAsync(grid, 0, (size_t)planes * p->k0 * p->k1 * sizeof(float2), st));
         rc = launch_interp_adj(p, kdata, grid, omega, planes, m, st);
     }
     if (rc) return rc;
-    const int out_planes = smaps ? batch : planes;
-    const long total = (long)out_planes * p->n0 * p->n1;
     note_kernel(sg ? OP_SMAPS_GRAD : OP_NUFFT_ADJ, "%s + %s + %s (%d planes of %dx%d, M=%ld)",
                 csr ? (compact ? "transpose_kdata_kernel + interp_adj_csrT_kernel (sorted gather: 4 lanes per cell x 16 planes, long rows by warps, non-empty cells only)"
                                : "transpose_kdata_kernel + interp_adj_csrT_kernel (sorted gather: 4 lanes per cell x 16 planes, long rows by warps)")
                     : "interp_adj_kernel (float2 atomics)",
                 variant == 2 ? (compact ? "ff_rows_adj_compact_kernel + ff_cols_adj_kernel (register-resident pruned FFT)"
                                         : "ff_rows_adj_kernel + ff_cols_adj_kernel (register-resident pruned FFT)")
-                             : (variant == 1 && p->pfft_ok ? "pfft_rows_adj_kernel + pfft_cols_adj_kernel (generic pruned FFT)"
-                                                           : "cuFFT C2C"),
+                             : (variant == 1 ? "pfft_rows_adj_kernel + pfft_cols_adj_kernel (generic pruned FFT)"
+                                             : "cuFFT C2C"),
                 sg ? "smaps_grad_kernel" : "crop_apod_kernel", planes, p->k0, p->k1, m);
+    // the planes the adjoint ends on, with their geometry: the pruned FFTs' cropped n0 x n1 planes U, or cuFFT's full grid
+    const float2* Ue = U;
+    NufftDims de = cropped_dims(p);
     if (variant == 2) {
-        float2* T = grid + (long)planes * p->k0 * p->k1;
-        float2* U = T + (long)planes * std::max((long)p->n0 * p->k1, (long)p->k0 * p->n1);
         const CsrView cv = compact ? csr_layout(p, m, const_cast<void*>(csr), false) : CsrView{};
         const int* nzi = compact ? cv.nz_idx : nullptr;
-        switch (p->k0) {
-            case 256: rc = ff_adjoint<256>(p, grid, T, U, planes, st, nzi); break;
-            case 512: rc = ff_adjoint<512>(p, grid, T, U, planes, st, nzi); break;
-            case 640: rc = ff_adjoint<640>(p, grid, T, U, planes, st, nzi); break;
-            case 1024: rc = ff_adjoint<1024>(p, grid, T, U, planes, st, nzi); break;
-            default: rc = ff_adjoint<2048>(p, grid, T, U, planes, st, nzi); break;
-        }
+        rc = with_fast_fft_size(p->k0, [&](auto k) { return ff_adjoint<decltype(k)::value>(p, grid, T, U, planes, st, nzi); });
         if (rc) return rc;
-        NufftDims dc = dims_of(p);          // the cropped result is a dense [n0][n1] "grid"
-        dc.k0 = dc.n0;
-        dc.k1 = dc.n1;
-        if (sg) return launch_smaps_grad(p, U, dc, coils, scale, *sg, st);
-        crop_apod_kernel<<<stream_grid(total), 256, 0, st>>>(U, smaps, image, p->d_s0, p->d_s1, dc, coils, smaps_batch, scale,
-                                                             total);
-        PDU_LAUNCHED();
-        return PDU_OK;
-    }
-    if (variant == 1 && p->pfft_ok) {
+    } else if (variant == 1) {
         // pruned inverse FFT: every row but only the n1 kept outputs, then the n1 kept columns and n0 kept outputs
-        float2* T = grid + (long)planes * p->k0 * p->k1;
-        float2* U = T + (long)planes * std::max((long)p->n0 * p->k1, (long)p->k0 * p->n1);
         const NufftDims d = dims_of(p);
         rc = pf_set_smem(pfft_rows_adj_kernel<PF_SEQ_ROWS>, pf_smem_bytes(PF_SEQ_ROWS, p->k1));
         if (rc) return rc;
@@ -2038,22 +2061,14 @@ static int nufft_adj_chunk(pdu_nufft_plan_t* p, const float2* kdata, float2* ima
         pfft_cols_adj_kernel<PF_SEQ_COLS><<<dim3((unsigned)cdiv(p->n1, PF_SEQ_COLS), (unsigned)planes), 256,
                                             pf_smem_bytes(PF_SEQ_COLS, p->k0), st>>>(T, U, p->d_w0, p->pf0, d, pfft_pitch(p->k0));
         PDU_LAUNCHED();
-        NufftDims dc = d;          // the cropped result is a dense [n0][n1] "grid"
-        dc.k0 = d.n0;
-        dc.k1 = d.n1;
-        if (sg) return launch_smaps_grad(p, U, dc, coils, scale, *sg, st);
-        crop_apod_kernel<<<stream_grid(total), 256, 0, st>>>(U, smaps, image, p->d_s0, p->d_s1, dc, coils, smaps_batch, scale,
-                                                             total);
-        PDU_LAUNCHED();
-        return PDU_OK;
+    } else {
+        rc = run_fft(p, grid, planes, CUFFT_INVERSE, st);
+        if (rc) return rc;
+        Ue = grid;
+        de = dims_of(p);
     }
-    rc = run_fft(p, grid, planes, CUFFT_INVERSE, st);
-    if (rc) return rc;
-    if (sg) return launch_smaps_grad(p, grid, dims_of(p), coils, scale, *sg, st);
-    crop_apod_kernel<<<stream_grid(total), 256, 0, st>>>(grid, smaps, image, p->d_s0, p->d_s1, dims_of(p), coils, smaps_batch,
-                                                         scale, total);
-    PDU_LAUNCHED();
-    return PDU_OK;
+    if (sg) return launch_smaps_grad(p, Ue, de, coils, scale, *sg, st);
+    return launch_crop_apod(p, Ue, de, smaps, image, smaps ? batch : planes, coils, smaps_batch, scale, 0, st);
 }
 
 int pdu_nufft_fwd_c64(pdu_nufft_plan_t* p, const float* image, float* kdata, const float* omega, const float* smaps,
@@ -2062,22 +2077,17 @@ int pdu_nufft_fwd_c64(pdu_nufft_plan_t* p, const float* image, float* kdata, con
     int rc = check_call(p, image, kdata, omega, batch, coils, smaps_batch, smaps, m, "pdu_nufft_fwd_c64");
     if (rc) return rc;
     PDU_CHECK_DEVICE("pdu_nufft_fwd_c64");
-    const int cb = batch_chunk(p, batch, coils);
-    const size_t need = pdu_nufft_workspace_bytes(p, cb * coils);
-    if (!workspace || workspace_bytes < need) {
-        set_error("pdu_nufft_fwd_c64: workspace of %zu bytes required, got %zu", need, workspace ? workspace_bytes : (size_t)0);
-        return PDU_ENOMEM;
-    }
+    const int cb = nufft_batch_chunk(p, batch, coils);
+    rc = check_workspace("pdu_nufft_fwd_c64", workspace, workspace_bytes, pdu_nufft_workspace_bytes(p, cb * coils), false,
+                         PDU_ENOMEM);
+    if (rc) return rc;
     const long plane = (long)p->n0 * p->n1;
     const long img_b = (smaps ? 1 : coils) * plane, smap_b = smaps_batch == 1 ? 0 : coils * plane;
-    for (int b0 = 0; b0 < batch; b0 += cb) {
-        const int nb = b0 + cb <= batch ? cb : batch - b0;
-        rc = nufft_fwd_chunk(p, (const float2*)image + b0 * img_b, (float2*)kdata + (long)b0 * coils * m, omega,
-                             smaps ? (const float2*)smaps + b0 * smap_b : nullptr, nb, coils, smaps_batch == 1 ? 1 : nb, m, scale,
-                             (float2*)workspace, (cudaStream_t)stream);
-        if (rc) return rc;
-    }
-    return PDU_OK;
+    return for_each_chunk(batch, cb, [&](int b0, int nb) {
+        return nufft_fwd_chunk(p, (const float2*)image + b0 * img_b, (float2*)kdata + (long)b0 * coils * m, omega,
+                               smaps ? (const float2*)smaps + b0 * smap_b : nullptr, nb, coils, smaps_batch == 1 ? 1 : nb, m,
+                               scale, (float2*)workspace, (cudaStream_t)stream);
+    });
 }
 
 size_t pdu_nufft_csr_bytes(const pdu_nufft_plan_t* p, long m) {
@@ -2124,22 +2134,17 @@ int pdu_nufft_adj_csr_c64(pdu_nufft_plan_t* p, const float* kdata, float* image,
     int rc = check_call(p, kdata, image, omega, batch, coils, smaps_batch, smaps, m, "pdu_nufft_adj_c64");
     if (rc) return rc;
     PDU_CHECK_DEVICE("pdu_nufft_adj_c64");
-    const int cb = batch_chunk(p, batch, coils);
-    const size_t need = pdu_nufft_workspace_bytes(p, cb * coils);
-    if (!workspace || workspace_bytes < need) {
-        set_error("pdu_nufft_adj_c64: workspace of %zu bytes required, got %zu", need, workspace ? workspace_bytes : (size_t)0);
-        return PDU_ENOMEM;
-    }
+    const int cb = nufft_batch_chunk(p, batch, coils);
+    rc = check_workspace("pdu_nufft_adj_c64", workspace, workspace_bytes, pdu_nufft_workspace_bytes(p, cb * coils), false,
+                         PDU_ENOMEM);
+    if (rc) return rc;
     const long plane = (long)p->n0 * p->n1;
     const long img_b = (smaps ? 1 : coils) * plane, smap_b = smaps_batch == 1 ? 0 : coils * plane;
-    for (int b0 = 0; b0 < batch; b0 += cb) {
-        const int nb = b0 + cb <= batch ? cb : batch - b0;
-        rc = nufft_adj_chunk(p, (const float2*)kdata + (long)b0 * coils * m, (float2*)image + b0 * img_b, omega,
-                             smaps ? (const float2*)smaps + b0 * smap_b : nullptr, nb, coils, smaps_batch == 1 ? 1 : nb, m, scale,
-                             (float2*)workspace, csr, (cudaStream_t)stream);
-        if (rc) return rc;
-    }
-    return PDU_OK;
+    return for_each_chunk(batch, cb, [&](int b0, int nb) {
+        return nufft_adj_chunk(p, (const float2*)kdata + (long)b0 * coils * m, (float2*)image + b0 * img_b, omega,
+                               smaps ? (const float2*)smaps + b0 * smap_b : nullptr, nb, coils, smaps_batch == 1 ? 1 : nb, m,
+                               scale, (float2*)workspace, csr, (cudaStream_t)stream);
+    });
 }
 
 int pdu_nufft_fwd_binned_c64(pdu_nufft_plan_t* p, const float* image, float* kdata, const float* smaps, int batch, int coils,
@@ -2152,12 +2157,9 @@ int pdu_nufft_fwd_binned_c64(pdu_nufft_plan_t* p, const float* image, float* kda
         set_error("pdu_nufft_fwd_binned_c64: grid %d x %d (J = %d) has no fused path; use pdu_nufft_fwd_c64", p->k0, p->k1, p->J);
         return PDU_EUNSUPPORTED;
     }
-    const size_t need = fused_workspace_bytes(p, batch * coils, m);
-    if (!workspace || workspace_bytes < need || ((uintptr_t)workspace & 255)) {
-        set_error("pdu_nufft_fwd_binned_c64: workspace of %zu bytes (256-byte aligned) required, got %zu", need,
-                  workspace ? workspace_bytes : (size_t)0);
-        return PDU_ENOMEM;
-    }
+    rc = check_workspace("pdu_nufft_fwd_binned_c64", workspace, workspace_bytes, fused_workspace_bytes(p, batch * coils, m), true,
+                         PDU_ENOMEM);
+    if (rc) return rc;
     return fused_forward(p, image, kdata, smaps, batch, coils, smaps_batch, m, scale, bins, flags, workspace, (cudaStream_t)stream);
 }
 
@@ -2171,12 +2173,9 @@ int pdu_nufft_adj_binned_c64(pdu_nufft_plan_t* p, const float* kdata, float* ima
         set_error("pdu_nufft_adj_binned_c64: grid %d x %d (J = %d) has no fused path; use pdu_nufft_adj_c64", p->k0, p->k1, p->J);
         return PDU_EUNSUPPORTED;
     }
-    const size_t need = fused_workspace_bytes(p, batch * coils, m);
-    if (!workspace || workspace_bytes < need || ((uintptr_t)workspace & 255)) {
-        set_error("pdu_nufft_adj_binned_c64: workspace of %zu bytes (256-byte aligned) required, got %zu", need,
-                  workspace ? workspace_bytes : (size_t)0);
-        return PDU_ENOMEM;
-    }
+    rc = check_workspace("pdu_nufft_adj_binned_c64", workspace, workspace_bytes, fused_workspace_bytes(p, batch * coils, m), true,
+                         PDU_ENOMEM);
+    if (rc) return rc;
     return fused_adjoint(p, kdata, image, smaps, kweight, batch, coils, smaps_batch, m, scale, bins, flags, workspace,
                          (cudaStream_t)stream);
 }
@@ -2197,35 +2196,25 @@ int pdu_nufft_adj_smaps_grad_c64(pdu_nufft_plan_t* p, const float* kdata, const 
             set_error("%s: grid %d x %d (J = %d) has no fused path; pass bins = NULL", who, p->k0, p->k1, p->J);
             return PDU_EUNSUPPORTED;
         }
-        const size_t need = fused_workspace_bytes(p, batch * coils, m);
-        if (!workspace || workspace_bytes < need || ((uintptr_t)workspace & 255)) {
-            set_error("%s: workspace of %zu bytes (256-byte aligned) required, got %zu", who, need,
-                      workspace ? workspace_bytes : (size_t)0);
-            return PDU_ENOMEM;
-        }
+        rc = check_workspace(who, workspace, workspace_bytes, fused_workspace_bytes(p, batch * coils, m), true, PDU_ENOMEM);
+        if (rc) return rc;
         const SmapsGrad sg{(float2*)gs, q, batch, per_batch, q_split, accumulate ? 1 : 0, 1.f};
         return fused_adjoint(p, kdata, nullptr, nullptr, kweight, batch, coils, 1, m, scale, bins, flags, workspace,
                              (cudaStream_t)stream, &sg);
     }
     // the plain-omega / CSR paths take complex64 kdata without weights, as pdu_nufft_adj_csr_c64 does
     PDU_REQUIRE(!kweight && !(flags & PDU_NUFFT_KDATA_SPLIT), "%s: kweight and split kdata need the row-binned path (bins)", who);
-    const int cb = batch_chunk(p, batch, coils);
-    const size_t need = pdu_nufft_workspace_bytes(p, cb * coils);
-    if (!workspace || workspace_bytes < need) {
-        set_error("%s: workspace of %zu bytes required, got %zu", who, need, workspace ? workspace_bytes : (size_t)0);
-        return PDU_ENOMEM;
-    }
+    const int cb = nufft_batch_chunk(p, batch, coils);
+    rc = check_workspace(who, workspace, workspace_bytes, pdu_nufft_workspace_bytes(p, cb * coils), false, PDU_ENOMEM);
+    if (rc) return rc;
     const long plane = (long)p->n0 * p->n1;
-    for (int b0 = 0; b0 < batch; b0 += cb) {
-        const int nb = b0 + cb <= batch ? cb : batch - b0;
+    return for_each_chunk(batch, cb, [&](int b0, int nb) {
         // a shared map's sum continues from chunk to chunk
         const SmapsGrad sg{(float2*)gs + (per_batch ? (long)b0 * coils * plane : 0), q + (long)b0 * 2 * plane, nb, per_batch,
                            q_split, (accumulate || (!per_batch && b0 > 0)) ? 1 : 0, 1.f};
-        rc = nufft_adj_chunk(p, (const float2*)kdata + (long)b0 * coils * m, nullptr, omega, nullptr, nb, coils, 1, m, scale,
-                             (float2*)workspace, csr, (cudaStream_t)stream, &sg);
-        if (rc) return rc;
-    }
-    return PDU_OK;
+        return nufft_adj_chunk(p, (const float2*)kdata + (long)b0 * coils * m, nullptr, omega, nullptr, nb, coils, 1, m, scale,
+                               (float2*)workspace, csr, (cudaStream_t)stream, &sg);
+    });
 }
 
 int pdu_complex_from_split_f32(const float* split, float* out, const float* weight, long planes, long n, pdu_stream_t stream) {
@@ -2270,43 +2259,17 @@ int pdu_toep_plan_create(pdu_nufft_plan_t** plan, int n0, int n1) {
                   "and fit the shared-memory FFT)", n0, n1, k0, k1);
         return PDU_EUNSUPPORTED;
     }
-    pdu_nufft_plan* p = new (std::nothrow) pdu_nufft_plan();
-    if (!p) {
-        set_error("pdu_toep_plan_create: out of host memory");
-        return PDU_ENOMEM;
-    }
-    p->n0 = n0; p->n1 = n1; p->k0 = k0; p->k1 = k1; p->J = 0; p->L = 0;
-    p->shift0 = p->shift1 = 0;
-    p->d_t0 = p->d_t1 = nullptr;
-    p->d_s0 = p->d_s1 = nullptr;
-    p->d_w0 = p->d_w1 = nullptr;
-    p->pfft_ok = true;
-    p->pf0 = pf0;
-    p->pf1 = pf1;
-    p->toep = true;
-    cudaError_t e = cudaGetDevice(&p->device);
-    for (int ax = 0; ax < 2 && e == cudaSuccess; ++ax) {
-        const int K = ax == 0 ? k0 : k1;
-        std::vector<float> ones((size_t)K, 1.f);        // unit apodisation (every entry a row / column pass may read)
-        std::vector<float2> w((size_t)K);
-        for (int i = 0; i < K; ++i) {
-            const double a = -2.0 * 3.14159265358979323846 * (double)i / (double)K;
-            w[i] = make_float2((float)cos(a), (float)sin(a));
-        }
-        float** s = ax == 0 ? &p->d_s0 : &p->d_s1;
-        float2** tw = ax == 0 ? &p->d_w0 : &p->d_w1;
-        e = cudaMalloc(s, (size_t)K * sizeof(float));
-        if (e == cudaSuccess) e = cudaMemcpy(*s, ones.data(), (size_t)K * sizeof(float), cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = cudaMalloc(tw, (size_t)K * sizeof(float2));
-        if (e == cudaSuccess) e = cudaMemcpy(*tw, w.data(), (size_t)K * sizeof(float2), cudaMemcpyHostToDevice);
-    }
-    if (e != cudaSuccess) {
-        set_error("pdu_toep_plan_create: %s", cudaGetErrorString(e));
-        pdu_nufft_plan_destroy(p);
-        return PDU_ECUDA;
-    }
-    *plan = p;
-    return PDU_OK;
+    return plan_create(plan, n0, n1, k0, k1, "pdu_toep_plan_create", [&](pdu_nufft_plan* p) {
+        p->pfft_ok = true;
+        p->pf0 = pf0;
+        p->pf1 = pf1;
+        p->toep = true;
+        const std::vector<float> ones((size_t)std::max(k0, k1), 1.f);   // unit apodisation (every entry a row / column pass may read)
+        cudaError_t e = upload(&p->d_s0, ones.data(), (size_t)k0);
+        if (e == cudaSuccess) e = upload(&p->d_s1, ones.data(), (size_t)k1);
+        if (e == cudaSuccess) e = upload_twiddles(p);
+        return e;
+    });
 }
 
 size_t pdu_toep_workspace_bytes(const pdu_nufft_plan_t* p, int planes) {
@@ -2316,19 +2279,13 @@ size_t pdu_toep_workspace_bytes(const pdu_nufft_plan_t* p, int planes) {
 
 int pdu_toep_kernel_c64(pdu_nufft_plan_t* p, const float* q1, const float* q2, float* kernel, int kernels, float scale,
                         void* ws, size_t ws_bytes, pdu_stream_t stream) {
-    PDU_REQUIRE(p != nullptr, "pdu_toep_kernel_c64: plan is null");
-    PDU_REQUIRE(p->toep, "pdu_toep_kernel_c64: not a Toeplitz plan (use pdu_toep_plan_create)");
-    PDU_REQUIRE(q1 && q2 && kernel, "pdu_toep_kernel_c64: null pointer");
-    PDU_REQUIRE(kernels > 0 && kernels <= 65535, "pdu_toep_kernel_c64: kernels must be in 1..65535");
-    const size_t need = (size_t)kernels * p->k0 * p->k1 * sizeof(float2);
-    if (!ws || ws_bytes < need) {
-        set_error("pdu_toep_kernel_c64: workspace of %zu bytes required, got %zu", need, ws ? ws_bytes : (size_t)0);
-        return PDU_ENOMEM;
-    }
-    int dev = -1;
-    PDU_CUDA(cudaGetDevice(&dev));
-    PDU_REQUIRE(dev == p->device, "pdu_toep_kernel_c64: plan was created on device %d, current device is %d", p->device, dev);
-    PDU_CHECK_DEVICE("pdu_toep_kernel_c64");
+    const char* who = "pdu_toep_kernel_c64";
+    int rc = check_toep_call(p, q1 && q2 && kernel, 1, 1, 1, nullptr, 1, who);     // no batch; the kernel count is checked next
+    if (rc) return rc;
+    PDU_REQUIRE(kernels > 0 && kernels <= 65535, "%s: kernels must be in 1..65535", who);
+    rc = check_workspace(who, ws, ws_bytes, (size_t)kernels * p->k0 * p->k1 * sizeof(float2), false, PDU_ENOMEM);
+    if (rc) return rc;
+    PDU_CHECK_DEVICE(who);
     cudaStream_t st = (cudaStream_t)stream;
     const long total = (long)kernels * p->k0 * p->k1;
     tz_assemble_kernel<<<stream_grid(total), 256, 0, st>>>((const float2*)q1, (const float2*)q2, (float2*)kernel, p->n0, p->n1,
@@ -2341,73 +2298,51 @@ int pdu_toep_kernel_c64(pdu_nufft_plan_t* p, const float* q1, const float* q2, f
 int pdu_toep_apply_c64(pdu_nufft_plan_t* p, const float* image, float* out, const float* kernel, int kernel_batch,
                        const float* smaps, int batch, int coils, int smaps_batch, int conj_kernel, void* ws, size_t ws_bytes,
                        pdu_stream_t stream) {
-    PDU_REQUIRE(p != nullptr, "pdu_toep_apply_c64: plan is null");
-    PDU_REQUIRE(p->toep, "pdu_toep_apply_c64: not a Toeplitz plan (use pdu_toep_plan_create)");
-    PDU_REQUIRE(image && out && kernel, "pdu_toep_apply_c64: null pointer");
-    PDU_REQUIRE(batch > 0 && coils > 0 && coils <= 65535, "pdu_toep_apply_c64: batch must be > 0 and coils in 1..65535");
-    PDU_REQUIRE(kernel_batch == 1 || kernel_batch == batch, "pdu_toep_apply_c64: kernel batch must be 1 or batch");
-    if (smaps) PDU_REQUIRE(smaps_batch == 1 || smaps_batch == batch, "pdu_toep_apply_c64: smaps batch must be 1 or batch");
+    const char* who = "pdu_toep_apply_c64";
+    int rc = check_toep_call(p, image && out && kernel, batch, coils, kernel_batch, smaps, smaps_batch, who);
+    if (rc) return rc;
     const int cb = tz_batch_chunk(p, batch, coils);
-    const size_t need = pdu_toep_workspace_bytes(p, cb * coils);
-    if (!ws || ws_bytes < need) {
-        set_error("pdu_toep_apply_c64: workspace of %zu bytes required, got %zu", need, ws ? ws_bytes : (size_t)0);
-        return PDU_ENOMEM;
-    }
-    int dev = -1;
-    PDU_CUDA(cudaGetDevice(&dev));
-    PDU_REQUIRE(dev == p->device, "pdu_toep_apply_c64: plan was created on device %d, current device is %d", p->device, dev);
-    PDU_CHECK_DEVICE("pdu_toep_apply_c64");
+    rc = check_workspace(who, ws, ws_bytes, pdu_toep_workspace_bytes(p, cb * coils), false, PDU_ENOMEM);
+    if (rc) return rc;
+    PDU_CHECK_DEVICE(who);
     const long plane = (long)p->n0 * p->n1, cells = (long)p->k0 * p->k1;
     const long img_b = (smaps ? 1 : coils) * plane, out_b = img_b, smap_b = smaps_batch == 1 ? 0 : coils * plane;
-    for (int b0 = 0; b0 < batch; b0 += cb) {
-        const int nb = b0 + cb <= batch ? cb : batch - b0;
-        int rc = tz_apply_chunk(p, (const float2*)image + b0 * img_b, (float2*)out + b0 * out_b,
-                                (const float2*)kernel + (kernel_batch == 1 ? 0 : b0 * cells), kernel_batch == 1 ? 1 : nb,
-                                smaps ? (const float2*)smaps + b0 * smap_b : nullptr, nb, coils, smaps_batch == 1 ? 1 : nb,
-                                conj_kernel ? 1 : 0, (float2*)ws, (cudaStream_t)stream);
-        if (rc) return rc;
-    }
-    return PDU_OK;
+    return for_each_chunk(batch, cb, [&](int b0, int nb) {
+        return tz_apply_chunk(p, (const float2*)image + b0 * img_b, (float2*)out + b0 * out_b,
+                              (const float2*)kernel + (kernel_batch == 1 ? 0 : b0 * cells), kernel_batch == 1 ? 1 : nb,
+                              smaps ? (const float2*)smaps + b0 * smap_b : nullptr, nb, coils, smaps_batch == 1 ? 1 : nb,
+                              conj_kernel ? 1 : 0, (float2*)ws, (cudaStream_t)stream);
+    });
 }
 
 int pdu_toep_smaps_grad_c64(pdu_nufft_plan_t* p, const float* x, const float* g, float* gs, const float* kernel,
                             int kernel_batch, const float* smaps, int batch, int coils, int smaps_batch, int conj_kernel,
                             float out_scale, int accumulate, void* ws, size_t ws_bytes, pdu_stream_t stream) {
-    PDU_REQUIRE(p != nullptr, "pdu_toep_smaps_grad_c64: plan is null");
-    PDU_REQUIRE(p->toep, "pdu_toep_smaps_grad_c64: not a Toeplitz plan (use pdu_toep_plan_create)");
-    PDU_REQUIRE(x && g && gs && kernel && smaps, "pdu_toep_smaps_grad_c64: null pointer");
-    PDU_REQUIRE(batch > 0 && coils > 0 && coils <= 65535, "pdu_toep_smaps_grad_c64: batch must be > 0 and coils in 1..65535");
-    PDU_REQUIRE(kernel_batch == 1 || kernel_batch == batch, "pdu_toep_smaps_grad_c64: kernel batch must be 1 or batch");
-    PDU_REQUIRE(smaps_batch == 1 || smaps_batch == batch, "pdu_toep_smaps_grad_c64: smaps batch must be 1 or batch");
+    const char* who = "pdu_toep_smaps_grad_c64";
+    int rc = check_toep_call(p, x && g && gs && kernel && smaps, batch, coils, kernel_batch, smaps, smaps_batch, who);
+    if (rc) return rc;
     const int cb = tz_batch_chunk(p, batch, coils);
-    const size_t need = pdu_toep_workspace_bytes(p, cb * coils);
-    if (!ws || ws_bytes < need) {
-        set_error("pdu_toep_smaps_grad_c64: workspace of %zu bytes required, got %zu", need, ws ? ws_bytes : (size_t)0);
-        return PDU_ENOMEM;
-    }
-    int dev = -1;
-    PDU_CUDA(cudaGetDevice(&dev));
-    PDU_REQUIRE(dev == p->device, "pdu_toep_smaps_grad_c64: plan was created on device %d, current device is %d", p->device, dev);
-    PDU_CHECK_DEVICE("pdu_toep_smaps_grad_c64");
+    rc = check_workspace(who, ws, ws_bytes, pdu_toep_workspace_bytes(p, cb * coils), false, PDU_ENOMEM);
+    if (rc) return rc;
+    PDU_CHECK_DEVICE(who);
     const long plane = (long)p->n0 * p->n1, cells = (long)p->k0 * p->k1;
     const int per_batch = smaps_batch == 1 ? 0 : 1;
     const long smap_b = per_batch ? coils * plane : 0;
-    for (int b0 = 0; b0 < batch; b0 += cb) {
-        const int nb = b0 + cb <= batch ? cb : batch - b0;
+    return for_each_chunk(batch, cb, [&](int b0, int nb) -> int {
         // term 0: T(S_c x_b) conj(g_b); term 1: T^H(S_c g_b) conj(x_b), added on top
         for (int term = 0; term < 2; ++term) {
             const float* image = term ? g : x;
             const float* q = term ? x : g;
             const int acc = (accumulate || term == 1 || (!per_batch && b0 > 0)) ? 1 : 0;
             const SmapsGrad sg{(float2*)gs + b0 * smap_b, q + 2 * b0 * plane, nb, per_batch, 0, acc, out_scale};
-            int rc = tz_apply_chunk(p, (const float2*)image + b0 * plane, nullptr,
-                                    (const float2*)kernel + (kernel_batch == 1 ? 0 : b0 * cells), kernel_batch == 1 ? 1 : nb,
-                                    (const float2*)smaps + b0 * smap_b, nb, coils, per_batch ? nb : 1,
-                                    (conj_kernel != 0) != (term == 1) ? 1 : 0, (float2*)ws, (cudaStream_t)stream, nullptr, &sg);
+            const int rc = tz_apply_chunk(p, (const float2*)image + b0 * plane, nullptr,
+                                          (const float2*)kernel + (kernel_batch == 1 ? 0 : b0 * cells), kernel_batch == 1 ? 1 : nb,
+                                          (const float2*)smaps + b0 * smap_b, nb, coils, per_batch ? nb : 1,
+                                          (conj_kernel != 0) != (term == 1) ? 1 : 0, (float2*)ws, (cudaStream_t)stream, nullptr, &sg);
             if (rc) return rc;
         }
-    }
-    return PDU_OK;
+        return PDU_OK;
+    });
 }
 
 size_t pdu_toep_cg_workspace_bytes(const pdu_nufft_plan_t* p, int batch, int coils, int has_smaps) {
@@ -2418,37 +2353,28 @@ size_t pdu_toep_cg_workspace_bytes(const pdu_nufft_plan_t* p, int batch, int coi
 int pdu_toep_cg_c64(pdu_nufft_plan_t* p, const float* b, const float* x0, float* x, const float* kernel, int kernel_batch,
                     const float* smaps, int batch, int coils, int smaps_batch, const float* lam, int lam_count, int max_iter,
                     float tol, int conj_kernel, void* ws, size_t ws_bytes, pdu_stream_t stream) {
-    PDU_REQUIRE(p != nullptr, "pdu_toep_cg_c64: plan is null");
-    PDU_REQUIRE(p->toep, "pdu_toep_cg_c64: not a Toeplitz plan (use pdu_toep_plan_create)");
-    PDU_REQUIRE(b && x && kernel, "pdu_toep_cg_c64: null pointer");
-    PDU_REQUIRE(batch > 0 && coils > 0 && coils <= 65535, "pdu_toep_cg_c64: batch must be > 0 and coils in 1..65535");
-    PDU_REQUIRE(kernel_batch == 1 || kernel_batch == batch, "pdu_toep_cg_c64: kernel batch must be 1 or batch");
-    if (smaps) PDU_REQUIRE(smaps_batch == 1 || smaps_batch == batch, "pdu_toep_cg_c64: smaps batch must be 1 or batch");
-    PDU_REQUIRE(lam_count == 1 || lam_count == batch, "pdu_toep_cg_c64: lam_count must be 1 or batch (got %d)", lam_count);
-    PDU_REQUIRE(max_iter >= 0, "pdu_toep_cg_c64: max_iter must be >= 0 (got %d)", max_iter);
-    PDU_REQUIRE(tol >= 0.f, "pdu_toep_cg_c64: tol must be >= 0");
+    const char* who = "pdu_toep_cg_c64";
+    int rc = check_toep_call(p, b && x && kernel, batch, coils, kernel_batch, smaps, smaps_batch, who);
+    if (rc) return rc;
+    PDU_REQUIRE(lam_count == 1 || lam_count == batch, "%s: lam_count must be 1 or batch (got %d)", who, lam_count);
+    PDU_REQUIRE(max_iter >= 0, "%s: max_iter must be >= 0 (got %d)", who, max_iter);
+    PDU_REQUIRE(tol >= 0.f, "%s: tol must be >= 0", who);
     const int cb = tz_batch_chunk(p, batch, coils);
     const CgWs w = cg_layout(p, cb, coils, smaps != nullptr, ws);
-    PDU_REQUIRE(ws && ws_bytes >= w.bytes, "pdu_toep_cg_c64: workspace of %zu bytes required, got %zu", w.bytes,
-                ws ? ws_bytes : (size_t)0);
-    int dev = -1;
-    PDU_CUDA(cudaGetDevice(&dev));
-    PDU_REQUIRE(dev == p->device, "pdu_toep_cg_c64: plan was created on device %d, current device is %d", p->device, dev);
-    PDU_CHECK_DEVICE("pdu_toep_cg_c64");
+    rc = check_workspace(who, ws, ws_bytes, w.bytes, false, PDU_EINVAL);
+    if (rc) return rc;
+    PDU_CHECK_DEVICE(who);
     const long plane = (long)p->n0 * p->n1, cells = (long)p->k0 * p->k1;
     const long img_b = (smaps ? 1 : coils) * plane, smap_b = smaps_batch == 1 ? 0 : coils * plane;
     const int lam_div = lam_count == 1 ? 0 : (smaps ? 1 : coils);   // system -> batch element within a chunk
     const double tol2 = (double)tol * (double)tol;
-    for (int b0 = 0; b0 < batch; b0 += cb) {
-        const int nb = b0 + cb <= batch ? cb : batch - b0;
-        int rc = tz_cg_chunk(p, (const float2*)b + b0 * img_b, x0 ? (const float2*)x0 + b0 * img_b : nullptr,
-                             (float2*)x + b0 * img_b, (const float2*)kernel + (kernel_batch == 1 ? 0 : b0 * cells),
-                             kernel_batch == 1 ? 1 : nb, smaps ? (const float2*)smaps + b0 * smap_b : nullptr, nb, coils,
-                             smaps_batch == 1 ? 1 : nb, lam ? lam + (lam_count == 1 ? 0 : b0) : nullptr, lam_div, max_iter,
-                             tol2, conj_kernel ? 1 : 0, w, (cudaStream_t)stream);
-        if (rc) return rc;
-    }
-    return PDU_OK;
+    return for_each_chunk(batch, cb, [&](int b0, int nb) {
+        return tz_cg_chunk(p, (const float2*)b + b0 * img_b, x0 ? (const float2*)x0 + b0 * img_b : nullptr,
+                           (float2*)x + b0 * img_b, (const float2*)kernel + (kernel_batch == 1 ? 0 : b0 * cells),
+                           kernel_batch == 1 ? 1 : nb, smaps ? (const float2*)smaps + b0 * smap_b : nullptr, nb, coils,
+                           smaps_batch == 1 ? 1 : nb, lam ? lam + (lam_count == 1 ? 0 : b0) : nullptr, lam_div, max_iter,
+                           tol2, conj_kernel ? 1 : 0, w, (cudaStream_t)stream);
+    });
 }
 
 }  // extern "C"

@@ -11,23 +11,23 @@
 #include "pfft_fast.cuh"
 
 struct pdu_nufft_plan {
-    int n0, n1, k0, k1, J, L, shift0, shift1;
+    int n0 = 0, n1 = 0, k0 = 0, k1 = 0, J = 0, L = 0, shift0 = 0, shift1 = 0;
     int device;
-    float2* d_t0;
-    float2* d_t1;
-    float* d_s0;
-    float* d_s1;
+    float2* d_t0 = nullptr;
+    float2* d_t1 = nullptr;
+    float* d_s0 = nullptr;
+    float* d_s1 = nullptr;
     std::map<int, cufftHandle> fft;   // batched 2-D C2C plans keyed by number of planes
     std::mutex mu;
     // own pruned FFT (pfft.cuh): per-axis radix plans and float64-computed twiddle tables; pfft_ok == false
     // (a grid size with a prime factor above 5) keeps the cuFFT path
-    bool pfft_ok;
+    bool pfft_ok = false;
     pdu::PfftPlan pf0, pf1;
-    float2* d_w0;
-    float2* d_w1;
+    float2* d_w0 = nullptr;
+    float2* d_w1 = nullptr;
     // a plan of the Toeplitz-embedded normal operator (pdu_toep_plan_create): grid 2 n, no interpolation tables, unit
     // apodisation tables of k0 / k1 entries; accepted only by the pdu_toep_* entry points
-    bool toep;
+    bool toep = false;
 };
 
 namespace pdu {
@@ -88,6 +88,14 @@ static inline NufftDims dims_of(const pdu_nufft_plan* p) {
     return d;
 }
 
+// the cropped planes U [planes][n0][n1] of an adjoint as a dense "grid" (k = n), for crop_apod_kernel / smaps_grad_kernel
+static inline NufftDims cropped_dims(const pdu_nufft_plan* p) {
+    NufftDims d = dims_of(p);
+    d.k0 = d.n0;
+    d.k1 = d.n1;
+    return d;
+}
+
 static inline size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 
 // The coil-map gradient ending of an adjoint (pdu_nufft_adj_smaps_grad_c64, pdu_toep_smaps_grad_c64): instead of
@@ -102,6 +110,10 @@ struct SmapsGrad {
     int accumulate;       // add to gs instead of overwriting it
     float scale;          // multiplies the transform's own scale (-1 for the conjugate-gradient solve)
 };
+// The two endings of an adjoint, from planes U [batch][coils] of geometry d (k0 x k1 planes, the n0 x n1 corner kept):
+// the image (x apodisation x scale, x conj(smaps) summed over coils), or the coil-map gradient into sg.gs
+int launch_crop_apod(pdu_nufft_plan* p, const float2* U, NufftDims d, const float2* smaps, float2* image, int out_planes,
+                     int coils, int smaps_batch, float scale, int split, cudaStream_t st);
 int launch_smaps_grad(pdu_nufft_plan* p, const float2* U, NufftDims d, int coils, float scale, const SmapsGrad& sg,
                       cudaStream_t st);
 

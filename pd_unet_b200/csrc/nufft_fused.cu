@@ -637,9 +637,6 @@ static int fused_forward_k(pdu_nufft_plan* p, const float* image, float* kdata, 
     return PDU_OK;
 }
 
-int launch_crop_apod(pdu_nufft_plan* p, const float2* U, const float2* smaps, float2* image, int out_planes, int coils,
-                     int smaps_batch, float scale, int split, cudaStream_t st);      // nufft.cu
-
 template <int K, int PG>
 static int fused_adjoint_k(pdu_nufft_plan* p, const float* kdata, float* image, const float2* smaps, const float* kweight,
                            int batch, int coils, int smaps_batch, long m, float scale, const BinsView& v, int flags, void* ws,
@@ -669,11 +666,8 @@ static int fused_adjoint_k(pdu_nufft_plan* p, const float* kdata, float* image, 
         fz_cols_adj_kernel<K, FZ_SEQ_COLS><<<gc, FZ_SEQ_COLS * FastFft<K>::TPS, fz_cols_smem<K>(), st>>>(
             T, (float*)U, p->d_s0, p->d_s1, p->d_w0, d, 1.f, 0, 0);
         PDU_LAUNCHED();
-        NufftDims dc = d;          // the cropped result is a dense [n0][n1] "grid"
-        dc.k0 = d.n0;
-        dc.k1 = d.n1;
-        int rc = sg ? launch_smaps_grad(p, U, dc, coils, scale, *sg, st)
-                    : launch_crop_apod(p, U, smaps, (float2*)image, batch, coils, smaps_batch, scale, split, st);
+        int rc = sg ? launch_smaps_grad(p, U, cropped_dims(p), coils, scale, *sg, st)
+                    : launch_crop_apod(p, U, cropped_dims(p), smaps, (float2*)image, batch, coils, smaps_batch, scale, split, st);
         if (rc) return rc;
     }
     note_kernel(sg ? OP_SMAPS_GRAD : OP_NUFFT_ADJ, "fz_rows_adj_kernel<%d,%d,%d> (in-row gather + inverse row FFT) + "
@@ -684,22 +678,32 @@ static int fused_adjoint_k(pdu_nufft_plan* p, const float* kdata, float* image, 
     return PDU_OK;
 }
 
+// f(std::integral_constant<int, PG>{}) for the planes per CTA of the fused row passes: 4, or 2 / 8 by the A/B option
+// opt; K = 2048 has no PG = 8 kernel and takes 4 there
+template <int K, typename Fn>
+static int with_fused_pg(int opt, Fn&& f) {
+    if (opt == 2) return f(std::integral_constant<int, 2>{});
+    if constexpr (K != 2048) {
+        if (opt == 8) return f(std::integral_constant<int, 8>{});
+    }
+    return f(std::integral_constant<int, 4>{});
+}
+
 int fused_forward(pdu_nufft_plan* p, const float* image, float* kdata, const float* smaps, int batch, int coils, int smaps_batch,
                   long m, float scale, const void* bins, int flags, void* ws, cudaStream_t st) {
     int rc = check_bins(p, bins, m, "pdu_nufft_fwd_binned_c64");
     if (rc) return rc;
-    const BinsView v = bins_layout(p, m, const_cast<void*>(bins), false);
-    const float2* sm = (const float2*)smaps;
-    const int pg = option(OPT_NUFFT_FWD) == 8 ? 8 : (option(OPT_NUFFT_FWD) == 2 ? 2 : 4);     // A/B: planes per CTA (default 4)
-    switch (p->k0) {
-        case 256: return pg == 8 ? fused_forward_k<256, 8>(p, image, kdata, sm, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : (pg == 2 ? fused_forward_k<256, 2>(p, image, kdata, sm, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : fused_forward_k<256, 4>(p, image, kdata, sm, batch, coils, smaps_batch, m, scale, v, flags, ws, st));
-        case 512: return pg == 8 ? fused_forward_k<512, 8>(p, image, kdata, sm, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : (pg == 2 ? fused_forward_k<512, 2>(p, image, kdata, sm, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : fused_forward_k<512, 4>(p, image, kdata, sm, batch, coils, smaps_batch, m, scale, v, flags, ws, st));
-        case 640: return pg == 8 ? fused_forward_k<640, 8>(p, image, kdata, sm, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : (pg == 2 ? fused_forward_k<640, 2>(p, image, kdata, sm, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : fused_forward_k<640, 4>(p, image, kdata, sm, batch, coils, smaps_batch, m, scale, v, flags, ws, st));
-        case 1024: return pg == 8 ? fused_forward_k<1024, 8>(p, image, kdata, sm, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : (pg == 2 ? fused_forward_k<1024, 2>(p, image, kdata, sm, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : fused_forward_k<1024, 4>(p, image, kdata, sm, batch, coils, smaps_batch, m, scale, v, flags, ws, st));
-        case 2048: return pg == 2 ? fused_forward_k<2048, 2>(p, image, kdata, sm, batch, coils, smaps_batch, m, scale, v, flags, ws, st) : fused_forward_k<2048, 4>(p, image, kdata, sm, batch, coils, smaps_batch, m, scale, v, flags, ws, st);
+    if (!fast_fft_size(p->k0)) {
+        set_error("pdu_nufft_fwd_binned_c64: grid %d has no fused path", p->k0);
+        return PDU_EUNSUPPORTED;
     }
-    set_error("pdu_nufft_fwd_binned_c64: grid %d has no fused path", p->k0);
-    return PDU_EUNSUPPORTED;
+    const BinsView v = bins_layout(p, m, const_cast<void*>(bins), false);
+    return with_fast_fft_size(p->k0, [&](auto k) {
+        return with_fused_pg<decltype(k)::value>(option(OPT_NUFFT_FWD), [&](auto pg) {
+            return fused_forward_k<decltype(k)::value, decltype(pg)::value>(p, image, kdata, (const float2*)smaps, batch, coils,
+                                                                            smaps_batch, m, scale, v, flags, ws, st);
+        });
+    });
 }
 
 int fused_adjoint(pdu_nufft_plan* p, const float* kdata, float* image, const float* smaps, const float* kweight, int batch,
@@ -707,18 +711,17 @@ int fused_adjoint(pdu_nufft_plan* p, const float* kdata, float* image, const flo
                   const SmapsGrad* sg) {
     int rc = check_bins(p, bins, m, "pdu_nufft_adj_binned_c64");
     if (rc) return rc;
-    const BinsView v = bins_layout(p, m, const_cast<void*>(bins), false);
-    const float2* sm = (const float2*)smaps;
-    const int pg = option(OPT_NUFFT_ADJ) == 8 ? 8 : (option(OPT_NUFFT_ADJ) == 2 ? 2 : 4);     // A/B: planes per CTA (default 4)
-    switch (p->k0) {
-        case 256: return pg == 8 ? fused_adjoint_k<256, 8>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : (pg == 2 ? fused_adjoint_k<256, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : fused_adjoint_k<256, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg));
-        case 512: return pg == 8 ? fused_adjoint_k<512, 8>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : (pg == 2 ? fused_adjoint_k<512, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : fused_adjoint_k<512, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg));
-        case 640: return pg == 8 ? fused_adjoint_k<640, 8>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : (pg == 2 ? fused_adjoint_k<640, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : fused_adjoint_k<640, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg));
-        case 1024: return pg == 8 ? fused_adjoint_k<1024, 8>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : (pg == 2 ? fused_adjoint_k<1024, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : fused_adjoint_k<1024, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg));
-        case 2048: return pg == 2 ? fused_adjoint_k<2048, 2>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg) : fused_adjoint_k<2048, 4>(p, kdata, image, sm, kweight, batch, coils, smaps_batch, m, scale, v, flags, ws, st, sg);
+    if (!fast_fft_size(p->k0)) {
+        set_error("pdu_nufft_adj_binned_c64: grid %d has no fused path", p->k0);
+        return PDU_EUNSUPPORTED;
     }
-    set_error("pdu_nufft_adj_binned_c64: grid %d has no fused path", p->k0);
-    return PDU_EUNSUPPORTED;
+    const BinsView v = bins_layout(p, m, const_cast<void*>(bins), false);
+    return with_fast_fft_size(p->k0, [&](auto k) {
+        return with_fused_pg<decltype(k)::value>(option(OPT_NUFFT_ADJ), [&](auto pg) {
+            return fused_adjoint_k<decltype(k)::value, decltype(pg)::value>(p, kdata, image, (const float2*)smaps, kweight, batch,
+                                                                            coils, smaps_batch, m, scale, v, flags, ws, st, sg);
+        });
+    });
 }
 
 }  // namespace pdu

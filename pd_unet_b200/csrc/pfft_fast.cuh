@@ -12,6 +12,8 @@
 // Pruning: HALF_IN  -- inputs K/2 .. K-1 are zero (zero padding of the image), never loaded;
 //          HALF_OUT -- outputs K/2 .. K-1 are not wanted (the crop of the adjoint), never stored.
 #pragma once
+#include <type_traits>
+
 #include "pfft.cuh"
 
 namespace pdu {
@@ -35,6 +37,17 @@ struct FastFft {
     }
 };
 static inline bool fast_fft_size(int K) { return K == 256 || K == 512 || K == 640 || K == 1024 || K == 2048; }
+// f(std::integral_constant<int, K>{}) for the run-time size K, one of fast_fft_size's; returns what f returns
+template <typename Fn>
+static int with_fast_fft_size(int K, Fn&& f) {
+    switch (K) {
+        case 256: return f(std::integral_constant<int, 256>{});
+        case 512: return f(std::integral_constant<int, 512>{});
+        case 640: return f(std::integral_constant<int, 640>{});
+        case 1024: return f(std::integral_constant<int, 1024>{});
+        default: return f(std::integral_constant<int, 2048>{});
+    }
+}
 template <int PS>
 __device__ __forceinline__ int ff_pos(int e) { return e + (e >> PS); }
 

@@ -64,10 +64,62 @@ def kaiser_bessel_scaling(n: int, k: int, numpoints: int, kbwidth: float) -> np.
 _DEFERRED_DESTROY: list = []
 
 
-class _Plan:
+class _DeviceHandles:
+    """Owns one pdu_nufft_plan_t per device, made on first use by the subclass's _create() (on the current device) and
+    destroyed with the owner, deferred while a CUDA graph is being captured (_DEFERRED_DESTROY)."""
+
+    def __init__(self):
+        self._handles: Dict[int, C.c_void_p] = {}
+
+    def handle(self, device: torch.device) -> C.c_void_p:
+        idx = device.index if device.index is not None else torch.cuda.current_device()
+        h = self._handles.get(idx)
+        if h is None:
+            with torch.cuda.device(idx):
+                h = self._create()
+            self._handles[idx] = h
+        return h
+
+    def __del__(self):
+        try:
+            if not self._handles:
+                return
+            _DEFERRED_DESTROY.extend(self._handles.values())
+            if torch.cuda.is_current_stream_capturing():
+                return
+            while _DEFERRED_DESTROY:
+                lib().pdu_nufft_plan_destroy(_DEFERRED_DESTROY.pop())
+        except Exception:
+            pass
+
+
+def _check_norm(norm: Optional[str]) -> None:
+    if norm not in (None, "ortho"):
+        raise ValueError("norm must be None or 'ortho'")
+
+
+def _check_smaps(smaps: Optional[torch.Tensor], batch: int, im_size: Tuple[int, int]):
+    """(smaps [1 or batch, coils, N0, N1], coils, smaps batch), or (None, 0, 1) without maps; 3-D maps get a batch axis."""
+    if smaps is None:
+        return None, 0, 1
+    smaps = require_cuda(smaps, torch.complex64, "smaps")
+    if smaps.dim() == 3:
+        smaps = smaps[None]
+    if smaps.dim() != 4 or tuple(smaps.shape[-2:]) != tuple(im_size) or smaps.shape[0] not in (1, batch):
+        raise ValueError(f"smaps must be [1 or {batch}, coils, {im_size[0]}, {im_size[1]}]")
+    return smaps, smaps.shape[1], smaps.shape[0]
+
+
+def _batch_slice(t: Optional[torch.Tensor], b0: int, b1: int) -> Optional[torch.Tensor]:
+    """Batch elements b0 .. b1 - 1 of t, or t itself when its one entry is shared by the batch."""
+    return t if t is None or t.shape[0] == 1 else t[b0:b1]
+
+
+class _Plan(_DeviceHandles):
     """Owns one pdu_nufft_plan_t per device."""
 
     def __init__(self, im_size, grid_size, numpoints, n_shift, table_oversamp, kbwidth, order):
+        super().__init__()
         if len(im_size) != 2:
             raise NotImplementedError("only 2-D transforms are implemented (radial MRI slices)")
         if float(order) != 0.0:
@@ -82,7 +134,6 @@ class _Plan:
                        for n, k in zip(self.im_size, self.grid_size)]
         self.scaling = [kaiser_bessel_scaling(n, k, self.numpoints, self.kbwidth).astype(np.float32)
                         for n, k in zip(self.im_size, self.grid_size)]
-        self._handles: Dict[int, C.c_void_p] = {}
         # per-trajectory precomputation (row bins of the fused path, CSR form of the adjoint interpolator), keyed by
         # the trajectory tensor's identity; a fixed trajectory is reused by every unrolled iteration / training step
         self._traj: "OrderedDict[tuple, dict]" = OrderedDict()
@@ -209,19 +260,14 @@ class _Plan:
             self._wait(ent)
         return ent["csr"]
 
-    def handle(self, device: torch.device) -> C.c_void_p:
-        idx = device.index if device.index is not None else torch.cuda.current_device()
-        h = self._handles.get(idx)
-        if h is None:
-            h = C.c_void_p()
-            t0, t1 = (np.ascontiguousarray(t) for t in self.tables)
-            s0, s1 = (np.ascontiguousarray(s) for s in self.scaling)
-            with torch.cuda.device(idx):
-                check(lib().pdu_nufft_plan_create(C.byref(h), self.im_size[0], self.im_size[1], self.grid_size[0],
-                                                  self.grid_size[1], self.numpoints, self.table_oversamp,
-                                                  self.n_shift[0], self.n_shift[1], t0.ctypes.data, t1.ctypes.data,
-                                                  s0.ctypes.data, s1.ctypes.data), "pdu_nufft_plan_create")
-            self._handles[idx] = h
+    def _create(self) -> C.c_void_p:
+        h = C.c_void_p()
+        t0, t1 = (np.ascontiguousarray(t) for t in self.tables)
+        s0, s1 = (np.ascontiguousarray(s) for s in self.scaling)
+        check(lib().pdu_nufft_plan_create(C.byref(h), self.im_size[0], self.im_size[1], self.grid_size[0], self.grid_size[1],
+                                          self.numpoints, self.table_oversamp, self.n_shift[0], self.n_shift[1],
+                                          t0.ctypes.data, t1.ctypes.data, s0.ctypes.data, s1.ctypes.data),
+              "pdu_nufft_plan_create")
         return h
 
     def __deepcopy__(self, memo):  # noqa: D105
@@ -231,24 +277,9 @@ class _Plan:
     def __getstate__(self):
         raise TypeError("a NUFFT plan holds device handles and cannot be pickled; rebuild the module instead")
 
-    def __del__(self):
-        try:
-            if not self._handles:
-                return
-            _DEFERRED_DESTROY.extend(self._handles.values())
-            if torch.cuda.is_current_stream_capturing():
-                return
-            while _DEFERRED_DESTROY:
-                lib().pdu_nufft_plan_destroy(_DEFERRED_DESTROY.pop())
-        except Exception:
-            pass
-
     def scale(self, norm: Optional[str]) -> float:
-        if norm is None:
-            return 1.0
-        if norm == "ortho":
-            return 1.0 / math.sqrt(self.grid_size[0] * self.grid_size[1])
-        raise ValueError("norm must be None or 'ortho'")
+        _check_norm(norm)
+        return 1.0 if norm is None else 1.0 / math.sqrt(self.grid_size[0] * self.grid_size[1])
 
     # -------------------------------------------------------------- C-ABI calls (single trajectory)
     def _omega(self, omega: torch.Tensor) -> torch.Tensor:
@@ -256,16 +287,6 @@ class _Plan:
         if omega.dim() != 2 or omega.shape[0] != 2:
             raise ValueError(f"omega must be [2, M], got {tuple(omega.shape)}")
         return omega
-
-    def _smaps(self, smaps, batch):
-        if smaps is None:
-            return None, 0, 1
-        smaps = require_cuda(smaps, torch.complex64, "smaps")
-        if smaps.dim() == 3:
-            smaps = smaps[None]
-        if smaps.dim() != 4 or tuple(smaps.shape[-2:]) != self.im_size or smaps.shape[0] not in (1, batch):
-            raise ValueError(f"smaps must be [1 or {batch}, coils, {self.im_size[0]}, {self.im_size[1]}]")
-        return smaps, smaps.shape[1], smaps.shape[0]
 
     # Layouts.  split=False: complex64 tensors, image [B, C, N0, N1], data [B, C, M] (torchkbnufft's).
     # split=True: float32 tensors with the real and imaginary parts as neighbouring channels, image [B, 2 C, N0, N1],
@@ -290,11 +311,15 @@ class _Plan:
                   "pdu_split_from_complex_f32")
         return out
 
-    def _chunks(self, L, h, B: int, coils: int, M: int):
-        """Batch chunks that keep the fused path's scratch under 1 GiB."""
+    @staticmethod
+    def _binned_chunks(L, h, B: int, coils: int, M: int, device: torch.device):
+        """(b0, b1, workspace) for the batch chunks of a fused-path call, which keep its scratch under 1 GiB."""
         per = max(1, L.pdu_nufft_binned_workspace_bytes(h, coils, M))
         cb = max(1, min(B, (1 << 30) // per))
-        return [(b0, min(B, b0 + cb)) for b0 in range(0, B, cb)]
+        for b0 in range(0, B, cb):
+            b1 = min(B, b0 + cb)
+            yield b0, b1, torch.empty(L.pdu_nufft_binned_workspace_bytes(h, (b1 - b0) * coils, M), dtype=torch.uint8,
+                                      device=device)
 
     def forward(self, image, omega, smaps, norm, split: bool = False):
         image = require_cuda(image, torch.float32 if split else torch.complex64, "image")
@@ -303,7 +328,7 @@ class _Plan:
         omega = self._omega(omega)
         B, M = image.shape[0], omega.shape[1]
         ci = image.shape[1] // 2 if split else image.shape[1]
-        smaps, coils, sb = self._smaps(smaps, B)
+        smaps, coils, sb = _check_smaps(smaps, B, self.im_size)
         if smaps is None:
             coils = ci
         elif ci != 1:
@@ -317,10 +342,9 @@ class _Plan:
             bins = self._bins_for(omega, B * coils, split=split)
             if bins is not None:
                 flags = (NUFFT_IMAGE_SPLIT | NUFFT_KDATA_SPLIT) if split else 0
-                for b0, b1 in self._chunks(L, h, B, coils, M):
+                for b0, b1, ws in self._binned_chunks(L, h, B, coils, M, image.device):
                     nb = b1 - b0
-                    ws = torch.empty(L.pdu_nufft_binned_workspace_bytes(h, nb * coils, M), dtype=torch.uint8, device=image.device)
-                    sm = None if smaps is None else (smaps if sb == 1 else smaps[b0:b1])
+                    sm = _batch_slice(smaps, b0, b1)
                     check(L.pdu_nufft_fwd_binned_c64(h, image[b0:b1].data_ptr(), out[b0:b1].data_ptr(),
                                                      sm.data_ptr() if sm is not None else None, nb, coils, 1 if sb == 1 else nb, M,
                                                      self.scale(norm), bins.data_ptr(), flags, ws.data_ptr(), ws.numel(),
@@ -342,7 +366,7 @@ class _Plan:
             raise ValueError(f"data must be [B, C, {omega.shape[1]}], got {tuple(data.shape)}")
         B, M = data.shape[0], data.shape[2]
         coils = data.shape[1] // 2 if split else data.shape[1]
-        smaps, sc, sb = self._smaps(smaps, B)
+        smaps, sc, sb = _check_smaps(smaps, B, self.im_size)
         if smaps is not None and sc != coils:
             raise ValueError(f"data has {coils} coils, smaps {sc}")
         if kweight is not None:
@@ -361,10 +385,9 @@ class _Plan:
             bins = self._bins_for(omega, B * coils, adjoint=True, split=split)
             if bins is not None:
                 flags = (NUFFT_IMAGE_SPLIT | NUFFT_KDATA_SPLIT) if split else 0
-                for b0, b1 in self._chunks(L, h, B, coils, M):
+                for b0, b1, ws in self._binned_chunks(L, h, B, coils, M, data.device):
                     nb = b1 - b0
-                    ws = torch.empty(L.pdu_nufft_binned_workspace_bytes(h, nb * coils, M), dtype=torch.uint8, device=data.device)
-                    sm = None if smaps is None else (smaps if sb == 1 else smaps[b0:b1])
+                    sm = _batch_slice(smaps, b0, b1)
                     check(L.pdu_nufft_adj_binned_c64(h, data[b0:b1].data_ptr(), out[b0:b1].data_ptr(),
                                                      sm.data_ptr() if sm is not None else None,
                                                      kweight.data_ptr() if kweight is not None else None, nb, coils,
@@ -403,10 +426,9 @@ class _Plan:
         bins = self._bins_for(omega, B * coils, adjoint=True, split=split)
         if bins is not None:
             flags = (NUFFT_IMAGE_SPLIT | NUFFT_KDATA_SPLIT) if split else 0
-            for b0, b1 in self._chunks(L, h, B, coils, M):
+            for b0, b1, ws in self._binned_chunks(L, h, B, coils, M, data.device):
                 nb = b1 - b0
-                ws = torch.empty(L.pdu_nufft_binned_workspace_bytes(h, nb * coils, M), dtype=torch.uint8, device=data.device)
-                g = gs[b0:b1] if per_batch else gs
+                g = _batch_slice(gs, b0, b1)
                 check(L.pdu_nufft_adj_smaps_grad_c64(h, data[b0:b1].data_ptr(), q[b0:b1].data_ptr(), g.data_ptr(), None, None,
                                                      bins.data_ptr(), kweight.data_ptr() if kweight is not None else None, nb,
                                                      coils, g.shape[0], M, self.scale(norm), flags,
@@ -619,25 +641,20 @@ def calc_density_compensation_function(ktraj: torch.Tensor, im_size: Sequence[in
 
 
 # ----------------------------------------------------------------------------- Toeplitz-embedded normal operator
-class _ToepPlan:
+class _ToepPlan(_DeviceHandles):
     """Owns one Toeplitz pdu_nufft_plan_t (grid 2 N, unit apodisation, no tables) per device for one image size."""
 
     def __init__(self, im_size: Tuple[int, int]):
+        super().__init__()
         self.im_size = im_size
-        self._handles: Dict[int, C.c_void_p] = {}
 
-    def handle(self, device: torch.device) -> C.c_void_p:
-        idx = device.index if device.index is not None else torch.cuda.current_device()
-        h = self._handles.get(idx)
-        if h is None:
-            h = C.c_void_p()
-            with torch.cuda.device(idx):
-                rc = lib().pdu_toep_plan_create(C.byref(h), self.im_size[0], self.im_size[1])
-            if rc == PDU_EUNSUPPORTED:
-                raise NotImplementedError(f"no Toeplitz path for a {self.im_size[0]} x {self.im_size[1]} image (the 2 N "
-                                          "embedding grid must factor into 2, 3, 5); there is no CPU fallback")
-            check(rc, "pdu_toep_plan_create")
-            self._handles[idx] = h
+    def _create(self) -> C.c_void_p:
+        h = C.c_void_p()
+        rc = lib().pdu_toep_plan_create(C.byref(h), self.im_size[0], self.im_size[1])
+        if rc == PDU_EUNSUPPORTED:
+            raise NotImplementedError(f"no Toeplitz path for a {self.im_size[0]} x {self.im_size[1]} image (the 2 N "
+                                      "embedding grid must factor into 2, 3, 5); there is no CPU fallback")
+        check(rc, "pdu_toep_plan_create")
         return h
 
     def workspace_bytes(self, h, batch: int, coils: int) -> int:
@@ -646,19 +663,6 @@ class _ToepPlan:
         per = int(L.pdu_toep_workspace_bytes(h, 1))
         cb = min(batch, max(1, min((512 << 20) // per, 65535) // coils))
         return int(L.pdu_toep_workspace_bytes(h, cb * coils))
-
-    def __del__(self):
-        # the same deferred destruction as _Plan: a collection during a CUDA-graph capture must not free device memory
-        try:
-            if not self._handles:
-                return
-            _DEFERRED_DESTROY.extend(self._handles.values())
-            if torch.cuda.is_current_stream_capturing():
-                return
-            while _DEFERRED_DESTROY:
-                lib().pdu_nufft_plan_destroy(_DEFERRED_DESTROY.pop())
-        except Exception:
-            pass
 
 
 _TOEP_PLANS: Dict[Tuple[int, int], _ToepPlan] = {}
@@ -674,11 +678,6 @@ def _toep_plan(im_size) -> _ToepPlan:
     return tp
 
 
-def _check_norm(norm: Optional[str]) -> None:
-    if norm not in (None, "ortho"):
-        raise ValueError("norm must be None or 'ortho'")
-
-
 def _toep_args(image: torch.Tensor, kernel: torch.Tensor, smaps: Optional[torch.Tensor], name: str = "image"):
     """Checked operands of a Toeplitz call: (image, kernel [1 or B, 2 N0, 2 N1], smaps or None, coils, smaps batch)."""
     image = require_cuda(image, torch.complex64, name)
@@ -691,16 +690,11 @@ def _toep_args(image: torch.Tensor, kernel: torch.Tensor, smaps: Optional[torch.
     if kernel.dim() != 3 or tuple(kernel.shape[1:]) != (2 * N0, 2 * N1) or kernel.shape[0] not in (1, B):
         raise ValueError(f"kernel must be [2 N0, 2 N1] = [{2 * N0}, {2 * N1}] or [1 or {B}, {2 * N0}, {2 * N1}] for this image, "
                          f"got {tuple(kernel.shape)}")
-    coils, sb = ci, 1
-    if smaps is not None:
-        smaps = require_cuda(smaps, torch.complex64, "smaps")
-        if smaps.dim() == 3:
-            smaps = smaps[None]
-        if smaps.dim() != 4 or tuple(smaps.shape[-2:]) != (N0, N1) or smaps.shape[0] not in (1, B):
-            raise ValueError(f"smaps must be [1 or {B}, coils, {N0}, {N1}]")
-        if ci != 1:
-            raise ValueError(f"with smaps the {name} must have one channel")
-        coils, sb = smaps.shape[1], smaps.shape[0]
+    smaps, coils, sb = _check_smaps(smaps, B, (N0, N1))
+    if smaps is None:
+        coils = ci
+    elif ci != 1:
+        raise ValueError(f"with smaps the {name} must have one channel")
     return image, kernel, smaps, coils, sb
 
 

@@ -14,7 +14,8 @@ namespace pdu {
 static thread_local char g_err[512] = "";
 static std::atomic<long> g_launches{0};
 static std::atomic<int> g_opts[OPT_COUNT] = {{-1}, {-1}, {-1}, {-1}, {-1}, {-1}, {-1}};
-static thread_local char g_kernel[OP_COUNT][192];
+// room for the longest record (the sorted-gather adjoint, the generic CG: about 270 characters) up to its shape
+static thread_local char g_kernel[OP_COUNT][512];
 
 void set_error(const char* fmt, ...) {
     va_list ap;

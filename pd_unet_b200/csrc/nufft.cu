@@ -1165,7 +1165,9 @@ static int check_workspace(const char* who, const void* ws, size_t bytes, size_t
 
 // A call is cut into batch chunks so that the scratch (plane_bytes per plane) stays under 512 MB and a chunk has at most
 // plane_cap planes.  Measured on B200: chunking the NUFFT down to L2-resident grids (56 MB) does NOT pay -- cuFFT runs at
-// ~3 TB/s either way and the gather / scatter lose parallelism -- so the budget only caps the workspace.
+// ~3 TB/s either way and the gather / scatter lose parallelism -- so the budget only caps the workspace.  Both callers
+// cap a chunk at 65535 planes: their FFT passes launch one grid row per plane (gridDim.y = planes), and on small grids
+// (a 16 x 16 image has 8 KB of oversampled grid, an 8 x 8 Toeplitz plane 3.5 KB) the budget alone allows more.
 static int batch_chunk(size_t plane_bytes, long plane_cap, int batch, int coils) {
     long planes = (long)(((size_t)512 << 20) / plane_bytes);
     if (planes > plane_cap) planes = plane_cap;
@@ -1948,9 +1950,9 @@ size_t pdu_nufft_workspace_bytes(const pdu_nufft_plan_t* p, int planes) {
     return (size_t)planes * (grid + mid + crop) * sizeof(float2);
 }
 
-// batch elements per chunk of the generic path, by its oversampled grids (no plane cap)
+// batch elements per chunk of the generic path, by its oversampled grids; a chunk's planes also fit gridDim.y
 static int nufft_batch_chunk(const pdu_nufft_plan* p, int batch, int coils) {
-    return batch_chunk((size_t)p->k0 * p->k1 * sizeof(float2), LONG_MAX, batch, coils);
+    return batch_chunk((size_t)p->k0 * p->k1 * sizeof(float2), 65535, batch, coils);
 }
 
 // variant 2 = the register-resident pruned FFT (pfft_fast.cuh), 1 = the generic pruned FFT (pfft.cuh), 0 = pad + cuFFT;
